@@ -29,6 +29,8 @@ A step = one pass of the hot path over the whole haystack:
               own (`--leg`), each with its own roofline and CPU baseline.
 
 `--impl reference` times only the reference's CPU implementation on the same workload definition.
+`--dump-outputs DIR` writes the records of the last timed step as .npy files (see dump_records), so
+that two builds can be compared output for output on the same seeded inputs.
 """
 from __future__ import annotations
 
@@ -228,6 +230,32 @@ class DevArray:
         self.__cuda_array_interface__ = {"shape": (count, 3), "typestr": "<i8", "data": (ptr, False), "version": 2}
 
 
+DUMP_MAX_RECORDS = 1 << 21  # three float64 arrays of this length: 48 MiB
+
+
+def dump_records(out_dir: str, torch, dev, rec_ptr: int, count: int):
+    """The records a caller of the timed path receives, as out_dir/<name>.npy (float64):
+    count.npy   [1]  the number of records,
+    index.npy   [k]  which records are stored: all of them, or for more than DUMP_MAX_RECORDS a
+                     fixed seeded sample (sorted), so that the files stay under 64 MB,
+    offset.npy  [k]  their offsets (exact: below 2**53), length.npy [k] their lengths.
+    (A record's `match` pointer is match_ptr_base + offset, with base 0 here: nothing to add.)"""
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    if count > DUMP_MAX_RECORDS:
+        idx = np.sort(np.random.default_rng(20261020).choice(count, DUMP_MAX_RECORDS, replace=False))
+    else:
+        idx = np.arange(count, dtype=np.int64)
+    rec = np.zeros((0, 3), dtype=np.int64)
+    if count:
+        rec = torch.as_tensor(DevArray(rec_ptr, count), device=dev)[torch.from_numpy(idx).to(dev)].cpu().numpy()
+    np.save(d / "count.npy", np.array([count], dtype=np.float64))
+    np.save(d / "index.npy", idx.astype(np.float64))
+    np.save(d / "offset.npy", rec[:, 0].astype(np.float64))
+    np.save(d / "length.npy", (rec[:, 1] & 0xFFFFFFFF).astype(np.float64))
+    log(f"[bench] wrote {idx.size} of {count} records of the last timed step to {d}")
+
+
 # ---------------------------------------------------------------------------------- CPU baseline
 
 def cpu_reference_setup(pattern_buf: bytes, store_flags):
@@ -382,10 +410,10 @@ def run_ours(args):
         t = m.last_timing()
         tot = cnt
         if world > 1:
-            tot, _ = m.gather_records(ptr, cnt, 0, no_overlap)
+            tot, ptr = m.gather_records(ptr, cnt, 0, no_overlap)
         elif no_overlap:
             tot = m.no_overlap_device(ptr, cnt)
-        return cnt, tot, t
+        return cnt, tot, t, ptr
 
     for _ in range(args.warmup):
         step()
@@ -398,9 +426,9 @@ def run_ours(args):
     barrier()
     torch.cuda.synchronize()
     t0 = time.perf_counter()
-    scan_ms, launches, cnt, merged_total = 0.0, 0, 0, 0
+    scan_ms, launches, cnt, merged_total, rec_ptr = 0.0, 0, 0, 0, 0
     for _ in range(args.steps):
-        cnt, merged_total, t = step()
+        cnt, merged_total, t, rec_ptr = step()
         scan_ms += t["scan_ms"]
         launches += int(t["kernel_launches"])
     torch.cuda.synchronize()
@@ -410,6 +438,8 @@ def run_ours(args):
     mx, sm = reduce_max_sum([dt, scan_ms / args.steps, float(cnt), float(launches)])
     dt, scan_ms_step, total_matches, launches = mx[0], mx[1], int(sm[2]), int(sm[3])
     value = total * args.steps / dt / 1e9
+    if args.dump_outputs and rank == 0:  # before the e2e calls below reuse the matcher's record buffer
+        dump_records(args.dump_outputs, torch, dev, rec_ptr, merged_total)
 
     # ---- e2e: host buffers, H2D + kernels (+ gather) + D2H inside the timed region
     own_len = sl_e - sl_b
@@ -684,7 +714,13 @@ def main():
     ap.add_argument("--no-extra", "--no-experimental", dest="no_extra", action="store_true",
                     help="skip other_workloads and the pageable e2e figure (N=1)")
     ap.add_argument("--leg", default=None, choices=sorted(WORKLOADS), help="internal: one other_workloads leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the records of the last timed step to DIR/<name>.npy (float64, at most 48 MiB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours (the reference arm times match counts only)")
     if args.leg:
         return leg_main(args)
     if args.warmup < 3 and args.impl == "ours":

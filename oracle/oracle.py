@@ -214,7 +214,7 @@ class RefLib:
     def lib(cls):
         if cls._lib is None:
             if not REF_SO.exists():
-                raise FileNotFoundError(f"{REF_SO} missing: run `make -C oracle ref` where /root/reference exists")
+                raise FileNotFoundError(f"{REF_SO} missing: run `make -C oracle ref REF=<reference checkout>`")
             cls._lib = bind_list_matcher_api(C.CDLL(str(REF_SO)))
         return cls._lib
 

@@ -1,11 +1,11 @@
 #!/usr/bin/env python3
 """Regenerates tests/golden/ from the reference checkout (run in the build container only).
 
-  python tests/golden/make_golden.py
+  OLM_REFERENCE_DIR=<reference checkout> python tests/golden/make_golden.py
 
 1. data/*.xz      -- the reference's own pattern lists, haystacks and expected-output files
-                     (reference data/, byte-identical, xz-compressed), so that GPU-box tests
-                     never read /root/reference.
+                     (reference data/, byte-identical, xz-compressed), so that the tests
+                     never read the reference checkout.
 2. vectors.json   -- results of the UNMODIFIED reference library (oracle/_ref, built by
                      `make -C oracle ref`) on seeded synthetic inputs over the flag matrix of
                      perf_test.py:69-91 plus word-prefix/word-suffix: match count and an
@@ -34,7 +34,10 @@ ROOT = HERE.parent.parent
 sys.path.insert(0, str(ROOT))
 sys.path.insert(0, str(ROOT / "tests"))
 
-REF_DATA = Path("/root/reference/data")
+if not os.environ.get("OLM_REFERENCE_DIR"):
+    sys.exit("usage: OLM_REFERENCE_DIR=<reference checkout> python tests/golden/make_golden.py "
+             "(oracle/_ref built from the same checkout: make -C oracle ref)")
+REF_DATA = Path(os.environ["OLM_REFERENCE_DIR"]) / "data"  # the checkout oracle/_ref was built from
 FILES = ["names.txt", "surnames_us_census.txt", "tlds.txt", "usernames.txt", "haystack_email.txt",
          "line_anchor_haystack.txt", "line_anchor_patterns.txt", "line_exact_match_haystack.txt",
          "line_exact_match_patterns.txt", "line_exact_haystack.txt", "line_exact_patterns.txt",
