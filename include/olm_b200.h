@@ -294,6 +294,41 @@ int olm_cuda_last_timing(const omega_list_matcher_t *matcher, olm_cuda_timing_t 
  * Also switched on for all matchers by the environment variable OLM_EXACT_STATS=1. */
 int olm_cuda_set_exact_stats(omega_list_matcher_t *matcher, int on);
 
+/* Pattern ids: which pattern of the store produced each match.
+ *
+ * The catalogue of a store is the list of its distinct normalised patterns, defined by the
+ * compiled file alone (stores written by the reference and by this library behave the same):
+ *   ids 0 .. n_long-1   the patterns of 5 or more bytes, in order of their offset in the file's
+ *                       pattern store, which is the order in which each distinct pattern first
+ *                       appeared in the compile input;
+ *   the next ids        the 1-byte, then 2-, 3- and 4-byte patterns, each length in ascending
+ *                       byte order.
+ * The bytes of an id are the pattern as stored: normalised when the store has a transform flag
+ * (`o-malley` in a haystack matches the stored `OMALLEY` of an ignore-case + ignore-punctuation
+ * store, and its id names `OMALLEY`).
+ *
+ * With ids on, omega_list_matcher_match, olm_cuda_match_device, olm_cuda_match_shard and
+ * olm_cuda_match_shard_host return records whose 4 pad bytes (after `len`) hold the id
+ * (olm_result_with_id_t names them); the records are otherwise byte for byte those of a call with
+ * ids off, where the pad bytes are 0.  The ids are resolved on the GPU after the filters, one more
+ * kernel per call, included in olm_cuda_timing_t.total_ms; sorting, no_overlap and the gathers
+ * move whole records, so ids follow their records.  Switching on first builds the catalogue and
+ * uploads a lookup table (about 24 bytes per pattern of device memory); it returns -1 for a store
+ * whose pattern records are malformed (out of range, or two at one offset).  A call fails (-1 /
+ * NULL, with a message on stderr) rather than return a record without its id. */
+typedef struct {
+  size_t offset;
+  uint32_t len;
+  uint32_t pattern_id;
+  const uint8_t *match;
+} olm_result_with_id_t; /* omega_match_result_t with the pad named (same layout) */
+int olm_cuda_set_pattern_ids(omega_list_matcher_t *matcher, int on); /* default off */
+/* Catalogue size, or -1 on a malformed store.  No GPU work. */
+int64_t olm_pattern_count(const omega_list_matcher_t *matcher);
+/* The bytes of pattern `id` (valid for the matcher's lifetime); -1 for an id out of range. */
+int olm_pattern_bytes(const omega_list_matcher_t *matcher, uint64_t id, const uint8_t **bytes,
+                      uint32_t *len);
+
 /* Pinned host memory helpers (so callers can hand DMA-able buffers to _match). */
 void *olm_cuda_host_alloc(size_t bytes);
 void olm_cuda_host_free(void *p);

@@ -5,7 +5,7 @@ ABI, see include/olm_b200.h); this package is the host-side mirror of the refere
 binding plus the device-resident / sharded entry points.
 """
 from .omega_match import (Compiler, Matcher, MatchResult, MatchStats, PatternStoreStats, get_library_info,
-                          get_version, MATCH_DTYPE, RECORD_DTYPE, FLAG_NAMES)
+                          get_version, MATCH_DTYPE, MATCH_IDS_DTYPE, RECORD_DTYPE, FLAG_NAMES)
 
 __all__ = ["Compiler", "Matcher", "MatchResult", "MatchStats", "PatternStoreStats", "get_version",
-           "get_library_info", "MATCH_DTYPE", "RECORD_DTYPE", "FLAG_NAMES"]
+           "get_library_info", "MATCH_DTYPE", "MATCH_IDS_DTYPE", "RECORD_DTYPE", "FLAG_NAMES"]

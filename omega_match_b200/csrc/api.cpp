@@ -2,10 +2,12 @@
 // include/olm_b200.h).  Thin: argument checking, file handling, and calls into Engine.
 #include <unistd.h>
 
+#include <cstddef>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <exception>
+#include <memory>
 #include <string>
 #include <thread>
 
@@ -33,7 +35,17 @@ struct omega_list_matcher_struct {
   bool exact_stats = false; // olm_cuda_set_exact_stats / OLM_EXACT_STATS=1
   int threads = 1;
   int chunk = 4096;
+  // pattern ids: the store's catalogue, built on first use (olm_pattern_count & co. are const)
+  mutable std::unique_ptr<olm::PatternCatalog> catalog;
+  mutable std::string catalog_err;
 };
+
+static_assert(sizeof(olm_result_with_id_t) == sizeof(omega_match_result_t) &&
+                  offsetof(olm_result_with_id_t, offset) == offsetof(omega_match_result_t, offset) &&
+                  offsetof(olm_result_with_id_t, len) == offsetof(omega_match_result_t, len) &&
+                  offsetof(olm_result_with_id_t, pattern_id) == offsetof(omega_match_result_t, len) + 4 &&
+                  offsetof(olm_result_with_id_t, match) == offsetof(omega_match_result_t, match),
+              "olm_result_with_id_t is omega_match_result_t with its pad named");
 
 namespace {
 
@@ -145,6 +157,26 @@ omega_list_matcher_t *create_on(const char *path, int case_insensitive, int igno
   omega_matcher_set_num_threads(m, 0); // matcher.c:509-511
   omega_matcher_set_chunk_size(m, 0);
   return m;
+}
+
+// the matcher's catalogue, built when first asked for; nullptr (and a message on stderr) for a
+// store the catalogue rejects
+const olm::PatternCatalog *catalog_of(const omega_list_matcher_t *m) {
+  if (!m || !m->file) return nullptr;
+  if (!m->catalog && m->catalog_err.empty()) {
+    olm::StoreView v;
+    std::string err = olm::parse_store(m->file, m->file_size, &v);
+    auto c = std::make_unique<olm::PatternCatalog>();
+    try {
+      if (err.empty()) err = olm::build_catalog(v, c.get());
+    } catch (const std::exception &ex) {
+      err = std::string("malformed store (") + ex.what() + ")";
+    }
+    if (err.empty()) m->catalog = std::move(c);
+    else m->catalog_err = err;
+  }
+  if (!m->catalog) std::fprintf(stderr, "libomega_match(b200): no pattern catalogue: %s\n", m->catalog_err.c_str());
+  return m->catalog.get();
 }
 } // namespace
 
@@ -329,6 +361,27 @@ int olm_cuda_set_exact_stats(omega_list_matcher_t *m, int on) {
   m->exact_stats = on != 0;
   if (m->multi) m->multi->set_exact_stats(m->exact_stats && m->stats);
   else m->engine->set_exact_stats(m->exact_stats && m->stats); // the kernel runs only for an attached struct
+  return 0;
+}
+
+int olm_cuda_set_pattern_ids(omega_list_matcher_t *m, int on) {
+  if (!m || !m->engine) return -1;
+  const olm::PatternCatalog *c = nullptr;
+  if (on && !(c = catalog_of(m))) return -1;
+  return m->multi ? m->multi->set_pattern_ids(on != 0, c) : m->engine->set_pattern_ids(on != 0, c);
+}
+
+int64_t olm_pattern_count(const omega_list_matcher_t *m) {
+  const olm::PatternCatalog *c = catalog_of(m);
+  return c ? int64_t(c->size()) : -1;
+}
+
+int olm_pattern_bytes(const omega_list_matcher_t *m, uint64_t id, const uint8_t **bytes, uint32_t *len) {
+  if (!bytes || !len) return -1;
+  const olm::PatternCatalog *c = catalog_of(m);
+  if (!c || id >= c->size()) return -1;
+  *bytes = c->bytes(id);
+  *len = c->refs[id].y;
   return 0;
 }
 

@@ -31,6 +31,7 @@
 
 #include "filters.cuh"
 #include "format.cuh"
+#include "pattern_ids.cuh"
 #include "scan.cuh"
 #include "stats.cuh"
 #include "transform.cuh"
@@ -143,6 +144,10 @@ struct EngineImpl {
   // statistics of the spans before the last one (collect_stats adds them to the last call's)
   uint64_t host_span = 0;
   omega_match_stats_t span_acc{};
+  // pattern ids (pattern_ids.cuh): tables uploaded when first switched on
+  bool want_ids = false;
+  PatternIdTables ids;
+  DevBuf d_id_table, d_id_refs, d_id_short;
 };
 
 namespace {
@@ -281,7 +286,7 @@ Engine::~Engine() {
   for (DevBuf *b : {&impl_->d_keys, &impl_->d_slots, &impl_->d_recs, &impl_->d_store, &impl_->d_g4, &impl_->d_p23, &impl_->d_sx, &impl_->d_set3,
                     &impl_->d_bitmap2, &impl_->hay, &impl_->out, &impl_->out2, &impl_->chunk_desc, &impl_->span_base, &impl_->temp, &impl_->tfblocks, &impl_->tfvisible, &impl_->tfplan, &impl_->tfextent, &impl_->misc,
                     &impl_->windows, &impl_->gather, &impl_->text, &impl_->ghost, &impl_->fscratch, &impl_->d_bloom, &impl_->d_smap,
-                    &impl_->d_slens})
+                    &impl_->d_slens, &impl_->d_id_table, &impl_->d_id_refs, &impl_->d_id_short})
     b->release();
   for (auto &ev : impl_->ev)
     if (ev) cudaEventDestroy(ev);
@@ -549,6 +554,28 @@ int Engine::match_device(const ScanRange &r, const MatchFlags &f, olm_cuda_resul
     E.last.kernel_launches += launches;
     std::swap(E.out, E.out2);
     final_records = E.out.p;
+  }
+  if (E.want_ids && total) {
+    unsigned long long *d_missing = d_total + 16; // (misc words 16.. are not cleared with the scan's)
+    unsigned long long missing = 0;
+    uint32_t launches = 0;
+    // (the host path: a record may end in a segment the scan did not have to wait for)
+    if (E.streaming && !E.seg_events.empty() && wait_segment(E, E.seg_events.size() - 1)) return -1;
+    OLM_CUDA(cudaMemsetAsync(d_missing, 0, sizeof missing, E.stream));
+    OLM_CUDA(cudaEventRecord(E.ev[2], E.stream));
+    OLM_CUDA(pattern_ids_launch(static_cast<Record *>(final_records), total, static_cast<const uint8_t *>(r.dev),
+                                r.slice_begin, E.ids, d_missing, E.sms, E.stream, &launches));
+    OLM_CUDA(cudaEventRecord(E.ev[3], E.stream));
+    OLM_CUDA(cudaMemcpyAsync(&missing, d_missing, sizeof missing, cudaMemcpyDeviceToHost, E.stream));
+    OLM_CUDA(cudaStreamSynchronize(E.stream));
+    cudaEventElapsedTime(&ms, E.ev[2], E.ev[3]);
+    E.last.total_ms += ms;
+    E.last.kernel_launches += launches;
+    if (missing) {
+      std::fprintf(stderr, "libomega_match(b200): %llu records matched no pattern of the catalogue (internal error)\n",
+                   missing);
+      return -1;
+    }
   }
   // statistics that do not need a kernel: long-path attempts without word_boundary
   if (E.hdr.largest >= 5 && !f.word_boundary && !windowed) {
@@ -903,6 +930,24 @@ int Engine::sync() {
 }
 
 void Engine::set_exact_stats(bool on) { impl_->want_stats = on; }
+
+int Engine::set_pattern_ids(bool on, const PatternCatalog *cat) {
+  EngineImpl &E = *impl_;
+  if (on && !E.ids.table) {
+    if (!cat) return -1;
+    OLM_CUDA(cudaSetDevice(E.device));
+    PatternIdTables t;
+    if (upload(E.d_id_table, cat->table, &t.table) || upload(E.d_id_refs, cat->refs, &t.refs) ||
+        upload(E.d_id_short, cat->short_bytes, &t.short_bytes))
+      return -1;
+    t.table_mask = cat->table_mask;
+    t.store = E.ds.store;
+    t.store_flags = E.hdr.flags;
+    E.ids = t;
+  }
+  E.want_ids = on;
+  return 0;
+}
 
 void Engine::collect_stats(omega_match_stats_t *s) {
   if (!s) return;

@@ -71,6 +71,10 @@ public:
   void set_exact_stats(bool on);
   // host threads that stage PAGEABLE haystacks through pinned memory (omega_matcher_set_num_threads)
   void set_host_threads(int n);
+  // While on, every call writes the id of each final record's pattern into its pad word
+  // (pattern_ids.cuh); off (default): the pad stays 0.  The first switch on uploads the catalogue's
+  // lookup table (`cat`, the catalogue of this engine's store; not needed to switch off).
+  int set_pattern_ids(bool on, const PatternCatalog *cat);
 
 private:
   Engine() = default;

@@ -337,6 +337,11 @@ void MultiMatcher::collect_stats(omega_match_stats_t *s) {
 void MultiMatcher::set_exact_stats(bool on) {
   for (Engine *e : engines_) e->set_exact_stats(on);
 }
+int MultiMatcher::set_pattern_ids(bool on, const PatternCatalog *cat) {
+  for (Engine *e : engines_)
+    if (e->set_pattern_ids(on, cat) != 0) return -1;
+  return 0;
+}
 
 // ================================ (2) one process per GPU =========================================
 

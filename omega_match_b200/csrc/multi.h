@@ -29,6 +29,7 @@ public:
   omega_match_results_t *match_host(const uint8_t *haystack, size_t n, const MatchFlags &f);
   void collect_stats(omega_match_stats_t *accum);
   void set_exact_stats(bool on);
+  int set_pattern_ids(bool on, const PatternCatalog *cat); // every engine (Engine::set_pattern_ids)
   const olm_cuda_timing_t &timing() const { return last_; }
   Engine *first() const { return engines_.front(); }
   int size() const { return (int)engines_.size(); }

@@ -483,6 +483,64 @@ std::string stage_stats(const StoreView &v, StagedStats *s) {
   return "";
 }
 
+std::string build_catalog(const StoreView &v, PatternCatalog *c) {
+  *c = PatternCatalog{};
+  const Header &h = v.hdr;
+  if (h.store_bytes >= 0xFFFFFFF0ull) return "pattern store of 4 GiB or more is not supported";
+  c->patterns = v.patterns;
+  // ---- long patterns: every bucket record, in order of store_off
+  for (uint64_t p = 0; p < h.blob_bytes;) {
+    if (p + 8 > h.blob_bytes) return "truncated bucket header";
+    const uint32_t count = rd32(v.blob + p + 4);
+    if (count == 0 || p + 8 + uint64_t(count) * kBucketRecordBytes > h.blob_bytes) return "bucket runs past the bucket data";
+    for (uint32_t j = 0; j < count; ++j) {
+      const uint64_t po = rd64(v.blob + p + 8 + 16ull * j);
+      const uint32_t pl = rd32(v.blob + p + 8 + 16ull * j + 8);
+      if (pl < 5 || po > h.store_bytes || pl > h.store_bytes - po) return "pattern record out of range";
+      c->refs.push_back(make_uint2(uint32_t(po), pl));
+    }
+    p += 8 + uint64_t(count) * kBucketRecordBytes;
+  }
+  std::sort(c->refs.begin(), c->refs.end(), [](const uint2 &a, const uint2 &b) { return a.x < b.x; });
+  for (size_t i = 1; i < c->refs.size(); ++i)
+    if (c->refs[i].x == c->refs[i - 1].x) return "two pattern records share a store offset";
+  c->n_long = uint32_t(c->refs.size());
+  // ---- short patterns, each length in ascending byte order
+  auto add_short = [&](uint32_t be, uint32_t len) { // be = the bytes packed big endian
+    c->refs.push_back(make_uint2(uint32_t(c->short_bytes.size()), len));
+    for (uint32_t k = len; k-- > 0;) c->short_bytes.push_back(uint8_t(be >> (8 * k)));
+  };
+  for (uint32_t b = 0; b < 256 && v.bitmap1; ++b)
+    if (v.bitmap1[b >> 3] & (1u << (b & 7))) add_short(b, 1);
+  for (uint32_t w = 0; w < 65536 && v.bitmap2; ++w)
+    if (v.bitmap2[w >> 3] & (1u << (w & 7))) add_short(w, 2);
+  for (uint32_t i = 0; i < v.n3; ++i) add_short(rd32(v.arr3 + 4ull * i) & 0xFFFFFFu, 3);
+  for (uint32_t i = 0; i < v.n4; ++i) add_short(rd32(v.arr4 + 4ull * i), 4);
+  if (c->refs.size() >= kNoPatternId) return "too many patterns";
+
+  // ---- lookup table; of two ids with the same bytes (a hand-made file) the lower one is kept
+  const uint32_t lg = std::max<uint32_t>(4, ceil_log2(uint64_t(c->refs.size()) * 2));
+  c->table.assign(size_t(1) << lg, make_uint2(kNoPatternId, 0));
+  c->table_mask = (1u << lg) - 1;
+  for (uint32_t id = 0; id < c->refs.size(); ++id) {
+    const uint8_t *b = c->bytes(id);
+    const uint32_t len = c->refs[id].y;
+    uint64_t hv = kPatternHashSeed;
+    for (uint32_t k = 0; k < len; ++k) hv = pattern_hash_step(hv, b[k]);
+    hv = pattern_hash_final(hv, len);
+    const uint32_t fp = pattern_fingerprint(hv);
+    for (uint32_t i = pattern_home(hv, c->table_mask);; i = (i + 1) & c->table_mask) {
+      uint2 &e = c->table[i];
+      if (e.x == kNoPatternId) {
+        e = make_uint2(id, fp);
+        break;
+      }
+      if (e.y == fp && c->refs[e.x].y == len && std::memcmp(c->bytes(e.x), b, len) == 0) break;
+    }
+  }
+  return "";
+}
+
 uint64_t check_staged_store(const StoreView &v, const StagedStore &s) {
   const DeviceStore &d = s.params;
   uint64_t bad = 0;

@@ -66,6 +66,61 @@ std::string stage_stats(const StoreView &v, StagedStats *out);
 // Used by CPU-only tests; it does not match haystacks.
 uint64_t check_staged_store(const StoreView &v, const StagedStore &s);
 
+// ---- pattern ids (include/olm_b200.h): the catalogue of a store and its lookup table
+//
+// Id i names the i-th distinct normalised pattern of the file: the long patterns (>= 5 bytes) in
+// order of their offset in the pattern store -- the order in which each first appeared in the
+// compile input -- then the 1-, 2-, 3- and 4-byte patterns, each length in ascending byte order
+// (bitmap1 bit order, bitmap2 bit order b0<<8|b1, arr3 order, arr4 order).  The catalogue is
+// defined by the .olm file alone and is built on the host when first asked for.
+//
+// The lookup table is open addressing over a 64-bit hash of (length, bytes): one 8-byte entry
+// {id, fingerprint} per pattern, load <= 0.5; the id pass (pattern_ids.cuh) probes it with the
+// hash of a record's normalised bytes and confirms a fingerprint hit with a full byte compare.
+struct PatternCatalog {
+  uint32_t n_long = 0;
+  std::vector<uint2> refs;          // per id: {offset, len}; offset into the pattern store (len >= 5) or into short_bytes
+  std::vector<uint8_t> short_bytes; // bytes of the 1..4 byte patterns, concatenated
+  const uint8_t *patterns = nullptr; // StoreView::patterns (the mapped file outlives the catalogue)
+  std::vector<uint2> table;         // {id, fingerprint}; id kNoPatternId = empty
+  uint32_t table_mask = 0;
+  uint64_t size() const { return refs.size(); }
+  const uint8_t *bytes(uint64_t id) const {
+    return refs[id].y >= 5 ? patterns + refs[id].x : short_bytes.data() + refs[id].x;
+  }
+};
+constexpr uint32_t kNoPatternId = 0xFFFFFFFFu;
+std::string build_catalog(const StoreView &v, PatternCatalog *out);
+
+// Hash of a pattern's normalised bytes, fed one byte at a time (the device feeds it while it
+// normalises a record's source span), then finished with the length.  FNV-1a 64 + a murmur3 finaliser.
+#if defined(__CUDACC__)
+__host__ __device__
+#endif
+inline uint64_t pattern_hash_step(uint64_t h, uint32_t byte) { return (h ^ byte) * 0x100000001B3ull; }
+constexpr uint64_t kPatternHashSeed = 0xCBF29CE484222325ull;
+#if defined(__CUDACC__)
+__host__ __device__
+#endif
+inline uint64_t pattern_hash_final(uint64_t h, uint32_t len) {
+  h ^= uint64_t(len) * 0x9E3779B97F4A7C15ull;
+  h ^= h >> 33;
+  h *= 0xFF51AFD7ED558CCDull;
+  h ^= h >> 33;
+  h *= 0xC4CEB9FE1A85EC53ull;
+  h ^= h >> 33;
+  return h;
+}
+// home slot of a hash / its fingerprint
+#if defined(__CUDACC__)
+__host__ __device__
+#endif
+inline uint32_t pattern_home(uint64_t h, uint32_t mask) { return uint32_t(h >> 32) & mask; }
+#if defined(__CUDACC__)
+__host__ __device__
+#endif
+inline uint32_t pattern_fingerprint(uint64_t h) { return uint32_t(h); }
+
 // host mirror of the device hashing (scan.cu uses the same expressions)
 inline uint32_t key_home(const DeviceStore &d, uint32_t key) { return key >> d.key_shift; }
 inline uint32_t g4_bit(const DeviceStore &d, uint32_t key) { return key >> d.g4_shift; }

@@ -8,7 +8,8 @@ omega_match_b200/lib/libomega_match.so (see INTEGRATION.md).
 
 Additions (not in the reference): `Matcher.match_arrays` (numpy result without per-match
 Python objects), `Matcher.match_device` / `match_shard` (device-resident haystack and
-results), `Matcher.last_timing`.
+results), `Matcher.last_timing`, pattern ids (`Matcher.match_ids`, `set_pattern_ids`,
+`pattern_count`, `pattern`).
 """
 from __future__ import annotations
 
@@ -23,6 +24,8 @@ from ._lib import (CudaResultsC, CudaTimingC, MatchStatsC, PatternStoreStatsC)
 
 # (offset, len) pairs as tests and benches consume them
 MATCH_DTYPE = np.dtype([("offset", "<u8"), ("len", "<u4"), ("_pad", "<u4")])
+# match_ids(): the same 16 bytes, the pad holding the pattern id (include/olm_b200.h)
+MATCH_IDS_DTYPE = np.dtype([("offset", "<u8"), ("len", "<u4"), ("pattern_id", "<u4")])
 # omega_match_result_t as the library writes it (24 bytes)
 RECORD_DTYPE = np.dtype([("offset", "<u8"), ("len", "<u4"), ("_pad", "<u4"), ("match", "<u8")])
 
@@ -142,6 +145,7 @@ class Compiler:
 
 class Matcher:
     _matcher = None
+    _pattern_ids = False
 
     def __init__(self, compiled_or_patterns_file: str, case_insensitive: bool = False,
                  ignore_punctuation: bool = False, elide_whitespace: bool = False,
@@ -252,9 +256,50 @@ class Matcher:
         out["len"] = rec["len"]
         return out
 
+    # -- pattern ids (include/olm_b200.h) ------------------------------------------------------
+    def set_pattern_ids(self, on: bool = True) -> None:
+        """While on, every match call writes the id of each record's pattern into the record's pad
+        word (RECORD_DTYPE `_pad`): match_device / match_shard / match_shard_host records carry ids.
+        Switching on the first time builds the catalogue and uploads its lookup table."""
+        if self._lib.olm_cuda_set_pattern_ids(self._matcher, int(bool(on))) != 0:
+            raise RuntimeError("olm_cuda_set_pattern_ids failed (malformed store? see stderr)")
+        self._pattern_ids = bool(on)
+
+    @property
+    def pattern_count(self) -> int:
+        """Number of distinct normalised patterns of the store: ids are 0 .. pattern_count - 1."""
+        n = self._lib.olm_pattern_count(self._matcher)
+        if n < 0:
+            raise RuntimeError("olm_pattern_count failed (malformed store? see stderr)")
+        return int(n)
+
+    def pattern(self, pattern_id: int) -> bytes:
+        """The stored (normalised) bytes of a pattern id."""
+        p, n = C.c_void_p(), C.c_uint32()
+        if pattern_id < 0 or self._lib.olm_pattern_bytes(self._matcher, pattern_id, C.byref(p), C.byref(n)) != 0:
+            raise IndexError(f"pattern id {pattern_id} out of range")
+        return C.string_at(p.value, n.value) if n.value else b""
+
+    def match_ids(self, haystack, **kw) -> np.ndarray:
+        """Like match_arrays(), with the id of each match's pattern: MATCH_IDS_DTYPE (offset, len,
+        pattern_id) in result order.  Ids are switched on for this call only."""
+        was = self._pattern_ids
+        self.set_pattern_ids(True)
+        try:
+            rec = self._match_records(haystack, **kw)
+        finally:
+            if not was:
+                self.set_pattern_ids(False)
+        out = np.zeros(rec.size, dtype=MATCH_IDS_DTYPE)
+        out["offset"] = rec["offset"]
+        out["len"] = rec["len"]
+        out["pattern_id"] = rec["_pad"]
+        return out
+
     def match_device(self, dev_ptr: int, size: int, match_ptr_base: Optional[int] = None, **kw):
         """Haystack already in HBM (16-byte aligned device pointer).  Returns (count, device
-        pointer of the 24-byte records); the records stay valid until the next call."""
+        pointer of the 24-byte records); the records stay valid until the next call.  With
+        set_pattern_ids(True) their pad words hold the pattern ids."""
         res = CudaResultsC()
         base = dev_ptr if match_ptr_base is None else match_ptr_base
         if self._lib.olm_cuda_match_device(self._matcher, dev_ptr, size, base, *_flag_ints(kw), C.byref(res)) != 0:
@@ -263,7 +308,8 @@ class Matcher:
 
     def match_shard(self, dev_ptr: int, slice_begin: int, slice_len: int, own_begin: int, own_end: int,
                     global_size: int, match_ptr_base: int = 0, **kw):
-        """One byte-range shard of a larger haystack (SURVEY 8e); no_overlap is not applied."""
+        """One byte-range shard of a larger haystack (SURVEY 8e); no_overlap is not applied.  With
+        set_pattern_ids(True) the records' pad words hold the pattern ids."""
         if kw.get("no_overlap"):
             raise ValueError("no_overlap crosses shards: apply Matcher.no_overlap_device on the gathered records")
         f = _flag_ints(kw)[1:]
@@ -276,7 +322,8 @@ class Matcher:
     def match_shard_host(self, host_ptr: int, slice_begin: int, slice_len: int, own_begin: int, own_end: int,
                          global_size: int, match_ptr_base: int = 0, **kw):
         """match_shard() for a slice in host memory: segmented H2D overlapped with the scan; the
-        records stay on the device (include/olm_b200.h olm_cuda_match_shard_host)."""
+        records stay on the device (include/olm_b200.h olm_cuda_match_shard_host).  With
+        set_pattern_ids(True) their pad words hold the pattern ids."""
         if kw.get("no_overlap"):
             raise ValueError("no_overlap crosses shards: apply Matcher.no_overlap_device on the gathered records")
         f = _flag_ints(kw)[1:]
