@@ -175,6 +175,9 @@ typedef struct {
  *                             spans of n bytes (bounded device memory; same results)
  *   OLM_SHORT_LOOK=0|1        never / whenever there is room: the second look at candidates of the
  *                             1..3 byte patterns (default: for stores with 1-byte patterns)
+ *   OLM_COUNT_TABLE=0|1       the histogram of the pattern counts without / with its per-block
+ *                             table of ids (default: with it from 64 records per catalogue pattern;
+ *                             same counts either way).  For tests and measurements of both.
  * and at olm_cuda_comm_create():
  *   OLM_GATHER_WINDOW=0       gather with ncclSend/ncclRecv instead of the IPC window */
 int olm_cuda_device_count(void);
@@ -328,6 +331,41 @@ int64_t olm_pattern_count(const omega_list_matcher_t *matcher);
 /* The bytes of pattern `id` (valid for the matcher's lifetime); -1 for an id out of range. */
 int olm_pattern_bytes(const omega_list_matcher_t *matcher, uint64_t id, const uint8_t **bytes,
                       uint32_t *len);
+
+/* Pattern counts: how often each pattern of the store occurs, without returning the records.
+ *
+ * A count call takes the haystack and the seven match flags of the match call it mirrors and adds to
+ * counts[id] one for every record that call would have returned (longest_only and no_overlap
+ * applied) whose pattern is `id` (the id defined above).  `counts` has olm_pattern_count() entries.
+ * The counts are ADDED (+=), as omega_match_stats_t is, so calls, spans, shards and GPUs sum without
+ * more API; *total receives the number of records this call counted, the `count` of the equivalent
+ * match call.
+ *   - Pattern ids may be on or off; a count call leaves that setting as it was (a later match call
+ *     with ids off still returns zero pads).  The first count call builds the catalogue and uploads
+ *     its lookup table, as olm_cuda_set_pattern_ids does.
+ *   - The records never leave the GPU; only the counts (8 bytes per pattern) are copied.
+ *   - A record whose bytes name no pattern of the catalogue, and a malformed store, fail the call
+ *     (-1, message on stderr); the contents of `counts` are then unspecified.
+ *   - The counting pass is part of olm_cuda_timing_t.total_ms, the copy of the counts of d2h_ms.
+ * On the device the ids of a call's final records are resolved as with ids on and added into a
+ * histogram; records in offset order repeat ids within a warp and a block, which the histogram
+ * aggregates before it adds to global memory. */
+/* host haystack -> host counts: the one-GPU path, OLM_HOST_SPAN_BYTES spans, multi-GPU matchers */
+int olm_cuda_count_patterns(const omega_list_matcher_t *matcher, const uint8_t *haystack, size_t size,
+                            int no_overlap, int longest_only, int word_boundary, int word_prefix,
+                            int word_suffix, int line_start, int line_end, uint64_t *counts, uint64_t *total);
+/* device haystack (the contract of olm_cuda_match_device) -> counts in device memory of the
+ * matcher's (first) GPU */
+int olm_cuda_count_patterns_device(const omega_list_matcher_t *matcher, const void *dev_haystack, size_t size,
+                                   int no_overlap, int longest_only, int word_boundary, int word_prefix,
+                                   int word_suffix, int line_start, int line_end, void *dev_counts,
+                                   uint64_t *total);
+/* Records in device memory of the matcher's (first) GPU whose pad words hold ids (made with ids on:
+ * shards, olm_cuda_gather_records) -> device counts.  One process per GPU counts each rank's shard
+ * and sums the ranks' counts by its own means, or gathers the records (no_overlap included) and
+ * counts on the root.  An id >= olm_pattern_count() fails the call (-1). */
+int olm_cuda_count_records(const omega_list_matcher_t *matcher, const void *dev_records, uint64_t count,
+                           void *dev_counts);
 
 /* Pinned host memory helpers (so callers can hand DMA-able buffers to _match). */
 void *olm_cuda_host_alloc(size_t bytes);

@@ -119,6 +119,9 @@ ABI = [
     ("olm_cuda_set_pattern_ids", _ci, [_vp, _ci]),
     ("olm_pattern_count", C.c_int64, [_vp]),
     ("olm_pattern_bytes", _ci, [_vp, C.c_uint64, C.POINTER(C.c_void_p), C.POINTER(C.c_uint32)]),
+    ("olm_cuda_count_patterns", _ci, [_vp, _vp, C.c_size_t] + _flags7 + [_vp, C.POINTER(C.c_uint64)]),
+    ("olm_cuda_count_patterns_device", _ci, [_vp, _vp, C.c_size_t] + _flags7 + [_vp, C.POINTER(C.c_uint64)]),
+    ("olm_cuda_count_records", _ci, [_vp, _vp, C.c_uint64, _vp]),
     ("olm_cuda_host_alloc", _vp, [C.c_size_t]),
     ("olm_cuda_host_free", None, [_vp]),
     ("olm_store_inspect", _ci, [_cp, C.POINTER(StoreInfoC)]),

@@ -385,6 +385,57 @@ int olm_pattern_bytes(const omega_list_matcher_t *m, uint64_t id, const uint8_t 
   return 0;
 }
 
+namespace {
+// the catalogue's lookup table on every GPU of the matcher (ids stay as they are); -1 on a malformed store
+int load_pattern_tables(const omega_list_matcher_t *m) {
+  const olm::PatternCatalog *c = catalog_of(m);
+  if (!c) return -1;
+  return m->multi ? m->multi->load_pattern_tables(c) : m->engine->load_pattern_tables(c);
+}
+} // namespace
+
+int olm_cuda_count_patterns(const omega_list_matcher_t *m, const uint8_t *haystack, size_t size, int no_overlap,
+                            int longest_only, int word_boundary, int word_prefix, int word_suffix, int line_start,
+                            int line_end, uint64_t *counts, uint64_t *total) {
+  if (!m || !m->engine || !counts || !total || (!haystack && size) || load_pattern_tables(m)) return -1;
+  const olm::MatchFlags f = to_flags(no_overlap, longest_only, word_boundary, word_prefix, word_suffix, line_start, line_end);
+  if (m->multi) {
+    const int rc = m->multi->count_host(haystack, size, f, counts, total);
+    if (rc == 0 && m->stats) m->multi->collect_stats(m->stats);
+    return rc;
+  }
+  const int rc = m->engine->count_host(haystack, size, f, counts, total);
+  if (rc == 0 && m->stats) m->engine->collect_stats(m->stats);
+  return rc;
+}
+
+int olm_cuda_count_patterns_device(const omega_list_matcher_t *m, const void *dev_haystack, size_t size,
+                                   int no_overlap, int longest_only, int word_boundary, int word_prefix,
+                                   int word_suffix, int line_start, int line_end, void *dev_counts, uint64_t *total) {
+  if (!m || !m->engine || !dev_counts || !total || load_pattern_tables(m)) return -1;
+  olm::ScanRange r;
+  r.dev = dev_haystack;
+  r.slice_begin = 0;
+  r.slice_len = size;
+  r.own_begin = 0;
+  r.own_end = size;
+  r.global_size = size;
+  r.match_ptr_base = reinterpret_cast<uint64_t>(dev_haystack);
+  olm_cuda_results_t res;
+  const int rc = m->engine->match_device(
+      r, to_flags(no_overlap, longest_only, word_boundary, word_prefix, word_suffix, line_start, line_end), &res,
+      dev_counts);
+  if (rc != 0) return rc;
+  if (m->stats) m->engine->collect_stats(m->stats);
+  *total = res.count;
+  return 0;
+}
+
+int olm_cuda_count_records(const omega_list_matcher_t *m, const void *dev_records, uint64_t count, void *dev_counts) {
+  if (!m || !m->engine || !dev_counts || (count && !dev_records) || load_pattern_tables(m)) return -1;
+  return m->engine->count_records(dev_records, count, dev_counts);
+}
+
 int olm_cuda_last_timing(const omega_list_matcher_t *m, olm_cuda_timing_t *out) {
   if (!m || !m->engine || !out) return -1;
   *out = m->multi ? m->multi->timing() : m->engine->timing();

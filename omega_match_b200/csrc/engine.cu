@@ -148,6 +148,11 @@ struct EngineImpl {
   bool want_ids = false;
   PatternIdTables ids;
   DevBuf d_id_table, d_id_refs, d_id_short;
+  // pattern counts of the host path: device scratch, zeroed per call, and its pinned host copy
+  DevBuf d_counts;
+  uint64_t *h_counts = nullptr;
+  size_t h_counts_cap = 0;
+  int count_table = -1; // OLM_COUNT_TABLE=0 / 1 (include/olm_b200.h): forces a counting histogram
 };
 
 namespace {
@@ -172,6 +177,9 @@ int wait_segment(EngineImpl &E, size_t idx) {
   }
   E.seg_waited = std::max(E.seg_waited, idx + 1);
   return 0;
+}
+bool count_block_table(const EngineImpl &E, uint64_t n) {
+  return E.count_table >= 0 ? E.count_table != 0 : pattern_counts_block_table(n, E.ids);
 }
 } // namespace
 
@@ -229,6 +237,7 @@ Engine *Engine::create(const uint8_t *file, size_t size, int device, std::string
     const unsigned long long v = std::strtoull(sp, nullptr, 10);
     impl->host_span = (v + kWindowBytes - 1) / kWindowBytes * kWindowBytes; // whole 4 MiB windows
   }
+  if (const char *ct = std::getenv("OLM_COUNT_TABLE")) impl->count_table = std::atoi(ct) != 0;
   {
     StagedStats ss;
     e = stage_stats(view, &ss);
@@ -286,8 +295,9 @@ Engine::~Engine() {
   for (DevBuf *b : {&impl_->d_keys, &impl_->d_slots, &impl_->d_recs, &impl_->d_store, &impl_->d_g4, &impl_->d_p23, &impl_->d_sx, &impl_->d_set3,
                     &impl_->d_bitmap2, &impl_->hay, &impl_->out, &impl_->out2, &impl_->chunk_desc, &impl_->span_base, &impl_->temp, &impl_->tfblocks, &impl_->tfvisible, &impl_->tfplan, &impl_->tfextent, &impl_->misc,
                     &impl_->windows, &impl_->gather, &impl_->text, &impl_->ghost, &impl_->fscratch, &impl_->d_bloom, &impl_->d_smap,
-                    &impl_->d_slens, &impl_->d_id_table, &impl_->d_id_refs, &impl_->d_id_short})
+                    &impl_->d_slens, &impl_->d_id_table, &impl_->d_id_refs, &impl_->d_id_short, &impl_->d_counts})
     b->release();
+  if (impl_->h_counts) cudaFreeHost(impl_->h_counts);
   for (auto &ev : impl_->ev)
     if (ev) cudaEventDestroy(ev);
   for (auto &ev : impl_->seg_events) cudaEventDestroy(ev);
@@ -302,7 +312,7 @@ int Engine::device() const { return impl_->device; }
 const Header &Engine::header() const { return impl_->hdr; }
 const olm_cuda_timing_t &Engine::timing() const { return impl_->last; }
 
-int Engine::match_device(const ScanRange &r, const MatchFlags &f, olm_cuda_results_t *res) {
+int Engine::match_device(const ScanRange &r, const MatchFlags &f, olm_cuda_results_t *res, void *dev_counts) {
   EngineImpl &E = *impl_;
   OLM_CUDA(cudaSetDevice(E.device));
   // device-resident input may have been produced on any stream of the caller
@@ -555,7 +565,7 @@ int Engine::match_device(const ScanRange &r, const MatchFlags &f, olm_cuda_resul
     std::swap(E.out, E.out2);
     final_records = E.out.p;
   }
-  if (E.want_ids && total) {
+  if ((E.want_ids || dev_counts) && total) {
     unsigned long long *d_missing = d_total + 16; // (misc words 16.. are not cleared with the scan's)
     unsigned long long missing = 0;
     uint32_t launches = 0;
@@ -563,8 +573,13 @@ int Engine::match_device(const ScanRange &r, const MatchFlags &f, olm_cuda_resul
     if (E.streaming && !E.seg_events.empty() && wait_segment(E, E.seg_events.size() - 1)) return -1;
     OLM_CUDA(cudaMemsetAsync(d_missing, 0, sizeof missing, E.stream));
     OLM_CUDA(cudaEventRecord(E.ev[2], E.stream));
-    OLM_CUDA(pattern_ids_launch(static_cast<Record *>(final_records), total, static_cast<const uint8_t *>(r.dev),
-                                r.slice_begin, E.ids, d_missing, E.sms, E.stream, &launches));
+    if (dev_counts) // instead of the ids: the count of the records per pattern
+      OLM_CUDA(pattern_counts_launch(static_cast<const Record *>(final_records), total, static_cast<const uint8_t *>(r.dev),
+                                     r.slice_begin, E.ids, count_block_table(E, total),
+                                     static_cast<unsigned long long *>(dev_counts), d_missing, E.sms, E.stream, &launches));
+    else
+      OLM_CUDA(pattern_ids_launch(static_cast<Record *>(final_records), total, static_cast<const uint8_t *>(r.dev),
+                                  r.slice_begin, E.ids, d_missing, E.sms, E.stream, &launches));
     OLM_CUDA(cudaEventRecord(E.ev[3], E.stream));
     OLM_CUDA(cudaMemcpyAsync(&missing, d_missing, sizeof missing, cudaMemcpyDeviceToHost, E.stream));
     OLM_CUDA(cudaStreamSynchronize(E.stream));
@@ -709,7 +724,7 @@ struct StreamingScope { // the device-resident entry points never see segments
 // One rank's byte range from HOST memory: the slice is copied in segments while the scan of the
 // earlier segments runs; the records stay on the device (like match_device with a shard range).
 int Engine::match_shard_host(const uint8_t *host_slice, const ScanRange &range, const MatchFlags &f,
-                             olm_cuda_results_t *out) {
+                             olm_cuda_results_t *out, void *dev_counts) {
   EngineImpl &E = *impl_;
   OLM_CUDA(cudaSetDevice(E.device));
   if (!host_slice || range.slice_len == 0) return -1;
@@ -717,7 +732,7 @@ int Engine::match_shard_host(const uint8_t *host_slice, const ScanRange &range, 
   StreamingScope scope(E);
   ScanRange r = range;
   r.dev = E.hay.p;
-  const int rc = match_device(r, f, out);
+  const int rc = match_device(r, f, out, dev_counts);
   if (finish_staging() != 0 || rc != 0) return -1;
   float ms = 0.f;
   OLM_CUDA(cudaStreamSynchronize(E.copy_stream));
@@ -931,22 +946,187 @@ int Engine::sync() {
 
 void Engine::set_exact_stats(bool on) { impl_->want_stats = on; }
 
-int Engine::set_pattern_ids(bool on, const PatternCatalog *cat) {
+int Engine::load_pattern_tables(const PatternCatalog *cat) {
   EngineImpl &E = *impl_;
-  if (on && !E.ids.table) {
-    if (!cat) return -1;
-    OLM_CUDA(cudaSetDevice(E.device));
-    PatternIdTables t;
-    if (upload(E.d_id_table, cat->table, &t.table) || upload(E.d_id_refs, cat->refs, &t.refs) ||
-        upload(E.d_id_short, cat->short_bytes, &t.short_bytes))
-      return -1;
-    t.table_mask = cat->table_mask;
-    t.store = E.ds.store;
-    t.store_flags = E.hdr.flags;
-    E.ids = t;
-  }
-  E.want_ids = on;
+  if (E.ids.table) return 0;
+  if (!cat) return -1;
+  OLM_CUDA(cudaSetDevice(E.device));
+  PatternIdTables t;
+  if (upload(E.d_id_table, cat->table, &t.table) || upload(E.d_id_refs, cat->refs, &t.refs) ||
+      upload(E.d_id_short, cat->short_bytes, &t.short_bytes))
+    return -1;
+  t.table_mask = cat->table_mask;
+  t.store = E.ds.store;
+  t.store_flags = E.hdr.flags;
+  t.count = uint32_t(cat->size());
+  E.ids = t;
   return 0;
+}
+
+int Engine::set_pattern_ids(bool on, const PatternCatalog *cat) {
+  if (on && load_pattern_tables(cat)) return -1;
+  impl_->want_ids = on;
+  return 0;
+}
+
+bool Engine::pattern_ids() const { return impl_->want_ids; }
+uint64_t Engine::pattern_count() const { return impl_->ids.count; }
+
+// ---- pattern counts (include/olm_b200.h): the tables are loaded (load_pattern_tables) before any
+// of these runs
+
+int Engine::count_records(const void *dev_records, uint64_t count, void *dev_counts) {
+  EngineImpl &E = *impl_;
+  OLM_CUDA(cudaSetDevice(E.device));
+  if (!E.ids.table) return -1;
+  if (count == 0) return 0;
+  OLM_CUDA(cudaDeviceSynchronize()); // see no_overlap_inplace
+  if (E.misc.ensure(size_t(kMaxBatches) * 8 + 256)) return -1;
+  unsigned long long *d_missing =
+      reinterpret_cast<unsigned long long *>(static_cast<uint8_t *>(E.misc.p) + size_t(kMaxBatches) * 8) + 16;
+  unsigned long long missing = 0;
+  uint32_t launches = 0;
+  OLM_CUDA(cudaMemsetAsync(d_missing, 0, sizeof missing, E.stream));
+  OLM_CUDA(pattern_counts_launch(static_cast<const Record *>(dev_records), count, nullptr, 0, E.ids,
+                                 count_block_table(E, count), static_cast<unsigned long long *>(dev_counts), d_missing,
+                                 E.sms, E.stream, &launches));
+  OLM_CUDA(cudaMemcpyAsync(&missing, d_missing, sizeof missing, cudaMemcpyDeviceToHost, E.stream));
+  OLM_CUDA(cudaStreamSynchronize(E.stream));
+  if (missing) {
+    std::fprintf(stderr, "libomega_match(b200): %llu records hold no pattern id of the catalogue (%u patterns)\n",
+                 missing, E.ids.count);
+    return -1;
+  }
+  return 0;
+}
+
+// the device scratch counts of the host path, zeroed on the stream
+unsigned long long *Engine::zeroed_counts() {
+  EngineImpl &E = *impl_;
+  const size_t bytes = std::max<size_t>(1, E.ids.count) * sizeof(uint64_t);
+  if (E.d_counts.ensure(bytes) || cudaMemsetAsync(E.d_counts.p, 0, bytes, E.stream) != cudaSuccess) return nullptr;
+  return static_cast<unsigned long long *>(E.d_counts.p);
+}
+
+// counts[] += the device scratch counts: one D2H of 8 bytes per pattern (d2h_ms)
+int Engine::add_counts_to_host(uint64_t *counts) {
+  EngineImpl &E = *impl_;
+  const size_t n = E.ids.count;
+  if (E.h_counts_cap < n) {
+    if (E.h_counts) cudaFreeHost(E.h_counts);
+    E.h_counts = nullptr;
+    E.h_counts_cap = 0;
+    OLM_CUDA(cudaHostAlloc(&E.h_counts, n * sizeof(uint64_t), cudaHostAllocDefault));
+    E.h_counts_cap = n;
+  }
+  float ms = 0.f;
+  OLM_CUDA(cudaEventRecord(E.ev[6], E.stream));
+  OLM_CUDA(cudaMemcpyAsync(E.h_counts, E.d_counts.p, n * sizeof(uint64_t), cudaMemcpyDeviceToHost, E.stream));
+  OLM_CUDA(cudaEventRecord(E.ev[7], E.stream));
+  OLM_CUDA(cudaStreamSynchronize(E.stream));
+  cudaEventElapsedTime(&ms, E.ev[6], E.ev[7]);
+  E.last.d2h_ms = ms;
+  for (size_t i = 0; i < n; ++i) counts[i] += E.h_counts[i];
+  return 0;
+}
+
+int Engine::count_shard_host(const uint8_t *host_slice, const ScanRange &range, const MatchFlags &f, uint64_t *counts,
+                             uint64_t *total) {
+  EngineImpl &E = *impl_;
+  OLM_CUDA(cudaSetDevice(E.device));
+  unsigned long long *d = zeroed_counts();
+  olm_cuda_results_t res;
+  if (!d || match_shard_host(host_slice, range, f, &res, d) != 0 || add_counts_to_host(counts) != 0) return -1;
+  *total = res.count;
+  return 0;
+}
+
+int Engine::count_host(const uint8_t *haystack, size_t n, const MatchFlags &f, uint64_t *counts, uint64_t *total) {
+  EngineImpl &E = *impl_;
+  *total = 0;
+  if (E.host_span && haystack && n > E.host_span) return count_host_spans(haystack, n, f, E.host_span, counts, total);
+  if (n == 0 || !haystack) { // (as match_host)
+    std::memset(E.counters, 0, sizeof E.counters);
+    std::memset(E.stat_counters, 0, sizeof E.stat_counters);
+    E.attempts_last = 0;
+    E.stats_valid = false;
+    E.last = olm_cuda_timing_t{};
+    return 0;
+  }
+  ScanRange r;
+  r.slice_begin = 0;
+  r.slice_len = n;
+  r.own_begin = 0;
+  r.own_end = n;
+  r.global_size = n;
+  r.match_ptr_base = reinterpret_cast<uint64_t>(haystack);
+  return count_shard_host(haystack, r, f, counts, total);
+}
+
+// match_host_spans() counting.  Without no_overlap every span counts on the device into one scratch
+// array; with it the spans write ids (their haystacks are gone when the filter runs), their records
+// are concatenated on the device, filtered once, and counted from the pads.
+int Engine::count_host_spans(const uint8_t *haystack, size_t n, const MatchFlags &f, uint64_t span, uint64_t *counts,
+                             uint64_t *total) {
+  EngineImpl &E = *impl_;
+  OLM_CUDA(cudaSetDevice(E.device));
+  const bool windowed = E.hdr.flags & kFlagAnyTransform;
+  const bool filter = f.no_overlap;
+  MatchFlags fs = f;
+  fs.no_overlap = false;
+  unsigned long long *d = zeroed_counts();
+  if (!d) return -1;
+  const bool ids_were = E.want_ids;
+  E.want_ids = filter;
+  uint64_t all = 0; // records concatenated in E.gather (no_overlap)
+  E.span_acc = omega_match_stats_t{};
+  int rc = 0;
+  for (uint64_t b = 0; b < n && rc == 0; b += span) {
+    const uint64_t e = std::min<uint64_t>(n, b + span);
+    ScanRange r;
+    r.own_begin = b;
+    r.own_end = e;
+    r.global_size = n;
+    r.match_ptr_base = reinterpret_cast<uint64_t>(haystack);
+    r.slice_begin = (windowed || b < 16) ? b : b - 16; // (b is a multiple of 4 MiB)
+    r.slice_len = (windowed ? e : std::min<uint64_t>(n, e + E.hdr.largest + 1)) - r.slice_begin;
+    olm_cuda_results_t res;
+    rc = match_shard_host(haystack + r.slice_begin, r, fs, &res, filter ? nullptr : d);
+    if (rc == 0 && filter && res.count) {
+      // grown geometrically (each growth copies what is there; it is not ordered after the stream's copies)
+      const size_t need = (all + res.count) * sizeof(Record);
+      if (need > E.gather.cap)
+        rc = cudaStreamSynchronize(E.stream) == cudaSuccess ? E.gather.ensure(std::max(need, 2 * E.gather.cap), true) : -1;
+      if (rc == 0 && cudaMemcpyAsync(static_cast<Record *>(E.gather.p) + all, res.records, res.count * sizeof(Record),
+                                     cudaMemcpyDeviceToDevice, E.stream) != cudaSuccess)
+        rc = -1;
+    }
+    all += res.count;
+    if (rc == 0 && e < n) { // (as match_host_spans)
+      omega_match_stats_t acc = E.span_acc;
+      E.span_acc = omega_match_stats_t{};
+      collect_stats(&acc);
+      E.span_acc = acc;
+    }
+  }
+  E.want_ids = ids_were;
+  if (rc != 0) return -1;
+  if (filter && all) {
+    const int64_t kept = no_overlap_inplace(E.gather.p, all);
+    if (kept < 0) return -1;
+    all = uint64_t(kept);
+    return count_records_to_host(E.gather.p, all, counts) != 0 ? -1 : (*total = all, 0);
+  }
+  if (add_counts_to_host(counts) != 0) return -1;
+  *total = all;
+  return 0;
+}
+
+int Engine::count_records_to_host(const void *dev_records, uint64_t count, uint64_t *counts) {
+  OLM_CUDA(cudaSetDevice(impl_->device));
+  unsigned long long *d = zeroed_counts();
+  if (!d || count_records(dev_records, count, d) != 0) return -1;
+  return add_counts_to_host(counts);
 }
 
 void Engine::collect_stats(omega_match_stats_t *s) {

@@ -41,13 +41,16 @@ public:
   int device() const;
   const Header &header() const;
 
-  // Device-resident input, device-resident output (records stay in the engine's buffer).
-  int match_device(const ScanRange &r, const MatchFlags &f, olm_cuda_results_t *out);
+  // Device-resident input, device-resident output (records stay in the engine's buffer).  With
+  // `dev_counts` (the pattern tables loaded: load_pattern_tables) the call adds the count of its
+  // final records per pattern to dev_counts[id] instead of writing ids, whether ids are on or off.
+  int match_device(const ScanRange &r, const MatchFlags &f, olm_cuda_results_t *out, void *dev_counts = nullptr);
   // Host input/output: H2D, match_device, D2H into a malloc'ed array.
   omega_match_results_t *match_host(const uint8_t *haystack, size_t n, const MatchFlags &f);
   // A byte range (range.dev is ignored) whose slice lies in HOST memory: segmented H2D overlapped
   // with the scan, device-resident records.
-  int match_shard_host(const uint8_t *host_slice, const ScanRange &range, const MatchFlags &f, olm_cuda_results_t *out);
+  int match_shard_host(const uint8_t *host_slice, const ScanRange &range, const MatchFlags &f, olm_cuda_results_t *out,
+                       void *dev_counts = nullptr);
 
   // "offset:bytes\n" for every record (the CLI's listing, main.c:89-133) as one device text buffer;
   // dev_haystack = device address of the haystack byte with offset `offset0`
@@ -75,6 +78,20 @@ public:
   // (pattern_ids.cuh); off (default): the pad stays 0.  The first switch on uploads the catalogue's
   // lookup table (`cat`, the catalogue of this engine's store; not needed to switch off).
   int set_pattern_ids(bool on, const PatternCatalog *cat);
+  bool pattern_ids() const;
+  // Uploads the catalogue's lookup table once (set_pattern_ids does when switching on; the counts
+  // need it without switching ids on).  0 when it is there already.
+  int load_pattern_tables(const PatternCatalog *cat);
+  uint64_t pattern_count() const; // of the loaded tables
+
+  // Pattern counts (include/olm_b200.h): counts[id] += the final records of pattern id, *total = their
+  // number; the records stay on the device.  Host counts: one device scratch array per call, copied
+  // back once.  count_records reads ids from the records' pads (-1 for an id out of range).
+  int count_host(const uint8_t *haystack, size_t n, const MatchFlags &f, uint64_t *counts, uint64_t *total);
+  int count_shard_host(const uint8_t *host_slice, const ScanRange &range, const MatchFlags &f, uint64_t *counts,
+                       uint64_t *total);
+  int count_records(const void *dev_records, uint64_t count, void *dev_counts);
+  int count_records_to_host(const void *dev_records, uint64_t count, uint64_t *counts); // counts[id] += ...
 
 private:
   Engine() = default;
@@ -82,6 +99,10 @@ private:
   int stage_pageable(const uint8_t *src, size_t n, uint64_t nseg);
   int finish_staging();
   omega_match_results_t *match_host_spans(const uint8_t *haystack, size_t n, const MatchFlags &f, uint64_t span);
+  int count_host_spans(const uint8_t *haystack, size_t n, const MatchFlags &f, uint64_t span, uint64_t *counts,
+                       uint64_t *total);
+  unsigned long long *zeroed_counts();
+  int add_counts_to_host(uint64_t *counts);
   EngineImpl *impl_ = nullptr;
 };
 

@@ -23,6 +23,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <functional>
 #include <string>
 #include <thread>
 #include <vector>
@@ -199,8 +200,6 @@ omega_match_results_t *MultiMatcher::match_host(const uint8_t *haystack, size_t 
     std::free(results);
     return nullptr;
   };
-  const Header &h = engines_[0]->header();
-  const bool windowed = h.flags & kFlagAnyTransform;
   // The stale-tail bytes of SURVEY H6 (2..4 byte patterns of a transforming store under word_boundary)
   // depend on the windows in front of a window -- which a shard does not see.  Such calls run on the
   // first GPU alone; all other calls shard, and afterwards every engine gets the scratch-buffer image
@@ -215,52 +214,19 @@ omega_match_results_t *MultiMatcher::match_host(const uint8_t *haystack, size_t 
     if (r) sync_ghost(0);
     return r;
   }
-  const std::vector<Shard> plan = plan_shards(n, N, h.largest, windowed);
   MatchFlags fs = f;
   fs.no_overlap = false; // crosses shards: once, on the gathered records
   std::vector<olm_cuda_results_t> res(N);
-  std::vector<int> rc(N, 0);
-  {
-    std::vector<std::thread> th;
-    for (int g = 0; g < N; ++g) {
-      res[g] = olm_cuda_results_t{0, nullptr, engines_[g]->device()};
-      const Shard &s = plan[g];
-      if (s.own_end <= s.own_begin) continue;
-      scanned_[g] = true;
-      th.emplace_back([&, g]() {
-        const Shard &sh = plan[g];
-        ScanRange r;
-        r.slice_begin = sh.slice_begin;
-        r.slice_len = sh.slice_end - sh.slice_begin;
-        r.own_begin = sh.own_begin;
-        r.own_end = sh.own_end;
-        r.global_size = n;
-        r.match_ptr_base = reinterpret_cast<uint64_t>(haystack);
-        rc[g] = engines_[g]->match_shard_host(haystack + sh.slice_begin, r, fs, &res[g]);
-      });
-    }
-    for (auto &t : th) t.join();
-  }
+  for (int g = 0; g < N; ++g) res[g] = olm_cuda_results_t{0, nullptr, engines_[g]->device()};
+  if (run_shards(haystack, n, [&](int g, const uint8_t *slice, const ScanRange &r) {
+        return engines_[g]->match_shard_host(slice, r, fs, &res[g]);
+      }) != 0)
+    return bail();
   uint64_t total = 0;
   std::vector<uint64_t> off(N, 0);
   for (int g = 0; g < N; ++g) {
-    if (rc[g] != 0) return bail();
     off[g] = total;
     total += res[g].count;
-    const olm_cuda_timing_t &t = engines_[g]->timing();
-    last_.scan_ms = std::max(last_.scan_ms, t.scan_ms);
-    last_.transform_ms = std::max(last_.transform_ms, t.transform_ms);
-    last_.total_ms = std::max(last_.total_ms, t.total_ms);
-    last_.h2d_ms = std::max(last_.h2d_ms, t.h2d_ms);
-    last_.scan_launches += t.scan_launches;
-    last_.kernel_launches += t.kernel_launches;
-    last_.matches_before_filter += t.matches_before_filter;
-  }
-  if (tails) {
-    int last = 0;
-    for (int g = 0; g < N; ++g)
-      if (scanned_[g]) last = g;
-    sync_ghost(last);
   }
   if (total == 0) return results;
 
@@ -268,20 +234,9 @@ omega_match_results_t *MultiMatcher::match_host(const uint8_t *haystack, size_t 
   const void *src0 = nullptr; // records that leave through the first GPU (no_overlap)
   uint64_t kept = total;
   if (f.no_overlap && total > 1) {
-    void *buf = E0->gather_buffer(total * sizeof(Record));
-    if (!buf) return bail();
-    cudaStream_t s0 = static_cast<cudaStream_t>(E0->stream());
-    for (int g = 0; g < N; ++g)
-      if (res[g].count &&
-          cudaMemcpyPeerAsync(static_cast<uint8_t *>(buf) + off[g] * sizeof(Record), E0->device(), res[g].records,
-                              engines_[g]->device(), res[g].count * sizeof(Record), s0) != cudaSuccess)
-        return bail();
-    if (cudaStreamSynchronize(s0) != cudaSuccess) return bail();
-    const int64_t k = E0->no_overlap_inplace(buf, total);
+    const int64_t k = gather_no_overlap(res, total, &src0);
     if (k < 0) return bail();
     kept = (uint64_t)k;
-    last_.filter_ms = E0->timing().filter_ms;
-    src0 = buf;
   }
   std::free(results->matches);
   const size_t rbytes = std::max<uint64_t>(kept, 1) * sizeof(omega_match_result_t);
@@ -317,6 +272,138 @@ omega_match_results_t *MultiMatcher::match_host(const uint8_t *haystack, size_t 
   return results;
 }
 
+// Runs scan(g, slice, range) for every GPU's shard of the host haystack, one host thread per GPU,
+// then takes the call's timing from the engines and, for stores whose windows leave stale tails,
+// gives every engine the scratch-buffer image of the engine that scanned the last windows.
+int MultiMatcher::run_shards(const uint8_t *haystack, size_t n,
+                             const std::function<int(int, const uint8_t *, const ScanRange &)> &scan) {
+  const int N = (int)engines_.size();
+  const Header &h = engines_[0]->header();
+  const std::vector<Shard> plan = plan_shards(n, N, h.largest, h.flags & kFlagAnyTransform);
+  std::vector<int> rc(N, 0);
+  {
+    std::vector<std::thread> th;
+    for (int g = 0; g < N; ++g) {
+      const Shard &s = plan[g];
+      if (s.own_end <= s.own_begin) continue;
+      scanned_[g] = true;
+      th.emplace_back([&, g]() {
+        const Shard &sh = plan[g];
+        ScanRange r;
+        r.slice_begin = sh.slice_begin;
+        r.slice_len = sh.slice_end - sh.slice_begin;
+        r.own_begin = sh.own_begin;
+        r.own_end = sh.own_end;
+        r.global_size = n;
+        r.match_ptr_base = reinterpret_cast<uint64_t>(haystack);
+        rc[g] = scan(g, haystack + sh.slice_begin, r);
+      });
+    }
+    for (auto &t : th) t.join();
+  }
+  for (int g = 0; g < N; ++g) {
+    if (rc[g] != 0) return -1;
+    const olm_cuda_timing_t &t = engines_[g]->timing();
+    last_.scan_ms = std::max(last_.scan_ms, t.scan_ms);
+    last_.transform_ms = std::max(last_.transform_ms, t.transform_ms);
+    last_.total_ms = std::max(last_.total_ms, t.total_ms);
+    last_.h2d_ms = std::max(last_.h2d_ms, t.h2d_ms);
+    last_.scan_launches += t.scan_launches;
+    last_.kernel_launches += t.kernel_launches;
+    last_.matches_before_filter += t.matches_before_filter;
+  }
+  if (engines_[0]->needs_window_tails()) {
+    int last = 0;
+    for (int g = 0; g < N; ++g)
+      if (scanned_[g]) last = g;
+    sync_ghost(last);
+  }
+  return 0;
+}
+
+// The shards' records (res, `total` in all) gathered on the first GPU over NVLink in shard order, and
+// no_overlap applied there; returns the number kept (*dst: where they are), -1 on failure.
+int64_t MultiMatcher::gather_no_overlap(const std::vector<olm_cuda_results_t> &res, uint64_t total, const void **dst) {
+  Engine *E0 = engines_[0];
+  void *buf = E0->gather_buffer(total * sizeof(Record));
+  if (!buf) return -1;
+  cudaStream_t s0 = static_cast<cudaStream_t>(E0->stream());
+  uint64_t off = 0;
+  for (size_t g = 0; g < res.size(); off += res[g].count, ++g)
+    if (res[g].count &&
+        cudaMemcpyPeerAsync(static_cast<uint8_t *>(buf) + off * sizeof(Record), E0->device(), res[g].records,
+                            engines_[g]->device(), res[g].count * sizeof(Record), s0) != cudaSuccess)
+      return -1;
+  if (cudaStreamSynchronize(s0) != cudaSuccess) return -1;
+  const int64_t k = E0->no_overlap_inplace(buf, total);
+  last_.filter_ms = E0->timing().filter_ms;
+  *dst = buf;
+  return k;
+}
+
+// match_host() counting (include/olm_b200.h olm_cuda_count_patterns).  Without no_overlap every GPU
+// counts its shard and the counts are summed on the host: no record moves.  With it the shards write
+// ids, the gather and the filter run as in match_host, and the first GPU counts the pads.
+int MultiMatcher::count_host(const uint8_t *haystack, size_t n, const MatchFlags &f, uint64_t *counts, uint64_t *total) {
+  const int N = (int)engines_.size();
+  last_ = olm_cuda_timing_t{};
+  scanned_.assign(N, false);
+  *total = 0;
+  if (n == 0 || !haystack) return 0;
+  if (engines_[0]->needs_window_tails() && f.word_boundary) { // (as match_host)
+    scanned_[0] = true;
+    const int rc = engines_[0]->count_host(haystack, n, f, counts, total);
+    last_ = engines_[0]->timing();
+    if (rc == 0) sync_ghost(0);
+    return rc;
+  }
+  MatchFlags fs = f;
+  fs.no_overlap = false;
+  const uint64_t P = engines_[0]->pattern_count();
+  if (!f.no_overlap) {
+    std::vector<std::vector<uint64_t>> part(N);
+    std::vector<uint64_t> tot(N, 0);
+    if (run_shards(haystack, n, [&](int g, const uint8_t *slice, const ScanRange &r) {
+          part[g].assign(P, 0);
+          return engines_[g]->count_shard_host(slice, r, fs, part[g].data(), &tot[g]);
+        }) != 0)
+      return -1;
+    for (int g = 0; g < N; ++g) {
+      if (!scanned_[g]) continue;
+      for (uint64_t i = 0; i < P; ++i) counts[i] += part[g][i];
+      *total += tot[g];
+      last_.d2h_ms = std::max(last_.d2h_ms, engines_[g]->timing().d2h_ms);
+    }
+    return 0;
+  }
+  std::vector<olm_cuda_results_t> res(N);
+  std::vector<bool> ids_were(N);
+  for (int g = 0; g < N; ++g) {
+    res[g] = olm_cuda_results_t{0, nullptr, engines_[g]->device()};
+    ids_were[g] = engines_[g]->pattern_ids();
+    engines_[g]->set_pattern_ids(true, nullptr); // (the tables are loaded)
+  }
+  int rc = run_shards(haystack, n, [&](int g, const uint8_t *slice, const ScanRange &r) {
+    return engines_[g]->match_shard_host(slice, r, fs, &res[g]);
+  });
+  for (int g = 0; g < N; ++g) engines_[g]->set_pattern_ids(ids_were[g], nullptr);
+  if (rc != 0) return -1;
+  uint64_t all = 0;
+  for (const olm_cuda_results_t &r : res) all += r.count;
+  if (all > 1) {
+    const void *recs = nullptr;
+    const int64_t k = gather_no_overlap(res, all, &recs);
+    if (k < 0 || engines_[0]->count_records_to_host(recs, uint64_t(k), counts) != 0) return -1;
+    all = uint64_t(k);
+    last_.d2h_ms = engines_[0]->timing().d2h_ms;
+  } else {
+    for (int g = 0; g < N; ++g) // (one record at most: nothing to filter)
+      if (res[g].count && engines_[g]->count_records_to_host(res[g].records, res[g].count, counts) != 0) return -1;
+  }
+  *total = all;
+  return 0;
+}
+
 // every engine's image of the reference's scratch buffer <- the one of engine `from`
 void MultiMatcher::sync_ghost(int from) {
   Engine *src = engines_[size_t(from)];
@@ -340,6 +427,11 @@ void MultiMatcher::set_exact_stats(bool on) {
 int MultiMatcher::set_pattern_ids(bool on, const PatternCatalog *cat) {
   for (Engine *e : engines_)
     if (e->set_pattern_ids(on, cat) != 0) return -1;
+  return 0;
+}
+int MultiMatcher::load_pattern_tables(const PatternCatalog *cat) {
+  for (Engine *e : engines_)
+    if (e->load_pattern_tables(cat) != 0) return -1;
   return 0;
 }
 

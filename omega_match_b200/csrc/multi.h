@@ -3,6 +3,7 @@
 #pragma once
 #include <cstddef>
 #include <cstdint>
+#include <functional>
 #include <string>
 #include <vector>
 
@@ -27,15 +28,20 @@ public:
   static MultiMatcher *create(const uint8_t *file, size_t size, const std::vector<int> &devices, std::string *err);
   ~MultiMatcher();
   omega_match_results_t *match_host(const uint8_t *haystack, size_t n, const MatchFlags &f);
+  // Engine::count_host over the GPUs (the pattern tables loaded on every engine)
+  int count_host(const uint8_t *haystack, size_t n, const MatchFlags &f, uint64_t *counts, uint64_t *total);
   void collect_stats(omega_match_stats_t *accum);
   void set_exact_stats(bool on);
   int set_pattern_ids(bool on, const PatternCatalog *cat); // every engine (Engine::set_pattern_ids)
+  int load_pattern_tables(const PatternCatalog *cat);      // every engine
   const olm_cuda_timing_t &timing() const { return last_; }
   Engine *first() const { return engines_.front(); }
   int size() const { return (int)engines_.size(); }
 
 private:
   void sync_ghost(int from);
+  int run_shards(const uint8_t *haystack, size_t n, const std::function<int(int, const uint8_t *, const ScanRange &)> &scan);
+  int64_t gather_no_overlap(const std::vector<olm_cuda_results_t> &res, uint64_t total, const void **dst);
   std::vector<Engine *> engines_;
   std::vector<bool> scanned_; // engines that took part in the last call
   olm_cuda_timing_t last_{};

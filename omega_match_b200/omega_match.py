@@ -9,7 +9,8 @@ omega_match_b200/lib/libomega_match.so (see INTEGRATION.md).
 Additions (not in the reference): `Matcher.match_arrays` (numpy result without per-match
 Python objects), `Matcher.match_device` / `match_shard` (device-resident haystack and
 results), `Matcher.last_timing`, pattern ids (`Matcher.match_ids`, `set_pattern_ids`,
-`pattern_count`, `pattern`).
+`pattern_count`, `pattern`), pattern counts (`Matcher.pattern_counts`, `pattern_counts_device`,
+`count_records_device`).
 """
 from __future__ import annotations
 
@@ -85,6 +86,15 @@ def _flag_ints(kw) -> List[int]:
     if bad:
         raise TypeError(f"unexpected match options: {sorted(bad)}")
     return [int(bool(kw.get(n, False))) for n in FLAG_NAMES]
+
+
+def _host_haystack(haystack):
+    """(object that keeps the bytes alive, address, size) of a bytes-like or numpy haystack."""
+    if isinstance(haystack, np.ndarray):
+        hay = np.ascontiguousarray(haystack, dtype=np.uint8)
+        return hay, hay.ctypes.data, hay.size
+    hay = (C.c_char * len(haystack)).from_buffer_copy(haystack) if len(haystack) else None
+    return hay, (C.addressof(hay) if hay is not None else None), len(haystack)
 
 
 class Compiler:
@@ -230,12 +240,7 @@ class Matcher:
     # -- additions -------------------------------------------------------------------------
     def _match_records(self, haystack, **kw) -> np.ndarray:
         """omega_list_matcher_match() on a host buffer -> copy of the 24-byte records."""
-        if isinstance(haystack, np.ndarray):
-            hay = np.ascontiguousarray(haystack, dtype=np.uint8)
-            ptr, n = hay.ctypes.data, hay.size
-        else:
-            hay = (C.c_char * len(haystack)).from_buffer_copy(haystack) if len(haystack) else None
-            ptr, n = (C.addressof(hay) if hay is not None else None), len(haystack)
+        hay, ptr, n = _host_haystack(haystack)
         res = self._lib.omega_list_matcher_match(self._matcher, ptr, n, *_flag_ints(kw))
         if not res:
             raise RuntimeError("omega_list_matcher_match failed (CUDA error, see stderr)")
@@ -295,6 +300,34 @@ class Matcher:
         out["len"] = rec["len"]
         out["pattern_id"] = rec["_pad"]
         return out
+
+    # -- pattern counts (include/olm_b200.h) ---------------------------------------------------
+    def pattern_counts(self, haystack, **kw) -> np.ndarray:
+        """How often each pattern occurs in a host haystack: uint64 array of pattern_count entries,
+        counts[id] = the records of pattern id that match() with the same options would return.
+        Only the counts leave the GPU; the ids setting is left as it is."""
+        hay, ptr, n = _host_haystack(haystack)
+        counts = np.zeros(self.pattern_count, dtype=np.uint64)
+        total = C.c_uint64()
+        if self._lib.olm_cuda_count_patterns(self._matcher, ptr, n, *_flag_ints(kw), counts.ctypes.data,
+                                             C.byref(total)) != 0:
+            raise RuntimeError("olm_cuda_count_patterns failed (see stderr)")
+        return counts
+
+    def pattern_counts_device(self, dev_ptr: int, size: int, counts_ptr: int, **kw) -> int:
+        """Device haystack (as match_device) -> counts ADDED into pattern_count uint64 words of device
+        memory at counts_ptr; returns the number of records counted."""
+        total = C.c_uint64()
+        if self._lib.olm_cuda_count_patterns_device(self._matcher, dev_ptr, size, *_flag_ints(kw), counts_ptr,
+                                                    C.byref(total)) != 0:
+            raise RuntimeError("olm_cuda_count_patterns_device failed (see stderr)")
+        return int(total.value)
+
+    def count_records_device(self, records_ptr: int, count: int, counts_ptr: int) -> None:
+        """Device records whose pad words hold ids (made with set_pattern_ids(True)) -> counts ADDED
+        into pattern_count uint64 words of device memory at counts_ptr."""
+        if self._lib.olm_cuda_count_records(self._matcher, records_ptr, count, counts_ptr) != 0:
+            raise RuntimeError("olm_cuda_count_records failed (id out of range? see stderr)")
 
     def match_device(self, dev_ptr: int, size: int, match_ptr_base: Optional[int] = None, **kw):
         """Haystack already in HBM (16-byte aligned device pointer).  Returns (count, device
