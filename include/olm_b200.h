@@ -264,7 +264,8 @@ int olm_cuda_comm_unique_id(void *id, size_t id_bytes);
 olm_cuda_comm_t *olm_cuda_comm_create(const omega_list_matcher_t *matcher, const void *id, int rank,
                                       int world);
 int olm_cuda_comm_destroy(olm_cuda_comm_t *comm);
-/* `out` is filled on the root only (device records, valid until the root's next gather). */
+/* `out` is filled on the root only (device records, valid until the root's next gather).  Records
+ * only: line positions (see "Lines" below) are not carried. */
 int olm_cuda_gather_records(olm_cuda_comm_t *comm, const void *dev_records, uint64_t count, int root,
                             int no_overlap, olm_cuda_results_t *out);
 
@@ -366,6 +367,67 @@ int olm_cuda_count_patterns_device(const omega_list_matcher_t *matcher, const vo
  * counts on the root.  An id >= olm_pattern_count() fails the call (-1). */
 int olm_cuda_count_records(const omega_list_matcher_t *matcher, const void *dev_records, uint64_t count,
                            void *dev_counts);
+
+/* Lines: on which line each match lies, and which lines match (grep -n, grep, grep -c).
+ *
+ * A line ends at a '\n' byte and at nothing else: "\r\n" is one line break whose line keeps the
+ * '\r', and a lone '\r' breaks no line -- what grep -n and wc -l count.  The anchors line_start /
+ * line_end differ here: they also accept '\r' next to a match.  For a record at offset o of a
+ * haystack h of n bytes:
+ *   line   the number of '\n' in h[0, o): 0-based, grep -n prints line + 1;
+ *   begin  one past the last '\n' before o, or 0;
+ *   end    the first '\n' at or after o, or n.  The line's bytes are h[begin, end), without its '\n'.
+ * A record belongs to the line of its first byte (a match of an elide-whitespace store can cross a
+ * '\n': it reports the line it starts on).  Offsets are source offsets for every store, as the
+ * records' are, and lines are counted on the source bytes: transform flags change nothing here.
+ * The matching lines of a call are its distinct record lines in order, each with the number of the
+ * call's final records on it (longest_only and no_overlap applied); their count is grep -c.
+ *
+ * On the GPU the newline facts of the haystack are found in 64 KiB tiles (one read) and scanned; the
+ * tiles that hold records and a '\n' are read once more to answer each record in O(1).  The passes run
+ * after the filters and the id pass, while the haystack is resident, and are part of
+ * olm_cuda_timing_t.total_ms.  Errors return -1 with a message on stderr: a record outside the given
+ * bytes, a null output, a CUDA failure. */
+typedef struct { uint64_t line, begin, end; } olm_line_pos_t;           /* per record, 24 bytes */
+typedef struct { uint64_t line, begin, end, records; } olm_line_t;      /* per matching line, 32 bytes */
+typedef struct { uint64_t newlines, first, last; } olm_newline_facts_t; /* first / last: UINT64_MAX if none */
+typedef struct { uint64_t line, begin, next_newline; } olm_line_origin_t;
+
+/* Host haystack: *results are exactly those of omega_list_matcher_match (ids included when ids are
+ * on; destroy with omega_match_results_destroy) and positions[i] is the position of record i (free
+ * with olm_lines_free).  The one-GPU path, OLM_HOST_SPAN_BYTES spans and multi-GPU matchers. */
+int olm_cuda_match_lines(const omega_list_matcher_t *matcher, const uint8_t *haystack, size_t size,
+                         int no_overlap, int longest_only, int word_boundary, int word_prefix,
+                         int word_suffix, int line_start, int line_end, omega_match_results_t **results,
+                         olm_line_pos_t **positions);
+/* Host haystack: only the matching lines leave the GPU (*lines, *n_lines of them; free with
+ * olm_lines_free); *total_records is the record count of the equivalent match call. */
+int olm_cuda_matching_lines(const omega_list_matcher_t *matcher, const uint8_t *haystack, size_t size,
+                            int no_overlap, int longest_only, int word_boundary, int word_prefix,
+                            int word_suffix, int line_start, int line_end, olm_line_t **lines,
+                            uint64_t *n_lines, uint64_t *total_records);
+void olm_lines_free(void *p);
+
+/* Device: the positions of `count` records (device, offset order, as every match call returns them)
+ * whose offsets lie in [bytes_begin, bytes_begin + bytes_len), into dev_positions (count entries).
+ * dev_bytes (16-byte aligned) is the device copy of those bytes; `origin` says what lies outside
+ * them: line = the '\n' count before bytes_begin, begin = the start of the line that holds
+ * bytes_begin, next_newline = the first '\n' at or after bytes_begin + bytes_len, or the haystack's
+ * size.  NULL: the bytes are the whole haystack (bytes_begin must be 0).  A shard of a
+ * one-process-per-GPU job passes its OWN range (its slice pointer + own_begin - slice_begin) and
+ * builds its origin from the facts of the shards before and after it (olm_cuda_newline_facts). */
+int olm_cuda_line_positions(const omega_list_matcher_t *matcher, const void *dev_records, uint64_t count,
+                            const void *dev_bytes, uint64_t bytes_begin, uint64_t bytes_len,
+                            const olm_line_origin_t *origin, void *dev_positions);
+/* The '\n' count, first and last '\n' of the device bytes [0, len) (positions relative to dev_bytes). */
+int olm_cuda_newline_facts(const omega_list_matcher_t *matcher, const void *dev_bytes, uint64_t len,
+                           olm_newline_facts_t *out);
+/* The matching lines of `count` device positions (in record order): *dev_lines is device memory
+ * owned by the matcher, valid until the next call. */
+int olm_cuda_matching_lines_device(const omega_list_matcher_t *matcher, const void *dev_positions,
+                                   uint64_t count, void **dev_lines, uint64_t *n_lines);
+/* olm_cuda_gather_records does not carry positions: gather the records, or compute the positions
+ * per shard and move them by the job's own means. */
 
 /* Pinned host memory helpers (so callers can hand DMA-able buffers to _match). */
 void *olm_cuda_host_alloc(size_t bytes);

@@ -52,6 +52,14 @@ class ShardC(C.Structure):
     _fields_ = [(n, C.c_uint64) for n in ("own_begin", "own_end", "slice_begin", "slice_end")]
 
 
+class NewlineFactsC(C.Structure):  # olm_newline_facts_t
+    _fields_ = [(n, C.c_uint64) for n in ("newlines", "first", "last")]
+
+
+class LineOriginC(C.Structure):  # olm_line_origin_t
+    _fields_ = [(n, C.c_uint64) for n in ("line", "begin", "next_newline")]
+
+
 class StoreInfoC(C.Structure):
     _fields_ = [(n, C.c_uint32) for n in ("flags", "smallest", "largest", "stored_patterns", "table_size",
                                          "occupied_buckets", "len1", "len2", "len3", "len4")] + [
@@ -122,6 +130,13 @@ ABI = [
     ("olm_cuda_count_patterns", _ci, [_vp, _vp, C.c_size_t] + _flags7 + [_vp, C.POINTER(C.c_uint64)]),
     ("olm_cuda_count_patterns_device", _ci, [_vp, _vp, C.c_size_t] + _flags7 + [_vp, C.POINTER(C.c_uint64)]),
     ("olm_cuda_count_records", _ci, [_vp, _vp, C.c_uint64, _vp]),
+    ("olm_cuda_match_lines", _ci, [_vp, _vp, C.c_size_t] + _flags7 + [C.POINTER(C.POINTER(MatchResultsC)), C.POINTER(_vp)]),
+    ("olm_cuda_matching_lines", _ci, [_vp, _vp, C.c_size_t] + _flags7
+     + [C.POINTER(_vp), C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
+    ("olm_lines_free", None, [_vp]),
+    ("olm_cuda_line_positions", _ci, [_vp, _vp, C.c_uint64, _vp, C.c_uint64, C.c_uint64, C.POINTER(LineOriginC), _vp]),
+    ("olm_cuda_newline_facts", _ci, [_vp, _vp, C.c_uint64, C.POINTER(NewlineFactsC)]),
+    ("olm_cuda_matching_lines_device", _ci, [_vp, _vp, C.c_uint64, C.POINTER(_vp), C.POINTER(C.c_uint64)]),
     ("olm_cuda_host_alloc", _vp, [C.c_size_t]),
     ("olm_cuda_host_free", None, [_vp]),
     ("olm_store_inspect", _ci, [_cp, C.POINTER(StoreInfoC)]),

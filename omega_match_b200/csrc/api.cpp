@@ -14,6 +14,7 @@
 #include "../../include/olm_b200.h"
 #include "engine.h"
 #include "host_util.h"
+#include "lines.cuh"
 #include "multi.h"
 #include "store.h"
 
@@ -40,6 +41,9 @@ struct omega_list_matcher_struct {
   mutable std::string catalog_err;
 };
 
+static_assert(sizeof(olm_line_pos_t) == sizeof(olm::LinePos) && sizeof(olm_line_t) == sizeof(olm::LineEntry) &&
+                  sizeof(olm_line_pos_t) == sizeof(omega_match_result_t),
+              "the line structs are lines.cuh's, and a position is as large as a record");
 static_assert(sizeof(olm_result_with_id_t) == sizeof(omega_match_result_t) &&
                   offsetof(olm_result_with_id_t, offset) == offsetof(omega_match_result_t, offset) &&
                   offsetof(olm_result_with_id_t, len) == offsetof(omega_match_result_t, len) &&
@@ -434,6 +438,94 @@ int olm_cuda_count_patterns_device(const omega_list_matcher_t *m, const void *de
 int olm_cuda_count_records(const omega_list_matcher_t *m, const void *dev_records, uint64_t count, void *dev_counts) {
   if (!m || !m->engine || !dev_counts || (count && !dev_records) || load_pattern_tables(m)) return -1;
   return m->engine->count_records(dev_records, count, dev_counts);
+}
+
+namespace {
+// olm_cuda_match_lines / olm_cuda_matching_lines: one GPU, spans or several GPUs; nothing is kept on failure
+int lines_call(const omega_list_matcher_t *m, const uint8_t *haystack, size_t size, const olm::MatchFlags &f,
+               bool lines_only, olm::LinesResult *r) {
+  const int rc = m->multi ? m->multi->lines_host(haystack, size, f, lines_only, r)
+                          : m->engine->lines_host(haystack, size, f, lines_only, r);
+  if (rc != 0) {
+    omega_match_results_destroy(r->results);
+    olm::host_result_free(r->positions);
+    olm::host_result_free(r->lines);
+    *r = olm::LinesResult{};
+    return -1;
+  }
+  if (m->stats) {
+    if (m->multi) m->multi->collect_stats(m->stats);
+    else m->engine->collect_stats(m->stats);
+  }
+  return 0;
+}
+bool null_output(const char *what) {
+  std::fprintf(stderr, "libomega_match(b200): %s: an output pointer is NULL\n", what);
+  return true;
+}
+} // namespace
+
+int olm_cuda_match_lines(const omega_list_matcher_t *m, const uint8_t *haystack, size_t size, int no_overlap,
+                         int longest_only, int word_boundary, int word_prefix, int word_suffix, int line_start,
+                         int line_end, omega_match_results_t **results, olm_line_pos_t **positions) {
+  if (!m || !m->engine || (!haystack && size)) return -1;
+  if ((!results || !positions) && null_output("olm_cuda_match_lines")) return -1;
+  *results = nullptr;
+  *positions = nullptr;
+  olm::LinesResult r;
+  if (lines_call(m, haystack, size,
+                 to_flags(no_overlap, longest_only, word_boundary, word_prefix, word_suffix, line_start, line_end), false,
+                 &r) != 0)
+    return -1;
+  *results = r.results;
+  *positions = r.positions;
+  return 0;
+}
+
+int olm_cuda_matching_lines(const omega_list_matcher_t *m, const uint8_t *haystack, size_t size, int no_overlap,
+                            int longest_only, int word_boundary, int word_prefix, int word_suffix, int line_start,
+                            int line_end, olm_line_t **lines, uint64_t *n_lines, uint64_t *total_records) {
+  if (!m || !m->engine || (!haystack && size)) return -1;
+  if ((!lines || !n_lines || !total_records) && null_output("olm_cuda_matching_lines")) return -1;
+  *lines = nullptr;
+  *n_lines = *total_records = 0;
+  olm::LinesResult r;
+  if (lines_call(m, haystack, size,
+                 to_flags(no_overlap, longest_only, word_boundary, word_prefix, word_suffix, line_start, line_end), true,
+                 &r) != 0)
+    return -1;
+  *lines = r.lines;
+  *n_lines = r.n_lines;
+  *total_records = r.total;
+  return 0;
+}
+
+void olm_lines_free(void *p) { olm::host_result_free(p); }
+
+int olm_cuda_line_positions(const omega_list_matcher_t *m, const void *dev_records, uint64_t count, const void *dev_bytes,
+                            uint64_t bytes_begin, uint64_t bytes_len, const olm_line_origin_t *origin,
+                            void *dev_positions) {
+  if (!m || !m->engine) return -1;
+  if (count && (!dev_positions || !dev_records) && null_output("olm_cuda_line_positions")) return -1;
+  if (!origin && bytes_begin != 0) {
+    std::fprintf(stderr, "libomega_match(b200): olm_cuda_line_positions: without an origin the bytes start at offset 0\n");
+    return -1;
+  }
+  const olm_line_origin_t o = origin ? *origin : olm_line_origin_t{0, 0, bytes_len};
+  return m->engine->line_positions(dev_records, count, dev_bytes, bytes_begin, bytes_len, o, dev_positions);
+}
+
+int olm_cuda_newline_facts(const omega_list_matcher_t *m, const void *dev_bytes, uint64_t len, olm_newline_facts_t *out) {
+  if (!m || !m->engine) return -1;
+  if (!out && null_output("olm_cuda_newline_facts")) return -1;
+  return m->engine->newline_facts(dev_bytes, len, out);
+}
+
+int olm_cuda_matching_lines_device(const omega_list_matcher_t *m, const void *dev_positions, uint64_t count,
+                                   void **dev_lines, uint64_t *n_lines) {
+  if (!m || !m->engine) return -1;
+  if ((!dev_lines || !n_lines || (count && !dev_positions)) && null_output("olm_cuda_matching_lines_device")) return -1;
+  return m->engine->matching_lines(dev_positions, count, dev_lines, n_lines);
 }
 
 int olm_cuda_last_timing(const omega_list_matcher_t *m, olm_cuda_timing_t *out) {

@@ -31,6 +31,7 @@
 
 #include "filters.cuh"
 #include "format.cuh"
+#include "lines.cuh"
 #include "pattern_ids.cuh"
 #include "scan.cuh"
 #include "stats.cuh"
@@ -153,6 +154,9 @@ struct EngineImpl {
   uint64_t *h_counts = nullptr;
   size_t h_counts_cap = 0;
   int count_table = -1; // OLM_COUNT_TABLE=0 / 1 (include/olm_b200.h): forces a counting histogram
+  // lines (lines.cuh): tile facts and scan, positions of a call (and compacted / gathered), matching
+  // lines and their scratch
+  DevBuf d_tiles, d_pos, d_pos2, d_pos_gather, d_lines, d_lscratch;
 };
 
 namespace {
@@ -295,7 +299,8 @@ Engine::~Engine() {
   for (DevBuf *b : {&impl_->d_keys, &impl_->d_slots, &impl_->d_recs, &impl_->d_store, &impl_->d_g4, &impl_->d_p23, &impl_->d_sx, &impl_->d_set3,
                     &impl_->d_bitmap2, &impl_->hay, &impl_->out, &impl_->out2, &impl_->chunk_desc, &impl_->span_base, &impl_->temp, &impl_->tfblocks, &impl_->tfvisible, &impl_->tfplan, &impl_->tfextent, &impl_->misc,
                     &impl_->windows, &impl_->gather, &impl_->text, &impl_->ghost, &impl_->fscratch, &impl_->d_bloom, &impl_->d_smap,
-                    &impl_->d_slens, &impl_->d_id_table, &impl_->d_id_refs, &impl_->d_id_short, &impl_->d_counts})
+                    &impl_->d_slens, &impl_->d_id_table, &impl_->d_id_refs, &impl_->d_id_short, &impl_->d_counts,
+                    &impl_->d_tiles, &impl_->d_pos, &impl_->d_pos2, &impl_->d_pos_gather, &impl_->d_lines, &impl_->d_lscratch})
     b->release();
   if (impl_->h_counts) cudaFreeHost(impl_->h_counts);
   for (auto &ev : impl_->ev)
@@ -882,7 +887,7 @@ int Engine::format_records(const void *dev_records, uint64_t count, const void *
   return 0;
 }
 
-int64_t Engine::no_overlap_inplace(void *dev_records, uint64_t count) {
+int64_t Engine::no_overlap_inplace(void *dev_records, uint64_t count, void *dev_positions) {
   EngineImpl &E = *impl_;
   OLM_CUDA(cudaSetDevice(E.device));
   if (count < 2) return (int64_t)count;
@@ -896,11 +901,15 @@ int64_t Engine::no_overlap_inplace(void *dev_records, uint64_t count) {
       reinterpret_cast<unsigned long long *>(static_cast<uint8_t *>(E.misc.p) + size_t(kMaxBatches) * 8) + 1;
   uint32_t launches = 0;
   unsigned long long total = 0;
+  if (dev_positions && E.d_pos2.ensure(count * sizeof(LinePos))) return -1;
   OLM_CUDA(no_overlap_launch(static_cast<const Record *>(dev_records), count, static_cast<Record *>(E.out2.p),
-                             E.fscratch.p, d_ftotal, E.stream, &launches));
+                             E.fscratch.p, d_ftotal, E.stream, &launches, static_cast<const LinePos *>(dev_positions),
+                             static_cast<LinePos *>(E.d_pos2.p)));
   OLM_CUDA(cudaMemcpyAsync(&total, d_ftotal, sizeof total, cudaMemcpyDeviceToHost, E.stream));
   OLM_CUDA(cudaStreamSynchronize(E.stream));
   OLM_CUDA(cudaMemcpyAsync(dev_records, E.out2.p, total * sizeof(Record), cudaMemcpyDeviceToDevice, E.stream));
+  if (dev_positions)
+    OLM_CUDA(cudaMemcpyAsync(dev_positions, E.d_pos2.p, total * sizeof(LinePos), cudaMemcpyDeviceToDevice, E.stream));
   OLM_CUDA(cudaStreamSynchronize(E.stream));
   return (int64_t)total;
 }
@@ -1127,6 +1136,276 @@ int Engine::count_records_to_host(const void *dev_records, uint64_t count, uint6
   unsigned long long *d = zeroed_counts();
   if (!d || count_records(dev_records, count, d) != 0) return -1;
   return add_counts_to_host(counts);
+}
+
+// ---- lines (lines.cuh, include/olm_b200.h "lines")
+
+void *host_result_alloc(size_t bytes) {
+  void *p = bytes >= kPinnedResultMin ? pinned_result_alloc(bytes) : nullptr;
+  return p ? p : std::malloc(std::max<size_t>(bytes, 1));
+}
+void host_result_free(void *p) {
+  if (p && !pinned_result_release(p)) std::free(p);
+}
+
+namespace {
+// the 32 words behind the batch tickets of match_device's misc buffer; the line passes use
+// [20] records outside, [21] matching lines, [24..26] newline facts
+unsigned long long *misc_words(EngineImpl &E) {
+  if (E.misc.ensure(size_t(kMaxBatches) * 8 + 256)) return nullptr;
+  return reinterpret_cast<unsigned long long *>(static_cast<uint8_t *>(E.misc.p) + size_t(kMaxBatches) * 8);
+}
+// the pass between ev[2] and ev[3] is part of the call's device time
+void add_pass_time(EngineImpl &E, uint32_t launches) {
+  float ms = 0.f;
+  cudaEventElapsedTime(&ms, E.ev[2], E.ev[3]);
+  E.last.total_ms += ms;
+  E.last.kernel_launches += launches;
+}
+bool bytes_unaligned(const void *p) {
+  if (!(reinterpret_cast<uintptr_t>(p) & 15)) return false;
+  std::fprintf(stderr, "libomega_match(b200): the device bytes of a line pass must be 16-byte aligned\n");
+  return true;
+}
+} // namespace
+
+const void *Engine::resident_haystack() const { return impl_->hay.p; }
+
+void *Engine::positions_buffer(size_t bytes, int which) {
+  DevBuf &b = which ? impl_->d_pos_gather : impl_->d_pos;
+  if (cudaSetDevice(impl_->device) != cudaSuccess || b.ensure(std::max<size_t>(bytes, 16))) return nullptr;
+  return b.p;
+}
+
+int Engine::copy_to_host(void *host_dst, const void *dev_src, size_t bytes) {
+  OLM_CUDA(cudaSetDevice(impl_->device));
+  if (bytes) OLM_CUDA(cudaMemcpyAsync(host_dst, dev_src, bytes, cudaMemcpyDeviceToHost, impl_->stream));
+  return 0;
+}
+
+int Engine::newline_facts(const void *dev_bytes, uint64_t len, olm_newline_facts_t *out) {
+  EngineImpl &E = *impl_;
+  OLM_CUDA(cudaSetDevice(E.device));
+  if (!out || (len && !dev_bytes) || bytes_unaligned(dev_bytes)) return -1;
+  OLM_CUDA(cudaDeviceSynchronize()); // the bytes may come from any stream (see no_overlap_inplace)
+  unsigned long long *w = misc_words(E);
+  if (!w || E.d_tiles.ensure(line_tiles_bytes(len))) return -1;
+  uint32_t launches = 0;
+  NewlineFacts f{};
+  OLM_CUDA(cudaEventRecord(E.ev[2], E.stream));
+  OLM_CUDA(newline_facts_launch(static_cast<const uint8_t *>(dev_bytes), len, E.d_tiles.p,
+                                reinterpret_cast<NewlineFacts *>(w + 24), E.stream, &launches));
+  OLM_CUDA(cudaEventRecord(E.ev[3], E.stream));
+  OLM_CUDA(cudaMemcpyAsync(&f, w + 24, sizeof f, cudaMemcpyDeviceToHost, E.stream));
+  OLM_CUDA(cudaStreamSynchronize(E.stream));
+  add_pass_time(E, launches);
+  *out = olm_newline_facts_t{f.newlines, f.first, f.last};
+  return 0;
+}
+
+int Engine::line_positions(const void *dev_records, uint64_t count, const void *dev_bytes, uint64_t bytes_begin,
+                           uint64_t len, const olm_line_origin_t &origin, void *dev_positions, bool tiles_ready) {
+  EngineImpl &E = *impl_;
+  OLM_CUDA(cudaSetDevice(E.device));
+  if (count == 0) return 0;
+  if (!dev_records || !dev_positions || (len && !dev_bytes) || bytes_unaligned(dev_bytes)) return -1;
+  if (!tiles_ready) {
+    olm_newline_facts_t f;
+    if (newline_facts(dev_bytes, len, &f) != 0) return -1;
+  } else {
+    OLM_CUDA(cudaDeviceSynchronize());
+  }
+  unsigned long long *w = misc_words(E);
+  if (!w) return -1;
+  uint32_t launches = 0;
+  unsigned long long outside = 0;
+  OLM_CUDA(cudaMemsetAsync(w + 20, 0, sizeof outside, E.stream));
+  OLM_CUDA(cudaEventRecord(E.ev[2], E.stream));
+  OLM_CUDA(line_positions_launch(static_cast<const Record *>(dev_records), count, static_cast<const uint8_t *>(dev_bytes),
+                                 bytes_begin, len, E.d_tiles.p, LineOrigin{origin.line, origin.begin, origin.next_newline},
+                                 static_cast<LinePos *>(dev_positions), w + 20, E.stream, &launches));
+  OLM_CUDA(cudaEventRecord(E.ev[3], E.stream));
+  OLM_CUDA(cudaMemcpyAsync(&outside, w + 20, sizeof outside, cudaMemcpyDeviceToHost, E.stream));
+  OLM_CUDA(cudaStreamSynchronize(E.stream));
+  add_pass_time(E, launches);
+  if (outside) {
+    std::fprintf(stderr, "libomega_match(b200): line positions: records outside the bytes [%llu, %llu) (or not in offset order)\n",
+                 (unsigned long long)bytes_begin, (unsigned long long)(bytes_begin + len));
+    return -1;
+  }
+  return 0;
+}
+
+int Engine::matching_lines(const void *dev_positions, uint64_t count, void **dev_lines, uint64_t *n_lines) {
+  EngineImpl &E = *impl_;
+  OLM_CUDA(cudaSetDevice(E.device));
+  if (!dev_lines || !n_lines || (count && !dev_positions)) return -1;
+  *dev_lines = nullptr;
+  *n_lines = 0;
+  OLM_CUDA(cudaDeviceSynchronize());
+  unsigned long long *w = misc_words(E);
+  if (!w || E.d_lines.ensure(std::max<uint64_t>(count, 1) * sizeof(LineEntry)) ||
+      E.d_lscratch.ensure(matching_lines_scratch_bytes(count)))
+    return -1;
+  uint32_t launches = 0;
+  unsigned long long m = 0;
+  OLM_CUDA(cudaEventRecord(E.ev[2], E.stream));
+  OLM_CUDA(matching_lines_launch(static_cast<const LinePos *>(dev_positions), count, static_cast<LineEntry *>(E.d_lines.p),
+                                 E.d_lscratch.p, w + 21, E.stream, &launches));
+  OLM_CUDA(cudaEventRecord(E.ev[3], E.stream));
+  OLM_CUDA(cudaMemcpyAsync(&m, w + 21, sizeof m, cudaMemcpyDeviceToHost, E.stream));
+  OLM_CUDA(cudaStreamSynchronize(E.stream));
+  add_pass_time(E, launches);
+  *dev_lines = E.d_lines.p;
+  *n_lines = m;
+  return 0;
+}
+
+// device records + positions -> host arrays (out->results / positions), or only their matching lines
+int Engine::lines_to_host(const void *dev_records, const void *dev_positions, uint64_t count, bool lines_only,
+                          LinesResult *out) {
+  EngineImpl &E = *impl_;
+  out->total = count;
+  void *dl = nullptr;
+  uint64_t m = 0;
+  if (lines_only && count && matching_lines(dev_positions, count, &dl, &m) != 0) return -1;
+  if (lines_only) {
+    out->lines = static_cast<olm_line_t *>(host_result_alloc(m * sizeof(olm_line_t)));
+    out->n_lines = m;
+  } else {
+    out->results = static_cast<omega_match_results_t *>(std::malloc(sizeof(omega_match_results_t)));
+    if (out->results) {
+      out->results->count = count;
+      out->results->matches = static_cast<omega_match_result_t *>(host_result_alloc(count * sizeof(omega_match_result_t)));
+    }
+    out->positions = static_cast<olm_line_pos_t *>(host_result_alloc(count * sizeof(olm_line_pos_t)));
+  }
+  if (lines_only ? !out->lines : (!out->results || !out->results->matches || !out->positions)) return -1;
+  if (lines_only ? m == 0 : count == 0) return 0;
+  float ms = 0.f;
+  OLM_CUDA(cudaEventRecord(E.ev[6], E.stream));
+  if (lines_only) {
+    OLM_CUDA(cudaMemcpyAsync(out->lines, dl, m * sizeof(olm_line_t), cudaMemcpyDeviceToHost, E.stream));
+  } else {
+    OLM_CUDA(cudaMemcpyAsync(out->results->matches, dev_records, count * sizeof(Record), cudaMemcpyDeviceToHost, E.stream));
+    OLM_CUDA(cudaMemcpyAsync(out->positions, dev_positions, count * sizeof(LinePos), cudaMemcpyDeviceToHost, E.stream));
+  }
+  OLM_CUDA(cudaEventRecord(E.ev[7], E.stream));
+  OLM_CUDA(cudaStreamSynchronize(E.stream));
+  cudaEventElapsedTime(&ms, E.ev[6], E.ev[7]);
+  E.last.d2h_ms = ms;
+  return 0;
+}
+
+int Engine::lines_host(const uint8_t *haystack, size_t n, const MatchFlags &f, bool lines_only, LinesResult *out) {
+  EngineImpl &E = *impl_;
+  *out = LinesResult{};
+  OLM_CUDA(cudaSetDevice(E.device));
+  if (E.host_span && haystack && n > E.host_span) return lines_host_spans(haystack, n, f, E.host_span, lines_only, out);
+  if (n == 0 || !haystack) { // (as match_host)
+    std::memset(E.counters, 0, sizeof E.counters);
+    std::memset(E.stat_counters, 0, sizeof E.stat_counters);
+    E.attempts_last = 0;
+    E.stats_valid = false;
+    E.last = olm_cuda_timing_t{};
+    return lines_to_host(nullptr, nullptr, 0, lines_only, out);
+  }
+  ScanRange r;
+  r.slice_begin = 0;
+  r.slice_len = n;
+  r.own_begin = 0;
+  r.own_end = n;
+  r.global_size = n;
+  r.match_ptr_base = reinterpret_cast<uint64_t>(haystack);
+  olm_cuda_results_t d;
+  if (match_shard_host(haystack, r, f, &d) != 0) return -1;
+  void *pos = nullptr;
+  if (d.count && (!(pos = positions_buffer(d.count * sizeof(LinePos), 0)) ||
+                  line_positions(d.records, d.count, E.hay.p, 0, n, olm_line_origin_t{0, 0, n}, pos) != 0))
+    return -1;
+  return lines_to_host(d.records, pos, d.count, lines_only, out);
+}
+
+// match_host_spans() with positions.  A span's line and line start carry in from the spans before it;
+// the records on its last line get their end from the first later span that holds a '\n' (or n).
+// With no_overlap, or for the matching lines, the concatenation goes back to the device.
+int Engine::lines_host_spans(const uint8_t *haystack, size_t n, const MatchFlags &f, uint64_t span, bool lines_only,
+                             LinesResult *out) {
+  EngineImpl &E = *impl_;
+  const bool windowed = E.hdr.flags & kFlagAnyTransform;
+  MatchFlags fs = f;
+  fs.no_overlap = false;
+  std::vector<Record> all;
+  std::vector<LinePos> pos;
+  uint64_t line = 0, begin = 0;
+  size_t pending = 0; // pos[pending, size()) lie on a line no span so far has ended
+  E.span_acc = omega_match_stats_t{};
+  for (uint64_t b = 0; b < n; b += span) {
+    const uint64_t e = std::min<uint64_t>(n, b + span);
+    ScanRange r;
+    r.own_begin = b;
+    r.own_end = e;
+    r.global_size = n;
+    r.match_ptr_base = reinterpret_cast<uint64_t>(haystack);
+    r.slice_begin = (windowed || b < 16) ? b : b - 16; // (b is a multiple of 4 MiB)
+    r.slice_len = (windowed ? e : std::min<uint64_t>(n, e + E.hdr.largest + 1)) - r.slice_begin;
+    olm_cuda_results_t d;
+    if (match_shard_host(haystack + r.slice_begin, r, fs, &d) != 0) return -1;
+    const uint8_t *own = static_cast<const uint8_t *>(E.hay.p) + (b - r.slice_begin);
+    olm_newline_facts_t nf;
+    if (newline_facts(own, e - b, &nf) != 0) return -1;
+    const size_t at = all.size();
+    if (d.count) {
+      void *dp = positions_buffer(d.count * sizeof(LinePos), 0);
+      if (!dp || line_positions(d.records, d.count, own, b, e - b, olm_line_origin_t{line, begin, kNoNewline}, dp, true) != 0)
+        return -1;
+      all.resize(at + d.count);
+      pos.resize(at + d.count);
+      if (copy_to_host(all.data() + at, d.records, d.count * sizeof(Record)) != 0 ||
+          copy_to_host(pos.data() + at, dp, d.count * sizeof(LinePos)) != 0 || sync() != 0)
+        return -1;
+    }
+    if (nf.newlines) {
+      for (size_t i = pending; i < at; ++i) pos[i].end = b + nf.first;
+      pending = pos.size();
+      while (pending > at && pos[pending - 1].end == kNoNewline) --pending;
+      line += nf.newlines;
+      begin = b + nf.last + 1;
+    }
+    if (e < n) { // (as match_host_spans)
+      omega_match_stats_t acc = E.span_acc;
+      E.span_acc = omega_match_stats_t{};
+      collect_stats(&acc);
+      E.span_acc = acc;
+    }
+  }
+  for (size_t i = pending; i < pos.size(); ++i) pos[i].end = n;
+  uint64_t total = all.size();
+  if ((f.no_overlap && total > 1) || (lines_only && total)) {
+    void *dp = positions_buffer(total * sizeof(LinePos), 0);
+    if (!dp || E.out.ensure(total * sizeof(Record))) return -1;
+    OLM_CUDA(cudaMemcpyAsync(E.out.p, all.data(), total * sizeof(Record), cudaMemcpyHostToDevice, E.stream));
+    OLM_CUDA(cudaMemcpyAsync(dp, pos.data(), total * sizeof(LinePos), cudaMemcpyHostToDevice, E.stream));
+    if (f.no_overlap && total > 1) {
+      const int64_t kept = no_overlap_inplace(E.out.p, total, dp);
+      if (kept < 0) return -1;
+      total = uint64_t(kept);
+    }
+    return lines_to_host(E.out.p, dp, total, lines_only, out);
+  }
+  if (lines_only) return lines_to_host(nullptr, nullptr, 0, true, out);
+  out->total = total;
+  out->results = static_cast<omega_match_results_t *>(std::malloc(sizeof(omega_match_results_t)));
+  if (!out->results) return -1;
+  out->results->count = total;
+  out->results->matches = static_cast<omega_match_result_t *>(host_result_alloc(total * sizeof(omega_match_result_t)));
+  out->positions = static_cast<olm_line_pos_t *>(host_result_alloc(total * sizeof(olm_line_pos_t)));
+  if (!out->results->matches || !out->positions) return -1;
+  if (total) {
+    std::memcpy(out->results->matches, all.data(), total * sizeof(Record));
+    std::memcpy(out->positions, pos.data(), total * sizeof(LinePos));
+  }
+  return 0;
 }
 
 void Engine::collect_stats(omega_match_stats_t *s) {

@@ -31,6 +31,17 @@ constexpr size_t kPinnedResultMin = size_t(1) << 20;
 
 struct EngineImpl;
 
+// What olm_cuda_match_lines / olm_cuda_matching_lines return.
+struct LinesResult {
+  omega_match_results_t *results = nullptr; // records (not for lines_only)
+  olm_line_pos_t *positions = nullptr;      // one per record
+  olm_line_t *lines = nullptr;              // lines_only
+  uint64_t n_lines = 0, total = 0;          // total: the call's record count
+};
+// Result arrays of the host API: pinned from kPinnedResultMin bytes (freed by host_result_free)
+void *host_result_alloc(size_t bytes);
+void host_result_free(void *p);
+
 class Engine {
 public:
   // Parses + re-stages the mapped store and uploads it.  On failure returns nullptr and
@@ -56,7 +67,8 @@ public:
   // dev_haystack = device address of the haystack byte with offset `offset0`
   int format_records(const void *dev_records, uint64_t count, const void *dev_haystack, uint64_t offset0,
                      void **dev_text, uint64_t *text_bytes);
-  int64_t no_overlap_inplace(void *dev_records, uint64_t count);
+  // (with dev_positions: the records' line positions are compacted with them)
+  int64_t no_overlap_inplace(void *dev_records, uint64_t count, void *dev_positions = nullptr);
   int sort_records(void *dev_records, uint64_t count);
 
   // for the multi-GPU layer (multi.cpp)
@@ -93,6 +105,25 @@ public:
   int count_records(const void *dev_records, uint64_t count, void *dev_counts);
   int count_records_to_host(const void *dev_records, uint64_t count, uint64_t *counts); // counts[id] += ...
 
+  // Lines (include/olm_b200.h "lines", lines.cuh).  newline_facts: the facts of the device bytes
+  // [0, len); the tile scan it leaves serves a following line_positions(..., tiles_ready = true) on the
+  // same bytes.  line_positions: one LinePos per device record (offsets in [bytes_begin, bytes_begin +
+  // len), dev_bytes the byte at bytes_begin).  matching_lines: run-length by line into a matcher-owned
+  // device array.  Each adds its time to timing().total_ms.
+  int newline_facts(const void *dev_bytes, uint64_t len, olm_newline_facts_t *out);
+  int line_positions(const void *dev_records, uint64_t count, const void *dev_bytes, uint64_t bytes_begin, uint64_t len,
+                     const olm_line_origin_t &origin, void *dev_positions, bool tiles_ready = false);
+  int matching_lines(const void *dev_positions, uint64_t count, void **dev_lines, uint64_t *n_lines);
+  // Host haystack: the records of match_host and their positions, or (lines_only) only the matching
+  // lines; the arrays are host_result_alloc'ed.  One GPU, or OLM_HOST_SPAN_BYTES spans.
+  int lines_host(const uint8_t *haystack, size_t n, const MatchFlags &f, bool lines_only, LinesResult *out);
+  // device records + positions -> host arrays, or (lines_only) their matching lines
+  int lines_to_host(const void *dev_records, const void *dev_positions, uint64_t count, bool lines_only,
+                    LinesResult *out);
+  const void *resident_haystack() const;           // the device copy of the last host haystack or slice
+  void *positions_buffer(size_t bytes, int which); // device buffers for positions: 0 = a call's, 1 = gathered
+  int copy_to_host(void *host_dst, const void *dev_src, size_t bytes); // asynchronous, on stream()
+
 private:
   Engine() = default;
   int stage_host(const uint8_t *src, size_t n);
@@ -101,6 +132,8 @@ private:
   omega_match_results_t *match_host_spans(const uint8_t *haystack, size_t n, const MatchFlags &f, uint64_t span);
   int count_host_spans(const uint8_t *haystack, size_t n, const MatchFlags &f, uint64_t span, uint64_t *counts,
                        uint64_t *total);
+  int lines_host_spans(const uint8_t *haystack, size_t n, const MatchFlags &f, uint64_t span, bool lines_only,
+                       LinesResult *out);
   unsigned long long *zeroed_counts();
   int add_counts_to_host(uint64_t *counts);
   EngineImpl *impl_ = nullptr;

@@ -20,86 +20,19 @@
 // one-block scan of the aggregates, per-block finish.
 #include "filters.cuh"
 
+#include "block_scan.cuh"
+
 namespace olm {
 
 namespace {
 
-constexpr int kFThreads = 256;
-constexpr int kFItems = 8;
-constexpr int kFBlock = kFThreads * kFItems; // records per block
-constexpr uint32_t kFull = 0xFFFFFFFFu;
-
-struct MaxOp {
-  __device__ static unsigned long long identity() { return 0ull; }
-  __device__ static unsigned long long apply(unsigned long long a, unsigned long long b) { return a > b ? a : b; }
-};
-struct SumOp {
-  __device__ static unsigned long long identity() { return 0ull; }
-  __device__ static unsigned long long apply(unsigned long long a, unsigned long long b) { return a + b; }
-};
-
-template <typename Op>
-__device__ unsigned long long block_exclusive_scan(unsigned long long v, unsigned long long *total) {
-  __shared__ unsigned long long s_w[kFThreads / 32];
-  const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  unsigned long long incl = v;
-#pragma unroll
-  for (int d = 1; d < 32; d <<= 1) {
-    const unsigned long long t = __shfl_up_sync(kFull, incl, d);
-    if (lane >= (uint32_t)d) incl = Op::apply(incl, t);
-  }
-  unsigned long long excl = __shfl_up_sync(kFull, incl, 1);
-  if (lane == 0) excl = Op::identity();
-  __syncthreads();
-  if (lane == 31) s_w[warp] = incl;
-  __syncthreads();
-  unsigned long long pre = Op::identity(), all = Op::identity();
-#pragma unroll
-  for (int w = 0; w < kFThreads / 32; ++w) {
-    if ((uint32_t)w < warp) pre = Op::apply(pre, s_w[w]);
-    all = Op::apply(all, s_w[w]);
-  }
-  *total = all;
-  return Op::apply(pre, excl);
-}
-
 __device__ __forceinline__ unsigned long long rec_end(const Record &r) { return r.offset + r.len; }
-
-// phase 1 of either scan: per-block aggregate of value(i)
-template <typename Op, typename F>
-__device__ void block_aggregate(uint64_t n, unsigned long long *agg, F value) {
-  const uint64_t base = (uint64_t)blockIdx.x * kFBlock + (uint64_t)threadIdx.x * kFItems;
-  unsigned long long a = Op::identity();
-#pragma unroll
-  for (int k = 0; k < kFItems; ++k)
-    if (base + k < n) a = Op::apply(a, value(base + k));
-  unsigned long long total;
-  block_exclusive_scan<Op>(a, &total);
-  if (threadIdx.x == 0) agg[blockIdx.x] = total;
-}
 
 __global__ void __launch_bounds__(kFThreads) end_max_aggregate_kernel(const Record *r, uint64_t n, unsigned long long *agg) {
   block_aggregate<MaxOp>(n, agg, [&](uint64_t i) { return rec_end(r[i]); });
 }
 __global__ void __launch_bounds__(kFThreads) keep_sum_aggregate_kernel(const uint8_t *keep, uint64_t n, unsigned long long *agg) {
   block_aggregate<SumOp>(n, agg, [&](uint64_t i) { return (unsigned long long)keep[i]; });
-}
-
-// phase 2: exclusive scan of the block aggregates by ONE block (in place); total -> *out_total
-template <typename Op>
-__global__ void __launch_bounds__(kFThreads) aggregate_scan_kernel(unsigned long long *agg, uint64_t n_blocks,
-                                                                   unsigned long long *out_total) {
-  unsigned long long carry = Op::identity();
-  for (uint64_t base = 0; base < n_blocks; base += kFThreads) {
-    const uint64_t i = base + threadIdx.x;
-    const unsigned long long v = i < n_blocks ? agg[i] : Op::identity();
-    unsigned long long total;
-    const unsigned long long excl = block_exclusive_scan<Op>(v, &total);
-    if (i < n_blocks) agg[i] = Op::apply(carry, excl);
-    carry = Op::apply(carry, total);
-    __syncthreads();
-  }
-  if (threadIdx.x == 0 && out_total) *out_total = carry;
 }
 
 // phase 3 (prefix max): certain-start flags
@@ -163,9 +96,10 @@ __global__ void __launch_bounds__(kFThreads) longest_flags_kernel(const Record *
   if (i < n) keep[i] = (i == 0 || r[i].offset != r[i - 1].offset) ? 1 : 0;
 }
 
-// phase 3 (prefix sum): scatter kept records
-__global__ void __launch_bounds__(kFThreads) compact_kernel(const Record *in, uint64_t n, const uint8_t *keep,
-                                                            const unsigned long long *agg, Record *out) {
+// phase 3 (prefix sum): scatter kept records (or the items of an array parallel to them)
+template <typename T>
+__global__ void __launch_bounds__(kFThreads) compact_kernel(const T *in, uint64_t n, const uint8_t *keep,
+                                                            const unsigned long long *agg, T *out) {
   const uint64_t base = (uint64_t)blockIdx.x * kFBlock + (uint64_t)threadIdx.x * kFItems;
   uint32_t k8[kFItems];
   unsigned long long a = 0;
@@ -200,7 +134,8 @@ static cudaError_t compact(const Record *in, uint64_t n, const uint8_t *keep, un
 }
 
 cudaError_t no_overlap_launch(const Record *in, uint64_t n, Record *out, void *scratch,
-                              unsigned long long *d_total, cudaStream_t st, uint32_t *launches) {
+                              unsigned long long *d_total, cudaStream_t st, uint32_t *launches,
+                              const LinePos *in_pos, LinePos *out_pos) {
   if (n == 0) return cudaSuccess;
   const uint32_t blocks = uint32_t((n + kFBlock - 1) / kFBlock);
   uint8_t *start = static_cast<uint8_t *>(scratch);
@@ -214,7 +149,11 @@ cudaError_t no_overlap_launch(const Record *in, uint64_t n, Record *out, void *s
   chain_walk_kernel<<<uint32_t((n + kFThreads - 1) / kFThreads), kFThreads, 0, st>>>(in, n, start, keep);
   *launches += 4;
   if ((e = cudaGetLastError()) != cudaSuccess) return e;
-  return compact(in, n, keep, agg, d_total, out, st, launches);
+  if ((e = compact(in, n, keep, agg, d_total, out, st, launches)) != cudaSuccess || !in_pos) return e;
+  // the positions of the records: the same keep flags, the block offsets compact() left in agg
+  compact_kernel<<<blocks, kFThreads, 0, st>>>(in_pos, n, keep, agg, out_pos);
+  *launches += 1;
+  return cudaGetLastError();
 }
 
 cudaError_t longest_launch(const Record *in, uint64_t n, Record *out, void *scratch,

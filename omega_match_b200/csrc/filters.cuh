@@ -5,6 +5,7 @@
 #include <cstdint>
 #include <cuda_runtime.h>
 
+#include "lines.cuh"
 #include "scan.cuh"
 
 namespace olm {
@@ -13,9 +14,11 @@ namespace olm {
 size_t filter_scratch_bytes(uint64_t n);
 
 // Greedy no-overlap over n sorted records: kept records are written to `out` (must not alias
-// `in`), their count to *d_total (device).  matcher.c:570-584.
+// `in`), their count to *d_total (device).  matcher.c:570-584.  With `in_pos`, the line positions
+// of the records (lines.cuh, one per record) are compacted with the same keep flags into `out_pos`.
 cudaError_t no_overlap_launch(const Record *in, uint64_t n, Record *out, void *scratch,
-                              unsigned long long *d_total, cudaStream_t st, uint32_t *launches);
+                              unsigned long long *d_total, cudaStream_t st, uint32_t *launches,
+                              const LinePos *in_pos = nullptr, LinePos *out_pos = nullptr);
 
 // Longest-only over n sorted records (first record of every offset).  matcher.c:564-579.
 cudaError_t longest_launch(const Record *in, uint64_t n, Record *out, void *scratch,

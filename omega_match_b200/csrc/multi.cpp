@@ -323,22 +323,144 @@ int MultiMatcher::run_shards(const uint8_t *haystack, size_t n,
 
 // The shards' records (res, `total` in all) gathered on the first GPU over NVLink in shard order, and
 // no_overlap applied there; returns the number kept (*dst: where they are), -1 on failure.
-int64_t MultiMatcher::gather_no_overlap(const std::vector<olm_cuda_results_t> &res, uint64_t total, const void **dst) {
+// With `positions` (per GPU, one per record) they travel with their records and are compacted with the
+// same keep flags (*pos_dst: where they are).
+int64_t MultiMatcher::gather_no_overlap(const std::vector<olm_cuda_results_t> &res, uint64_t total, const void **dst,
+                                        const std::vector<void *> *positions, void **pos_dst) {
   Engine *E0 = engines_[0];
   void *buf = E0->gather_buffer(total * sizeof(Record));
-  if (!buf) return -1;
+  void *pbuf = positions ? E0->positions_buffer(total * sizeof(Record), 1) : nullptr;
+  if (!buf || (positions && !pbuf)) return -1;
   cudaStream_t s0 = static_cast<cudaStream_t>(E0->stream());
   uint64_t off = 0;
-  for (size_t g = 0; g < res.size(); off += res[g].count, ++g)
-    if (res[g].count &&
-        cudaMemcpyPeerAsync(static_cast<uint8_t *>(buf) + off * sizeof(Record), E0->device(), res[g].records,
+  for (size_t g = 0; g < res.size(); off += res[g].count, ++g) {
+    if (!res[g].count) continue;
+    if (cudaMemcpyPeerAsync(static_cast<uint8_t *>(buf) + off * sizeof(Record), E0->device(), res[g].records,
                             engines_[g]->device(), res[g].count * sizeof(Record), s0) != cudaSuccess)
       return -1;
+    if (positions && cudaMemcpyPeerAsync(static_cast<uint8_t *>(pbuf) + off * sizeof(olm_line_pos_t), E0->device(),
+                                         (*positions)[g], engines_[g]->device(), res[g].count * sizeof(olm_line_pos_t),
+                                         s0) != cudaSuccess)
+      return -1;
+  }
   if (cudaStreamSynchronize(s0) != cudaSuccess) return -1;
-  const int64_t k = E0->no_overlap_inplace(buf, total);
+  const int64_t k = E0->no_overlap_inplace(buf, total, pbuf);
   last_.filter_ms = E0->timing().filter_ms;
   *dst = buf;
+  if (pos_dst) *pos_dst = pbuf;
   return k;
+}
+
+int MultiMatcher::lines_host(const uint8_t *haystack, size_t n, const MatchFlags &f, bool lines_only, LinesResult *out) {
+  const int N = (int)engines_.size();
+  *out = LinesResult{};
+  last_ = olm_cuda_timing_t{};
+  scanned_.assign(N, false);
+  if (n == 0 || !haystack) return engines_[0]->lines_host(haystack, n, f, lines_only, out);
+  if (engines_[0]->needs_window_tails() && f.word_boundary) { // (as match_host)
+    scanned_[0] = true;
+    const int rc = engines_[0]->lines_host(haystack, n, f, lines_only, out);
+    last_ = engines_[0]->timing();
+    if (rc == 0) sync_ghost(0);
+    return rc;
+  }
+  MatchFlags fs = f;
+  fs.no_overlap = false;
+  std::vector<olm_cuda_results_t> res(N);
+  std::vector<olm_newline_facts_t> facts(N, olm_newline_facts_t{0, ~0ull, ~0ull});
+  std::vector<uint64_t> own_begin(N, 0), own_end(N, 0), slice_begin(N, 0);
+  for (int g = 0; g < N; ++g) res[g] = olm_cuda_results_t{0, nullptr, engines_[g]->device()};
+  if (run_shards(haystack, n, [&](int g, const uint8_t *slice, const ScanRange &r) {
+        own_begin[g] = r.own_begin;
+        own_end[g] = r.own_end;
+        slice_begin[g] = r.slice_begin;
+        if (engines_[g]->match_shard_host(slice, r, fs, &res[g]) != 0) return -1;
+        const uint8_t *own = static_cast<const uint8_t *>(engines_[g]->resident_haystack()) + (r.own_begin - r.slice_begin);
+        return engines_[g]->newline_facts(own, r.own_end - r.own_begin, &facts[g]);
+      }) != 0)
+    return -1;
+  // every GPU's origin from the facts of the ranges before and after it (shard order = byte order)
+  std::vector<olm_line_origin_t> origin(N);
+  uint64_t line = 0, begin = 0;
+  for (int g = 0; g < N; ++g) {
+    origin[g].line = line;
+    origin[g].begin = begin;
+    line += facts[g].newlines;
+    if (facts[g].newlines) begin = own_begin[g] + facts[g].last + 1;
+  }
+  uint64_t next = n;
+  for (int g = N - 1; g >= 0; --g) {
+    origin[g].next_newline = next;
+    if (facts[g].newlines) next = own_begin[g] + facts[g].first;
+  }
+  std::vector<void *> pos(N, nullptr);
+  std::vector<int> rc(N, 0);
+  {
+    std::vector<std::thread> th;
+    for (int g = 0; g < N; ++g) {
+      if (!res[g].count) continue;
+      th.emplace_back([&, g]() {
+        Engine *e = engines_[g];
+        const uint8_t *own = static_cast<const uint8_t *>(e->resident_haystack()) + (own_begin[g] - slice_begin[g]);
+        pos[g] = e->positions_buffer(res[g].count * sizeof(olm_line_pos_t), 0);
+        rc[g] = !pos[g] || e->line_positions(res[g].records, res[g].count, own, own_begin[g], own_end[g] - own_begin[g],
+                                             origin[g], pos[g], true) != 0;
+      });
+    }
+    for (auto &t : th) t.join();
+  }
+  uint64_t total = 0;
+  std::vector<uint64_t> off(N, 0);
+  for (int g = 0; g < N; ++g) {
+    if (rc[g]) return -1;
+    off[g] = total;
+    total += res[g].count;
+    last_.total_ms = std::max(last_.total_ms, engines_[g]->timing().total_ms);
+  }
+  Engine *E0 = engines_[0];
+  if (f.no_overlap && total > 1) { // the records and their positions on the first GPU, filtered once
+    const void *recs = nullptr;
+    void *p0 = nullptr;
+    const int64_t k = gather_no_overlap(res, total, &recs, &pos, &p0);
+    if (k < 0) return -1;
+    return E0->lines_to_host(recs, p0, uint64_t(k), lines_only, out);
+  }
+  out->total = total;
+  if (lines_only) { // per GPU, then one entry for a line that continues on the next GPU
+    std::vector<olm_line_t> all;
+    for (int g = 0; g < N; ++g) {
+      if (!res[g].count) continue;
+      void *dl = nullptr;
+      uint64_t m = 0;
+      if (engines_[g]->matching_lines(pos[g], res[g].count, &dl, &m) != 0) return -1;
+      const size_t at = all.size();
+      all.resize(at + m);
+      if (engines_[g]->copy_to_host(all.data() + at, dl, m * sizeof(olm_line_t)) != 0 || engines_[g]->sync() != 0) return -1;
+      if (at && m && all[at - 1].line == all[at].line) {
+        all[at - 1].records += all[at].records;
+        all.erase(all.begin() + at);
+      }
+    }
+    out->lines = static_cast<olm_line_t *>(host_result_alloc(all.size() * sizeof(olm_line_t)));
+    if (!out->lines) return -1;
+    if (!all.empty()) std::memcpy(out->lines, all.data(), all.size() * sizeof(olm_line_t));
+    out->n_lines = all.size();
+    return 0;
+  }
+  out->results = static_cast<omega_match_results_t *>(std::malloc(sizeof(omega_match_results_t)));
+  if (!out->results) return -1;
+  out->results->count = total;
+  out->results->matches = static_cast<omega_match_result_t *>(host_result_alloc(total * sizeof(omega_match_result_t)));
+  out->positions = static_cast<olm_line_pos_t *>(host_result_alloc(total * sizeof(olm_line_pos_t)));
+  if (!out->results->matches || !out->positions) return -1;
+  bool ok = true; // every GPU copies into its range of the arrays, all links at once
+  for (int g = 0; g < N && ok; ++g)
+    if (res[g].count)
+      ok = engines_[g]->records_to_host(out->results->matches + off[g], res[g].records, res[g].count) == 0 &&
+           engines_[g]->copy_to_host(out->positions + off[g], pos[g], res[g].count * sizeof(olm_line_pos_t)) == 0;
+  for (int g = 0; g < N; ++g)
+    if (engines_[g]->sync() != 0) ok = false;
+  return ok ? 0 : -1;
 }
 
 // match_host() counting (include/olm_b200.h olm_cuda_count_patterns).  Without no_overlap every GPU

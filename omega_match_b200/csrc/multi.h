@@ -30,6 +30,9 @@ public:
   omega_match_results_t *match_host(const uint8_t *haystack, size_t n, const MatchFlags &f);
   // Engine::count_host over the GPUs (the pattern tables loaded on every engine)
   int count_host(const uint8_t *haystack, size_t n, const MatchFlags &f, uint64_t *counts, uint64_t *total);
+  // Engine::lines_host over the GPUs: every GPU takes the newline facts of its own range, the host
+  // combines them into each GPU's origin, and every GPU resolves its records with it
+  int lines_host(const uint8_t *haystack, size_t n, const MatchFlags &f, bool lines_only, LinesResult *out);
   void collect_stats(omega_match_stats_t *accum);
   void set_exact_stats(bool on);
   int set_pattern_ids(bool on, const PatternCatalog *cat); // every engine (Engine::set_pattern_ids)
@@ -41,7 +44,8 @@ public:
 private:
   void sync_ghost(int from);
   int run_shards(const uint8_t *haystack, size_t n, const std::function<int(int, const uint8_t *, const ScanRange &)> &scan);
-  int64_t gather_no_overlap(const std::vector<olm_cuda_results_t> &res, uint64_t total, const void **dst);
+  int64_t gather_no_overlap(const std::vector<olm_cuda_results_t> &res, uint64_t total, const void **dst,
+                            const std::vector<void *> *positions = nullptr, void **pos_dst = nullptr);
   std::vector<Engine *> engines_;
   std::vector<bool> scanned_; // engines that took part in the last call
   olm_cuda_timing_t last_{};

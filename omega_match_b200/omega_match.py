@@ -10,7 +10,8 @@ Additions (not in the reference): `Matcher.match_arrays` (numpy result without p
 Python objects), `Matcher.match_device` / `match_shard` (device-resident haystack and
 results), `Matcher.last_timing`, pattern ids (`Matcher.match_ids`, `set_pattern_ids`,
 `pattern_count`, `pattern`), pattern counts (`Matcher.pattern_counts`, `pattern_counts_device`,
-`count_records_device`).
+`count_records_device`), lines (`Matcher.match_lines`, `matching_lines`, `line_positions_device`,
+`newline_facts_device`, `matching_lines_device`).
 """
 from __future__ import annotations
 
@@ -27,6 +28,15 @@ from ._lib import (CudaResultsC, CudaTimingC, MatchStatsC, PatternStoreStatsC)
 MATCH_DTYPE = np.dtype([("offset", "<u8"), ("len", "<u4"), ("_pad", "<u4")])
 # match_ids(): the same 16 bytes, the pad holding the pattern id (include/olm_b200.h)
 MATCH_IDS_DTYPE = np.dtype([("offset", "<u8"), ("len", "<u4"), ("pattern_id", "<u4")])
+# match_lines(): a record with the line it lies on (include/olm_b200.h "lines"); pattern_id is there
+# only while pattern ids are on
+LINE_MATCH_DTYPE = np.dtype([("offset", "<u8"), ("len", "<u4"), ("line", "<u8"), ("line_begin", "<u8"),
+                             ("line_end", "<u8")])
+LINE_MATCH_IDS_DTYPE = np.dtype([("offset", "<u8"), ("len", "<u4"), ("pattern_id", "<u4"), ("line", "<u8"),
+                                 ("line_begin", "<u8"), ("line_end", "<u8")])
+# olm_line_pos_t (per record) and olm_line_t (per matching line)
+LINE_POS_DTYPE = np.dtype([("line", "<u8"), ("begin", "<u8"), ("end", "<u8")])
+LINE_DTYPE = np.dtype([("line", "<u8"), ("begin", "<u8"), ("end", "<u8"), ("records", "<u8")])
 # omega_match_result_t as the library writes it (24 bytes)
 RECORD_DTYPE = np.dtype([("offset", "<u8"), ("len", "<u4"), ("_pad", "<u4"), ("match", "<u8")])
 
@@ -328,6 +338,77 @@ class Matcher:
         into pattern_count uint64 words of device memory at counts_ptr."""
         if self._lib.olm_cuda_count_records(self._matcher, records_ptr, count, counts_ptr) != 0:
             raise RuntimeError("olm_cuda_count_records failed (id out of range? see stderr)")
+
+    # -- lines (include/olm_b200.h "lines") ----------------------------------------------------
+    def match_lines(self, haystack, **kw) -> np.ndarray:
+        """Like match_arrays(), with the line of every match: LINE_MATCH_DTYPE (offset, len, line,
+        line_begin, line_end) in result order; with pattern ids on, LINE_MATCH_IDS_DTYPE, which adds
+        pattern_id.  line is 0-based (grep -n prints line + 1); the line's bytes are
+        haystack[line_begin:line_end], without its '\n'."""
+        hay, ptr, n = _host_haystack(haystack)
+        res, pos = C.POINTER(_lib.MatchResultsC)(), C.c_void_p()
+        if self._lib.olm_cuda_match_lines(self._matcher, ptr, n, *_flag_ints(kw), C.byref(res), C.byref(pos)) != 0:
+            raise RuntimeError("olm_cuda_match_lines failed (see stderr)")
+        try:
+            cnt = res.contents.count
+            rec = np.zeros(cnt, dtype=RECORD_DTYPE)
+            lp = np.zeros(cnt, dtype=LINE_POS_DTYPE)
+            if cnt:
+                C.memmove(rec.ctypes.data, res.contents.matches, cnt * RECORD_DTYPE.itemsize)
+                C.memmove(lp.ctypes.data, pos.value, cnt * LINE_POS_DTYPE.itemsize)
+        finally:
+            self._lib.omega_match_results_destroy(res)
+            self._lib.olm_lines_free(pos)
+        out = np.zeros(cnt, dtype=LINE_MATCH_IDS_DTYPE if self._pattern_ids else LINE_MATCH_DTYPE)
+        out["offset"] = rec["offset"]
+        out["len"] = rec["len"]
+        if self._pattern_ids:
+            out["pattern_id"] = rec["_pad"]
+        out["line"], out["line_begin"], out["line_end"] = lp["line"], lp["begin"], lp["end"]
+        return out
+
+    def matching_lines(self, haystack, **kw) -> np.ndarray:
+        """The distinct lines that hold a match, in order: LINE_DTYPE (line, begin, end, records), records
+        = the matches match() with the same options returns on that line.  len() is grep -c.  Only the
+        lines leave the GPU."""
+        hay, ptr, n = _host_haystack(haystack)
+        lines, n_lines, total = C.c_void_p(), C.c_uint64(), C.c_uint64()
+        if self._lib.olm_cuda_matching_lines(self._matcher, ptr, n, *_flag_ints(kw), C.byref(lines), C.byref(n_lines),
+                                             C.byref(total)) != 0:
+            raise RuntimeError("olm_cuda_matching_lines failed (see stderr)")
+        out = np.zeros(n_lines.value, dtype=LINE_DTYPE)
+        if n_lines.value:
+            C.memmove(out.ctypes.data, lines.value, n_lines.value * LINE_DTYPE.itemsize)
+        self._lib.olm_lines_free(lines)
+        return out
+
+    def line_positions_device(self, records_ptr: int, count: int, bytes_ptr: int, bytes_begin: int, bytes_len: int,
+                              positions_ptr: int, origin=None) -> None:
+        """Device records (offsets in [bytes_begin, bytes_begin + bytes_len)) -> one olm_line_pos_t (3
+        uint64: line, begin, end) per record at positions_ptr.  bytes_ptr holds those bytes; `origin` =
+        (line, begin, next_newline) of what lies outside them (sharding.line_origins), None for a whole
+        haystack (bytes_begin 0)."""
+        o = C.byref(_lib.LineOriginC(*origin)) if origin is not None else None
+        if self._lib.olm_cuda_line_positions(self._matcher, records_ptr, count, bytes_ptr, bytes_begin, bytes_len, o,
+                                             positions_ptr) != 0:
+            raise RuntimeError("olm_cuda_line_positions failed (see stderr)")
+
+    def newline_facts_device(self, bytes_ptr: int, size: int):
+        """(newlines, first, last) of the device bytes [0, size), positions relative to them; first and
+        last are None without a '\n'."""
+        f = _lib.NewlineFactsC()
+        if self._lib.olm_cuda_newline_facts(self._matcher, bytes_ptr, size, C.byref(f)) != 0:
+            raise RuntimeError("olm_cuda_newline_facts failed (see stderr)")
+        none = (1 << 64) - 1
+        return (int(f.newlines), None if f.first == none else int(f.first), None if f.last == none else int(f.last))
+
+    def matching_lines_device(self, positions_ptr: int, count: int):
+        """Device positions (record order) -> (n_lines, device pointer of n_lines olm_line_t: 4 uint64
+        line, begin, end, records), valid until the next call."""
+        p, n = C.c_void_p(), C.c_uint64()
+        if self._lib.olm_cuda_matching_lines_device(self._matcher, positions_ptr, count, C.byref(p), C.byref(n)) != 0:
+            raise RuntimeError("olm_cuda_matching_lines_device failed (see stderr)")
+        return int(n.value), int(p.value or 0)
 
     def match_device(self, dev_ptr: int, size: int, match_ptr_base: Optional[int] = None, **kw):
         """Haystack already in HBM (16-byte aligned device pointer).  Returns (count, device

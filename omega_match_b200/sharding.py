@@ -18,11 +18,12 @@ in the tests, with the scan itself supplied by the caller).
 from __future__ import annotations
 
 from dataclasses import dataclass
-from typing import List, Optional
+from typing import List, Optional, Tuple
 
 WINDOW = 4 * 1024 * 1024
 ALIGN = 16
 RECORD_BYTES = 24
+NO_NEWLINE = 2**64 - 1  # olm_newline_facts_t first / last of a range without '\n'
 
 
 @dataclass(frozen=True)
@@ -54,6 +55,42 @@ def shard_plan(size: int, world: int, largest_pattern: int, windowed: bool) -> L
             raise RuntimeError("olm_shard_plan failed")
         shards.append(Shard(r, sh.own_begin, sh.own_end, sh.slice_begin, sh.slice_end))
     return shards
+
+
+def line_origins(facts, own_ranges, global_size: int) -> List[Tuple[int, int, int]]:
+    """Every shard's line origin (include/olm_b200.h olm_line_origin_t: line, begin, next_newline) from
+    the newline facts of all shards.  `facts[k]` = (newlines, first, last) of shard k's OWN range
+    (olm_cuda_newline_facts: positions relative to the range; first / last None or 2**64-1 when it has no
+    '\n'), `own_ranges[k]` = (own_begin, own_end); the ranges lie in byte order and cover
+    [0, global_size) without gaps.  Pure host logic: a one-process-per-GPU job exchanges the facts (3
+    words per rank) by its own means and calls this on every rank."""
+    if len(facts) != len(own_ranges):
+        raise ValueError("one facts entry per range")
+    at = 0
+    for b, e in own_ranges:
+        if b != at or e < b:
+            raise ValueError("the own ranges must cover [0, global_size) in order without gaps")
+        at = e
+    if at != global_size:
+        raise ValueError("the own ranges must cover [0, global_size) in order without gaps")
+
+    def none(v):
+        return v is None or v == NO_NEWLINE
+
+    out = []
+    line = begin = 0
+    for (count, first, last), (b, _) in zip(facts, own_ranges):
+        out.append([line, begin, 0])
+        line += int(count)
+        if count:
+            begin = b + int(last) + 1
+    nxt = global_size
+    for k in range(len(facts) - 1, -1, -1):
+        out[k][2] = nxt
+        count, first, _ = facts[k]
+        if count and not none(first):
+            nxt = own_ranges[k][0] + int(first)
+    return [tuple(o) for o in out]
 
 
 def gather_records(local, dist, dst: int = 0, group=None):
