@@ -182,6 +182,13 @@ const olm::PatternCatalog *catalog_of(const omega_list_matcher_t *m) {
   if (!m->catalog) std::fprintf(stderr, "libomega_match(b200): no pattern catalogue: %s\n", m->catalog_err.c_str());
   return m->catalog.get();
 }
+
+// the device haystack [0, n) at `dev` as one range
+olm::ScanRange whole_haystack(const omega_list_matcher_t *m, const void *dev, uint64_t n, const void *match_ptr_base) {
+  const olm::Header &h = m->engine->header();
+  return olm::scan_range(olm::shard_of(0, n, n, h.largest, h.flags & olm::kFlagAnyTransform), n,
+                         reinterpret_cast<uint64_t>(match_ptr_base), dev);
+}
 } // namespace
 
 omega_list_matcher_t *omega_list_matcher_create_from_buffer(const char *compiled_file, const uint8_t *patterns_buffer,
@@ -251,7 +258,7 @@ omega_match_results_t *omega_list_matcher_match(const omega_list_matcher_t *m, c
 
 void omega_match_results_destroy(omega_match_results_t *results) {
   if (!results) return;
-  if (!olm::pinned_result_release(results->matches)) std::free(results->matches);
+  olm::host_result_free(results->matches);
   results->matches = nullptr;
   results->count = 0;
   std::free(results);
@@ -291,16 +298,8 @@ int olm_cuda_match_device(const omega_list_matcher_t *m, const void *dev_haystac
                           const void *match_ptr_base, int no_overlap, int longest_only, int word_boundary,
                           int word_prefix, int word_suffix, int line_start, int line_end, olm_cuda_results_t *out) {
   if (!m || !m->engine || !out) return -1;
-  olm::ScanRange r;
-  r.dev = dev_haystack;
-  r.slice_begin = 0;
-  r.slice_len = n;
-  r.own_begin = 0;
-  r.own_end = n;
-  r.global_size = n;
-  r.match_ptr_base = reinterpret_cast<uint64_t>(match_ptr_base);
   const int rc = m->engine->match_device(
-      r, to_flags(no_overlap, longest_only, word_boundary, word_prefix, word_suffix, line_start, line_end), out);
+      whole_haystack(m, dev_haystack, n, match_ptr_base), to_flags(no_overlap, longest_only, word_boundary, word_prefix, word_suffix, line_start, line_end), out);
   if (rc == 0 && m->stats) m->engine->collect_stats(m->stats);
   return rc;
 }
@@ -417,17 +416,9 @@ int olm_cuda_count_patterns_device(const omega_list_matcher_t *m, const void *de
                                    int no_overlap, int longest_only, int word_boundary, int word_prefix,
                                    int word_suffix, int line_start, int line_end, void *dev_counts, uint64_t *total) {
   if (!m || !m->engine || !dev_counts || !total || load_pattern_tables(m)) return -1;
-  olm::ScanRange r;
-  r.dev = dev_haystack;
-  r.slice_begin = 0;
-  r.slice_len = size;
-  r.own_begin = 0;
-  r.own_end = size;
-  r.global_size = size;
-  r.match_ptr_base = reinterpret_cast<uint64_t>(dev_haystack);
   olm_cuda_results_t res;
   const int rc = m->engine->match_device(
-      r, to_flags(no_overlap, longest_only, word_boundary, word_prefix, word_suffix, line_start, line_end), &res,
+      whole_haystack(m, dev_haystack, size, dev_haystack), to_flags(no_overlap, longest_only, word_boundary, word_prefix, word_suffix, line_start, line_end), &res,
       dev_counts);
   if (rc != 0) return rc;
   if (m->stats) m->engine->collect_stats(m->stats);

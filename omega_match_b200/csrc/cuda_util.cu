@@ -1,6 +1,8 @@
 // cuda_util.cu -- small CUDA-facing entry points of the C ABI that do not belong to a matcher.
 #include <cuda_runtime.h>
 
+#include <algorithm>
+#include <cstdlib>
 #include <mutex>
 #include <vector>
 
@@ -22,7 +24,7 @@ struct PinnedBlock {
 std::mutex g_pin_mu;
 std::vector<PinnedBlock> g_pin;
 constexpr size_t kMaxIdleBlocks = 4;
-} // namespace
+constexpr size_t kPinnedResultMin = size_t(1) << 20;
 
 void *pinned_result_alloc(size_t bytes) {
   std::lock_guard<std::mutex> lk(g_pin_mu);
@@ -43,6 +45,7 @@ void *pinned_result_alloc(size_t bytes) {
   return p;
 }
 
+// false: not one of ours (plain malloc)
 bool pinned_result_release(void *p) {
   std::lock_guard<std::mutex> lk(g_pin_mu);
   size_t idle = 0;
@@ -59,6 +62,28 @@ bool pinned_result_release(void *p) {
     g_pin.pop_back();
   }
   return true;
+}
+} // namespace
+
+void *host_result_alloc(size_t bytes) {
+  void *p = bytes >= kPinnedResultMin ? pinned_result_alloc(bytes) : nullptr;
+  return p ? p : std::malloc(std::max<size_t>(bytes, 1));
+}
+
+void host_result_free(void *p) {
+  if (p && !pinned_result_release(p)) std::free(p);
+}
+
+omega_match_results_t *host_results(uint64_t count) {
+  auto *r = static_cast<omega_match_results_t *>(std::malloc(sizeof(omega_match_results_t)));
+  if (!r) return nullptr;
+  r->count = count;
+  r->matches = static_cast<omega_match_result_t *>(host_result_alloc(count * sizeof(omega_match_result_t)));
+  if (!r->matches) {
+    std::free(r);
+    return nullptr;
+  }
+  return r;
 }
 
 } // namespace olm

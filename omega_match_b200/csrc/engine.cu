@@ -160,6 +160,27 @@ struct EngineImpl {
 };
 
 namespace {
+// The words behind the batch tickets and redo flags of the misc buffer.  Every scan clears `scan`
+// with one memset; the other words belong to the passes that use them.
+struct MiscWords {
+  struct {
+    unsigned long long total, filter_total, counters[8], temp_count;
+    unsigned long long stats[5]; // stats_kernel (stats.cuh)
+  } scan;
+  unsigned long long missing_ids; // records without a pattern of the catalogue (ids, counts)
+  unsigned long long unused17[3];
+  unsigned long long records_outside; // line positions: records outside their bytes
+  unsigned long long matching_lines;
+  unsigned long long unused22[2];
+  NewlineFacts newline_facts;
+};
+static_assert(sizeof(MiscWords) <= 256, "the misc words fit the 256 bytes behind the tickets");
+
+// misc: [0, kMaxBatches) u32 tickets | [kMaxBatches, 2 kMaxBatches) u32 redo flags | MiscWords
+MiscWords *misc_words(EngineImpl &E) {
+  if (E.misc.ensure(size_t(kMaxBatches) * 8 + 256)) return nullptr;
+  return reinterpret_cast<MiscWords *>(static_cast<uint8_t *>(E.misc.p) + size_t(kMaxBatches) * 8);
+}
 // index of the event after which the first `bytes` bytes of the slice are in HBM
 size_t seg_event_for(const EngineImpl &E, uint64_t bytes) {
   if (E.seg_events.size() <= 1 || E.seg_bytes == 0 || bytes == 0) return 0;
@@ -367,10 +388,8 @@ int Engine::match_device(const ScanRange &r, const MatchFlags &f, olm_cuda_resul
     std::fprintf(stderr, "libomega_match(b200): haystack too large for one call\n");
     return -1;
   }
-  // misc: [0..kMaxBatches) u32 tickets | [..2*kMaxBatches) u32 redo counts | total (u64),
-  // filter total (u64), counters[8]
-  const size_t misc_total_off = size_t(kMaxBatches) * 8;
-  if (E.misc.ensure(misc_total_off + 256)) return -1;
+  MiscWords *w = misc_words(E);
+  if (!w) return -1;
   unsigned int *d_tickets = static_cast<unsigned int *>(E.misc.p);
   unsigned int *d_redo_flags = d_tickets + kMaxBatches;
   const uint64_t tiles_per_launch =
@@ -378,11 +397,10 @@ int Engine::match_device(const ScanRange &r, const MatchFlags &f, olm_cuda_resul
   const uint64_t chunks_per_launch = tiles_per_launch * kTileChunks;
   if (E.chunk_desc.ensure((chunks_per_launch + 1) * sizeof(ChunkDesc))) return -1;
   if (E.span_base.ensure((chunks_per_launch / kPrefixSpan + 2) * 8)) return -1;
-  unsigned long long *d_total = reinterpret_cast<unsigned long long *>(static_cast<uint8_t *>(E.misc.p) + misc_total_off);
-  unsigned long long *d_ftotal = d_total + 1;
-  unsigned long long *d_counters = d_total + 2;
-  unsigned long long *d_temp_count = d_total + 10;
-  unsigned long long *d_stats = d_total + 11; // five counters of stats_kernel (the memset below clears 16 words)
+  unsigned long long *d_total = &w->scan.total;
+  unsigned long long *d_counters = w->scan.counters;
+  unsigned long long *d_temp_count = &w->scan.temp_count;
+  unsigned long long *d_stats = w->scan.stats;
   E.stats_valid = false;
 
   const bool identity_map = windowed && !(E.hdr.flags & (kFlagIgnorePunct | kFlagElideSpace));
@@ -433,7 +451,7 @@ int Engine::match_device(const ScanRange &r, const MatchFlags &f, olm_cuda_resul
     if (E.temp.ensure(temp_cap * 4)) return -1;
     OLM_CUDA(cudaMemsetAsync(d_tickets, 0, n_batches * 4, E.stream));
     OLM_CUDA(cudaMemsetAsync(d_redo_flags, 0, n_batches * 4, E.stream));
-    OLM_CUDA(cudaMemsetAsync(d_total, 0, 128, E.stream));
+    OLM_CUDA(cudaMemsetAsync(&w->scan, 0, sizeof w->scan, E.stream));
     uint32_t launches = 0, scan_launches = 0;
     uint64_t tf_batches = 0;
     OLM_CUDA(cudaEventRecord(E.ev[0], E.stream));
@@ -559,9 +577,9 @@ int Engine::match_device(const ScanRange &r, const MatchFlags &f, olm_cuda_resul
     uint32_t launches = 0;
     OLM_CUDA(cudaEventRecord(E.ev[2], E.stream));
     OLM_CUDA(no_overlap_launch(static_cast<const Record *>(E.out.p), total, static_cast<Record *>(E.out2.p),
-                               E.fscratch.p, d_ftotal, E.stream, &launches));
+                               E.fscratch.p, &w->scan.filter_total, E.stream, &launches));
     OLM_CUDA(cudaEventRecord(E.ev[3], E.stream));
-    OLM_CUDA(cudaMemcpyAsync(&total, d_ftotal, sizeof total, cudaMemcpyDeviceToHost, E.stream));
+    OLM_CUDA(cudaMemcpyAsync(&total, &w->scan.filter_total, sizeof total, cudaMemcpyDeviceToHost, E.stream));
     OLM_CUDA(cudaStreamSynchronize(E.stream));
     cudaEventElapsedTime(&ms, E.ev[2], E.ev[3]);
     E.last.filter_ms = ms;
@@ -571,7 +589,7 @@ int Engine::match_device(const ScanRange &r, const MatchFlags &f, olm_cuda_resul
     final_records = E.out.p;
   }
   if ((E.want_ids || dev_counts) && total) {
-    unsigned long long *d_missing = d_total + 16; // (misc words 16.. are not cleared with the scan's)
+    unsigned long long *d_missing = &w->missing_ids;
     unsigned long long missing = 0;
     uint32_t launches = 0;
     // (the host path: a record may end in a segment the scan did not have to wait for)
@@ -746,47 +764,80 @@ int Engine::match_shard_host(const uint8_t *host_slice, const ScanRange &range, 
   return 0;
 }
 
-// A host haystack in consecutive spans of `span` start positions (opt-in: OLM_HOST_SPAN_BYTES; written
-// for haystacks that should not be resident in HBM all at once; NOT yet run on a GPU -- DESIGN 7b).
-// Every span is a byte-range shard of the whole (SURVEY 8e: same ownership rule, halo and
-// global-size predicates as the multi-GPU path), scanned from host memory with the copy
-// overlapped; the records of the spans are concatenated in order, and `no_overlap` -- the one
-// filter that crosses span edges -- runs once on the concatenation, on the device.
-omega_match_results_t *Engine::match_host_spans(const uint8_t *haystack, size_t n, const MatchFlags &f, uint64_t span) {
+// A host haystack in consecutive spans of host_span start positions (opt-in: OLM_HOST_SPAN_BYTES; for
+// haystacks that should not be resident in HBM all at once), or in one span of all n bytes.  Every span
+// is a byte-range shard of the whole (SURVEY 8e: same ownership rule, halo and global-size predicates
+// as the multi-GPU path), scanned from host memory with the copy overlapped; step(span, its records,
+// several) runs after each.  With several spans, `no_overlap` -- the one filter that crosses span
+// edges -- is left to the caller, to run once on the concatenation, and nothing is counted into
+// dev_counts (counts follow the filter).  Returns the number of spans, -1 on failure.
+int Engine::host_spans(const uint8_t *haystack, size_t n, const MatchFlags &f, void *dev_counts, const SpanStep &step) {
   EngineImpl &E = *impl_;
-  static_assert(sizeof(Record) == sizeof(omega_match_result_t), "records are copied out verbatim");
-  const bool windowed = E.hdr.flags & kFlagAnyTransform;
-  MatchFlags fs = f;
-  fs.no_overlap = false;
-  std::vector<omega_match_result_t> all;
+  OLM_CUDA(cudaSetDevice(E.device));
   E.span_acc = omega_match_stats_t{};
-  for (uint64_t b = 0; b < n; b += span) {
-    const uint64_t e = std::min<uint64_t>(n, b + span);
-    ScanRange r;
-    r.own_begin = b;
-    r.own_end = e;
-    r.global_size = n;
-    r.match_ptr_base = reinterpret_cast<uint64_t>(haystack);
-    r.slice_begin = (windowed || b < 16) ? b : b - 16; // (b is a multiple of 4 MiB)
-    r.slice_len = (windowed ? e : std::min<uint64_t>(n, e + E.hdr.largest + 1)) - r.slice_begin;
+  if (n == 0 || !haystack) { // nothing scanned: collect_stats() and timing() must not report the previous call
+    std::memset(E.counters, 0, sizeof E.counters);
+    std::memset(E.stat_counters, 0, sizeof E.stat_counters);
+    E.attempts_last = 0;
+    E.stats_valid = false;
+    E.last = olm_cuda_timing_t{};
+    return 0;
+  }
+  const uint64_t span = E.host_span && n > E.host_span ? E.host_span : n;
+  const bool several = span < n;
+  MatchFlags fs = f;
+  if (several && f.no_overlap) {
+    fs.no_overlap = false;
+    dev_counts = nullptr;
+  }
+  int spans = 0;
+  for (uint64_t b = 0; b < n; b += span, ++spans) {
+    const Shard s = shard_of(b, std::min<uint64_t>(n, b + span), n, E.hdr.largest, E.hdr.flags & kFlagAnyTransform);
     olm_cuda_results_t d;
-    if (match_shard_host(haystack + r.slice_begin, r, fs, &d) != 0) return nullptr;
-    if (d.count) {
-      const size_t at = all.size();
-      all.resize(at + d.count);
-      if (cudaMemcpyAsync(all.data() + at, d.records, d.count * sizeof(Record), cudaMemcpyDeviceToHost, E.stream) != cudaSuccess ||
-          cudaStreamSynchronize(E.stream) != cudaSuccess)
-        return nullptr;
-    }
-    if (e < n) { // the last span's counters are collected by the caller, like those of a plain call
+    if (match_shard_host(haystack + s.slice_begin, scan_range(s, n, reinterpret_cast<uint64_t>(haystack)), fs, &d,
+                         dev_counts) != 0 ||
+        step(s, d, several) != 0)
+      return -1;
+    if (s.own_end < n) { // the last span's counters are collected by the caller, like those of a plain call
       omega_match_stats_t acc = E.span_acc;
       E.span_acc = omega_match_stats_t{};
       collect_stats(&acc);
       E.span_acc = acc;
     }
   }
+  return spans;
+}
+
+omega_match_results_t *Engine::match_host(const uint8_t *haystack, size_t n, const MatchFlags &f) {
+  EngineImpl &E = *impl_;
+  static_assert(sizeof(Record) == sizeof(omega_match_result_t), "records are copied out verbatim");
+  omega_match_results_t *results = nullptr; // one span: its records, straight from the device
+  std::vector<Record> all;                  // several: their records, concatenated on the host
+  const int spans = host_spans(haystack, n, f, nullptr, [&](const Shard &, const olm_cuda_results_t &d, bool several) {
+    if (several) {
+      if (!d.count) return 0;
+      const size_t at = all.size();
+      all.resize(at + d.count);
+      return copy_to_host(all.data() + at, d.records, d.count * sizeof(Record)) == 0 && sync() == 0 ? 0 : -1;
+    }
+    if (!(results = host_results(d.count))) return -1;
+    if (!d.count) return 0;
+    float ms = 0.f;
+    cudaEventRecord(E.ev[6], E.stream);
+    OLM_CUDA(cudaMemcpyAsync(results->matches, d.records, d.count * sizeof(Record), cudaMemcpyDeviceToHost, E.stream));
+    cudaEventRecord(E.ev[7], E.stream);
+    OLM_CUDA(cudaStreamSynchronize(E.stream));
+    cudaEventElapsedTime(&ms, E.ev[6], E.ev[7]);
+    E.last.d2h_ms = ms;
+    return 0;
+  });
+  if (spans < 0) {
+    omega_match_results_destroy(results);
+    return nullptr;
+  }
+  if (results) return results;
   uint64_t total = all.size();
-  if (f.no_overlap && total > 1) {
+  if (f.no_overlap && total > 1) { // several spans: the filter once, on the device
     if (E.out.ensure(total * sizeof(Record))) return nullptr;
     if (cudaMemcpyAsync(E.out.p, all.data(), total * sizeof(Record), cudaMemcpyHostToDevice, E.stream) != cudaSuccess) return nullptr;
     const int64_t kept = no_overlap_inplace(E.out.p, total);
@@ -796,67 +847,8 @@ omega_match_results_t *Engine::match_host_spans(const uint8_t *haystack, size_t 
         cudaStreamSynchronize(E.stream) != cudaSuccess)
       return nullptr;
   }
-  auto *results = static_cast<omega_match_results_t *>(std::malloc(sizeof(omega_match_results_t)));
-  if (!results) return nullptr;
-  results->matches = static_cast<omega_match_result_t *>(std::malloc(std::max<size_t>(1, total) * sizeof(omega_match_result_t)));
-  if (!results->matches) {
-    std::free(results);
-    return nullptr;
-  }
-  if (total) std::memcpy(results->matches, all.data(), total * sizeof(omega_match_result_t));
-  results->count = total;
-  return results;
-}
-
-omega_match_results_t *Engine::match_host(const uint8_t *haystack, size_t n, const MatchFlags &f) {
-  EngineImpl &E = *impl_;
-  if (E.host_span && haystack && n > E.host_span) return match_host_spans(haystack, n, f, E.host_span);
-  auto *results = static_cast<omega_match_results_t *>(std::malloc(sizeof(omega_match_results_t)));
-  if (!results) return nullptr;
-  results->count = 0;
-  results->matches = static_cast<omega_match_result_t *>(std::malloc(sizeof(omega_match_result_t)));
-  if (n == 0 || !haystack) { // nothing scanned: collect_stats() must not add the previous call's counters again
-    std::memset(E.counters, 0, sizeof E.counters);
-    std::memset(E.stat_counters, 0, sizeof E.stat_counters);
-    E.attempts_last = 0;
-    E.stats_valid = false;
-    return results;
-  }
-  auto bail = [&]() -> omega_match_results_t * {
-    if (!pinned_result_release(results->matches)) std::free(results->matches);
-    std::free(results);
-    return nullptr;
-  };
-  ScanRange r;
-  r.slice_begin = 0;
-  r.slice_len = n;
-  r.own_begin = 0;
-  r.own_end = n;
-  r.global_size = n;
-  r.match_ptr_base = reinterpret_cast<uint64_t>(haystack);
-  olm_cuda_results_t dres;
-  if (match_shard_host(haystack, r, f, &dres) != 0) return bail();
-  float ms = 0.f;
-  if (dres.count) {
-    std::free(results->matches);
-    const size_t rbytes = dres.count * sizeof(omega_match_result_t);
-    results->matches = nullptr;
-    if (rbytes >= kPinnedResultMin) results->matches = static_cast<omega_match_result_t *>(pinned_result_alloc(rbytes));
-    if (!results->matches) results->matches = static_cast<omega_match_result_t *>(std::malloc(rbytes));
-    if (!results->matches) {
-      std::free(results);
-      return nullptr;
-    }
-    cudaEventRecord(E.ev[6], E.stream);
-    if (cudaMemcpyAsync(results->matches, dres.records, dres.count * sizeof(Record), cudaMemcpyDeviceToHost,
-                        E.stream) != cudaSuccess)
-      return bail();
-    cudaEventRecord(E.ev[7], E.stream);
-    if (cudaStreamSynchronize(E.stream) != cudaSuccess) return bail();
-    cudaEventElapsedTime(&ms, E.ev[6], E.ev[7]);
-    E.last.d2h_ms = ms;
-  }
-  results->count = dres.count;
+  if (!(results = host_results(total))) return nullptr;
+  if (total) std::memcpy(results->matches, all.data(), total * sizeof(Record));
   return results;
 }
 
@@ -869,9 +861,9 @@ int Engine::format_records(const void *dev_records, uint64_t count, const void *
   if (count == 0) return 0;
   OLM_CUDA(cudaDeviceSynchronize()); // records and haystack may come from any stream of the caller
   if (E.fscratch.ensure(format_scratch_bytes(count))) return -1;
-  if (E.misc.ensure(size_t(kMaxBatches) * 8 + 256)) return -1;
-  unsigned long long *d_total =
-      reinterpret_cast<unsigned long long *>(static_cast<uint8_t *>(E.misc.p) + size_t(kMaxBatches) * 8) + 1;
+  MiscWords *w = misc_words(E);
+  if (!w) return -1;
+  unsigned long long *d_total = &w->scan.filter_total;
   uint32_t launches = 0;
   unsigned long long total = 0;
   const Record *rec = static_cast<const Record *>(dev_records);
@@ -896,9 +888,9 @@ int64_t Engine::no_overlap_inplace(void *dev_records, uint64_t count, void *dev_
   OLM_CUDA(cudaDeviceSynchronize());
   if (E.out2.ensure(count * sizeof(Record))) return -1;
   if (E.fscratch.ensure(filter_scratch_bytes(count))) return -1;
-  if (E.misc.ensure(size_t(kMaxBatches) * 8 + 256)) return -1;
-  unsigned long long *d_ftotal =
-      reinterpret_cast<unsigned long long *>(static_cast<uint8_t *>(E.misc.p) + size_t(kMaxBatches) * 8) + 1;
+  MiscWords *w = misc_words(E);
+  if (!w) return -1;
+  unsigned long long *d_ftotal = &w->scan.filter_total;
   uint32_t launches = 0;
   unsigned long long total = 0;
   if (dev_positions && E.d_pos2.ensure(count * sizeof(LinePos))) return -1;
@@ -938,13 +930,6 @@ void *Engine::gather_buffer(size_t bytes, size_t *cap) {
   if ((bytes || !cap) && impl_->gather.ensure(bytes ? bytes : 16)) return nullptr;
   if (cap) *cap = impl_->gather.cap;
   return impl_->gather.p;
-}
-
-int Engine::records_to_host(void *host_dst, const void *dev_records, uint64_t count) {
-  EngineImpl &E = *impl_;
-  OLM_CUDA(cudaSetDevice(E.device));
-  if (count) OLM_CUDA(cudaMemcpyAsync(host_dst, dev_records, count * sizeof(Record), cudaMemcpyDeviceToHost, E.stream));
-  return 0;
 }
 
 int Engine::sync() {
@@ -990,9 +975,9 @@ int Engine::count_records(const void *dev_records, uint64_t count, void *dev_cou
   if (!E.ids.table) return -1;
   if (count == 0) return 0;
   OLM_CUDA(cudaDeviceSynchronize()); // see no_overlap_inplace
-  if (E.misc.ensure(size_t(kMaxBatches) * 8 + 256)) return -1;
-  unsigned long long *d_missing =
-      reinterpret_cast<unsigned long long *>(static_cast<uint8_t *>(E.misc.p) + size_t(kMaxBatches) * 8) + 16;
+  MiscWords *w = misc_words(E);
+  if (!w) return -1;
+  unsigned long long *d_missing = &w->missing_ids;
   unsigned long long missing = 0;
   uint32_t launches = 0;
   OLM_CUDA(cudaMemsetAsync(d_missing, 0, sizeof missing, E.stream));
@@ -1050,81 +1035,36 @@ int Engine::count_shard_host(const uint8_t *host_slice, const ScanRange &range, 
   return 0;
 }
 
+// Without no_overlap, or in one span, every span counts on the device into one scratch array.  Several
+// spans under no_overlap write ids instead (their haystacks are gone when the filter runs): their
+// records are concatenated on the device, filtered once, and counted from the pads.
 int Engine::count_host(const uint8_t *haystack, size_t n, const MatchFlags &f, uint64_t *counts, uint64_t *total) {
   EngineImpl &E = *impl_;
   *total = 0;
-  if (E.host_span && haystack && n > E.host_span) return count_host_spans(haystack, n, f, E.host_span, counts, total);
-  if (n == 0 || !haystack) { // (as match_host)
-    std::memset(E.counters, 0, sizeof E.counters);
-    std::memset(E.stat_counters, 0, sizeof E.stat_counters);
-    E.attempts_last = 0;
-    E.stats_valid = false;
-    E.last = olm_cuda_timing_t{};
-    return 0;
-  }
-  ScanRange r;
-  r.slice_begin = 0;
-  r.slice_len = n;
-  r.own_begin = 0;
-  r.own_end = n;
-  r.global_size = n;
-  r.match_ptr_base = reinterpret_cast<uint64_t>(haystack);
-  return count_shard_host(haystack, r, f, counts, total);
-}
-
-// match_host_spans() counting.  Without no_overlap every span counts on the device into one scratch
-// array; with it the spans write ids (their haystacks are gone when the filter runs), their records
-// are concatenated on the device, filtered once, and counted from the pads.
-int Engine::count_host_spans(const uint8_t *haystack, size_t n, const MatchFlags &f, uint64_t span, uint64_t *counts,
-                             uint64_t *total) {
-  EngineImpl &E = *impl_;
   OLM_CUDA(cudaSetDevice(E.device));
-  const bool windowed = E.hdr.flags & kFlagAnyTransform;
-  const bool filter = f.no_overlap;
-  MatchFlags fs = f;
-  fs.no_overlap = false;
   unsigned long long *d = zeroed_counts();
   if (!d) return -1;
-  const bool ids_were = E.want_ids;
-  E.want_ids = filter;
-  uint64_t all = 0; // records concatenated in E.gather (no_overlap)
-  E.span_acc = omega_match_stats_t{};
-  int rc = 0;
-  for (uint64_t b = 0; b < n && rc == 0; b += span) {
-    const uint64_t e = std::min<uint64_t>(n, b + span);
-    ScanRange r;
-    r.own_begin = b;
-    r.own_end = e;
-    r.global_size = n;
-    r.match_ptr_base = reinterpret_cast<uint64_t>(haystack);
-    r.slice_begin = (windowed || b < 16) ? b : b - 16; // (b is a multiple of 4 MiB)
-    r.slice_len = (windowed ? e : std::min<uint64_t>(n, e + E.hdr.largest + 1)) - r.slice_begin;
-    olm_cuda_results_t res;
-    rc = match_shard_host(haystack + r.slice_begin, r, fs, &res, filter ? nullptr : d);
-    if (rc == 0 && filter && res.count) {
-      // grown geometrically (each growth copies what is there; it is not ordered after the stream's copies)
-      const size_t need = (all + res.count) * sizeof(Record);
-      if (need > E.gather.cap)
-        rc = cudaStreamSynchronize(E.stream) == cudaSuccess ? E.gather.ensure(std::max(need, 2 * E.gather.cap), true) : -1;
-      if (rc == 0 && cudaMemcpyAsync(static_cast<Record *>(E.gather.p) + all, res.records, res.count * sizeof(Record),
-                                     cudaMemcpyDeviceToDevice, E.stream) != cudaSuccess)
-        rc = -1;
-    }
+  PatternIdsOn ids({this}, f.no_overlap); // (a span that counts into d writes no ids)
+  uint64_t all = 0; // records concatenated in E.gather (several spans under no_overlap)
+  const int spans = host_spans(haystack, n, f, d, [&](const Shard &, const olm_cuda_results_t &res, bool several) {
+    const uint64_t at = all;
     all += res.count;
-    if (rc == 0 && e < n) { // (as match_host_spans)
-      omega_match_stats_t acc = E.span_acc;
-      E.span_acc = omega_match_stats_t{};
-      collect_stats(&acc);
-      E.span_acc = acc;
-    }
-  }
-  E.want_ids = ids_were;
-  if (rc != 0) return -1;
-  if (filter && all) {
+    if (!several || !f.no_overlap || !res.count) return 0;
+    // grown geometrically (each growth copies what is there; it is not ordered after the stream's copies)
+    const size_t need = all * sizeof(Record);
+    if (need > E.gather.cap &&
+        (cudaStreamSynchronize(E.stream) != cudaSuccess || E.gather.ensure(std::max(need, 2 * E.gather.cap), true)))
+      return -1;
+    OLM_CUDA(cudaMemcpyAsync(static_cast<Record *>(E.gather.p) + at, res.records, res.count * sizeof(Record),
+                             cudaMemcpyDeviceToDevice, E.stream));
+    return 0;
+  });
+  if (spans <= 0) return spans;
+  if (f.no_overlap && spans > 1 && all) {
     const int64_t kept = no_overlap_inplace(E.gather.p, all);
-    if (kept < 0) return -1;
-    all = uint64_t(kept);
-    return count_records_to_host(E.gather.p, all, counts) != 0 ? -1 : (*total = all, 0);
+    if (kept < 0 || count_records_to_host(E.gather.p, uint64_t(kept), counts) != 0) return -1;
+    *total = uint64_t(kept);
+    return 0;
   }
   if (add_counts_to_host(counts) != 0) return -1;
   *total = all;
@@ -1140,21 +1080,7 @@ int Engine::count_records_to_host(const void *dev_records, uint64_t count, uint6
 
 // ---- lines (lines.cuh, include/olm_b200.h "lines")
 
-void *host_result_alloc(size_t bytes) {
-  void *p = bytes >= kPinnedResultMin ? pinned_result_alloc(bytes) : nullptr;
-  return p ? p : std::malloc(std::max<size_t>(bytes, 1));
-}
-void host_result_free(void *p) {
-  if (p && !pinned_result_release(p)) std::free(p);
-}
-
 namespace {
-// the 32 words behind the batch tickets of match_device's misc buffer; the line passes use
-// [20] records outside, [21] matching lines, [24..26] newline facts
-unsigned long long *misc_words(EngineImpl &E) {
-  if (E.misc.ensure(size_t(kMaxBatches) * 8 + 256)) return nullptr;
-  return reinterpret_cast<unsigned long long *>(static_cast<uint8_t *>(E.misc.p) + size_t(kMaxBatches) * 8);
-}
 // the pass between ev[2] and ev[3] is part of the call's device time
 void add_pass_time(EngineImpl &E, uint32_t launches) {
   float ms = 0.f;
@@ -1188,15 +1114,15 @@ int Engine::newline_facts(const void *dev_bytes, uint64_t len, olm_newline_facts
   OLM_CUDA(cudaSetDevice(E.device));
   if (!out || (len && !dev_bytes) || bytes_unaligned(dev_bytes)) return -1;
   OLM_CUDA(cudaDeviceSynchronize()); // the bytes may come from any stream (see no_overlap_inplace)
-  unsigned long long *w = misc_words(E);
+  MiscWords *w = misc_words(E);
   if (!w || E.d_tiles.ensure(line_tiles_bytes(len))) return -1;
   uint32_t launches = 0;
   NewlineFacts f{};
   OLM_CUDA(cudaEventRecord(E.ev[2], E.stream));
-  OLM_CUDA(newline_facts_launch(static_cast<const uint8_t *>(dev_bytes), len, E.d_tiles.p,
-                                reinterpret_cast<NewlineFacts *>(w + 24), E.stream, &launches));
+  OLM_CUDA(newline_facts_launch(static_cast<const uint8_t *>(dev_bytes), len, E.d_tiles.p, &w->newline_facts, E.stream,
+                                &launches));
   OLM_CUDA(cudaEventRecord(E.ev[3], E.stream));
-  OLM_CUDA(cudaMemcpyAsync(&f, w + 24, sizeof f, cudaMemcpyDeviceToHost, E.stream));
+  OLM_CUDA(cudaMemcpyAsync(&f, &w->newline_facts, sizeof f, cudaMemcpyDeviceToHost, E.stream));
   OLM_CUDA(cudaStreamSynchronize(E.stream));
   add_pass_time(E, launches);
   *out = olm_newline_facts_t{f.newlines, f.first, f.last};
@@ -1215,17 +1141,17 @@ int Engine::line_positions(const void *dev_records, uint64_t count, const void *
   } else {
     OLM_CUDA(cudaDeviceSynchronize());
   }
-  unsigned long long *w = misc_words(E);
+  MiscWords *w = misc_words(E);
   if (!w) return -1;
   uint32_t launches = 0;
   unsigned long long outside = 0;
-  OLM_CUDA(cudaMemsetAsync(w + 20, 0, sizeof outside, E.stream));
+  OLM_CUDA(cudaMemsetAsync(&w->records_outside, 0, sizeof outside, E.stream));
   OLM_CUDA(cudaEventRecord(E.ev[2], E.stream));
   OLM_CUDA(line_positions_launch(static_cast<const Record *>(dev_records), count, static_cast<const uint8_t *>(dev_bytes),
                                  bytes_begin, len, E.d_tiles.p, LineOrigin{origin.line, origin.begin, origin.next_newline},
-                                 static_cast<LinePos *>(dev_positions), w + 20, E.stream, &launches));
+                                 static_cast<LinePos *>(dev_positions), &w->records_outside, E.stream, &launches));
   OLM_CUDA(cudaEventRecord(E.ev[3], E.stream));
-  OLM_CUDA(cudaMemcpyAsync(&outside, w + 20, sizeof outside, cudaMemcpyDeviceToHost, E.stream));
+  OLM_CUDA(cudaMemcpyAsync(&outside, &w->records_outside, sizeof outside, cudaMemcpyDeviceToHost, E.stream));
   OLM_CUDA(cudaStreamSynchronize(E.stream));
   add_pass_time(E, launches);
   if (outside) {
@@ -1243,7 +1169,7 @@ int Engine::matching_lines(const void *dev_positions, uint64_t count, void **dev
   *dev_lines = nullptr;
   *n_lines = 0;
   OLM_CUDA(cudaDeviceSynchronize());
-  unsigned long long *w = misc_words(E);
+  MiscWords *w = misc_words(E);
   if (!w || E.d_lines.ensure(std::max<uint64_t>(count, 1) * sizeof(LineEntry)) ||
       E.d_lscratch.ensure(matching_lines_scratch_bytes(count)))
     return -1;
@@ -1251,9 +1177,9 @@ int Engine::matching_lines(const void *dev_positions, uint64_t count, void **dev
   unsigned long long m = 0;
   OLM_CUDA(cudaEventRecord(E.ev[2], E.stream));
   OLM_CUDA(matching_lines_launch(static_cast<const LinePos *>(dev_positions), count, static_cast<LineEntry *>(E.d_lines.p),
-                                 E.d_lscratch.p, w + 21, E.stream, &launches));
+                                 E.d_lscratch.p, &w->matching_lines, E.stream, &launches));
   OLM_CUDA(cudaEventRecord(E.ev[3], E.stream));
-  OLM_CUDA(cudaMemcpyAsync(&m, w + 21, sizeof m, cudaMemcpyDeviceToHost, E.stream));
+  OLM_CUDA(cudaMemcpyAsync(&m, &w->matching_lines, sizeof m, cudaMemcpyDeviceToHost, E.stream));
   OLM_CUDA(cudaStreamSynchronize(E.stream));
   add_pass_time(E, launches);
   *dev_lines = E.d_lines.p;
@@ -1273,14 +1199,10 @@ int Engine::lines_to_host(const void *dev_records, const void *dev_positions, ui
     out->lines = static_cast<olm_line_t *>(host_result_alloc(m * sizeof(olm_line_t)));
     out->n_lines = m;
   } else {
-    out->results = static_cast<omega_match_results_t *>(std::malloc(sizeof(omega_match_results_t)));
-    if (out->results) {
-      out->results->count = count;
-      out->results->matches = static_cast<omega_match_result_t *>(host_result_alloc(count * sizeof(omega_match_result_t)));
-    }
+    out->results = host_results(count);
     out->positions = static_cast<olm_line_pos_t *>(host_result_alloc(count * sizeof(olm_line_pos_t)));
   }
-  if (lines_only ? !out->lines : (!out->results || !out->results->matches || !out->positions)) return -1;
+  if (lines_only ? !out->lines : (!out->results || !out->positions)) return -1;
   if (lines_only ? m == 0 : count == 0) return 0;
   float ms = 0.f;
   OLM_CUDA(cudaEventRecord(E.ev[6], E.stream));
@@ -1297,68 +1219,29 @@ int Engine::lines_to_host(const void *dev_records, const void *dev_positions, ui
   return 0;
 }
 
+// match_host with positions.  Several spans: a span's line and line start carry in from the spans before
+// it; the records on its last line get their end from the first later span that holds a '\n' (or n).
+// With no_overlap, or for the matching lines, their concatenation goes back to the device.
 int Engine::lines_host(const uint8_t *haystack, size_t n, const MatchFlags &f, bool lines_only, LinesResult *out) {
   EngineImpl &E = *impl_;
   *out = LinesResult{};
-  OLM_CUDA(cudaSetDevice(E.device));
-  if (E.host_span && haystack && n > E.host_span) return lines_host_spans(haystack, n, f, E.host_span, lines_only, out);
-  if (n == 0 || !haystack) { // (as match_host)
-    std::memset(E.counters, 0, sizeof E.counters);
-    std::memset(E.stat_counters, 0, sizeof E.stat_counters);
-    E.attempts_last = 0;
-    E.stats_valid = false;
-    E.last = olm_cuda_timing_t{};
-    return lines_to_host(nullptr, nullptr, 0, lines_only, out);
-  }
-  ScanRange r;
-  r.slice_begin = 0;
-  r.slice_len = n;
-  r.own_begin = 0;
-  r.own_end = n;
-  r.global_size = n;
-  r.match_ptr_base = reinterpret_cast<uint64_t>(haystack);
-  olm_cuda_results_t d;
-  if (match_shard_host(haystack, r, f, &d) != 0) return -1;
-  void *pos = nullptr;
-  if (d.count && (!(pos = positions_buffer(d.count * sizeof(LinePos), 0)) ||
-                  line_positions(d.records, d.count, E.hay.p, 0, n, olm_line_origin_t{0, 0, n}, pos) != 0))
-    return -1;
-  return lines_to_host(d.records, pos, d.count, lines_only, out);
-}
-
-// match_host_spans() with positions.  A span's line and line start carry in from the spans before it;
-// the records on its last line get their end from the first later span that holds a '\n' (or n).
-// With no_overlap, or for the matching lines, the concatenation goes back to the device.
-int Engine::lines_host_spans(const uint8_t *haystack, size_t n, const MatchFlags &f, uint64_t span, bool lines_only,
-                             LinesResult *out) {
-  EngineImpl &E = *impl_;
-  const bool windowed = E.hdr.flags & kFlagAnyTransform;
-  MatchFlags fs = f;
-  fs.no_overlap = false;
-  std::vector<Record> all;
+  std::vector<Record> all; // several spans: records and positions concatenated on the host
   std::vector<LinePos> pos;
   uint64_t line = 0, begin = 0;
   size_t pending = 0; // pos[pending, size()) lie on a line no span so far has ended
-  E.span_acc = omega_match_stats_t{};
-  for (uint64_t b = 0; b < n; b += span) {
-    const uint64_t e = std::min<uint64_t>(n, b + span);
-    ScanRange r;
-    r.own_begin = b;
-    r.own_end = e;
-    r.global_size = n;
-    r.match_ptr_base = reinterpret_cast<uint64_t>(haystack);
-    r.slice_begin = (windowed || b < 16) ? b : b - 16; // (b is a multiple of 4 MiB)
-    r.slice_len = (windowed ? e : std::min<uint64_t>(n, e + E.hdr.largest + 1)) - r.slice_begin;
-    olm_cuda_results_t d;
-    if (match_shard_host(haystack + r.slice_begin, r, fs, &d) != 0) return -1;
-    const uint8_t *own = static_cast<const uint8_t *>(E.hay.p) + (b - r.slice_begin);
-    olm_newline_facts_t nf;
-    if (newline_facts(own, e - b, &nf) != 0) return -1;
+  const int spans = host_spans(haystack, n, f, nullptr, [&](const Shard &s, const olm_cuda_results_t &d, bool several) {
+    const uint8_t *own = static_cast<const uint8_t *>(E.hay.p) + (s.own_begin - s.slice_begin);
+    const uint64_t len = s.own_end - s.own_begin;
+    olm_newline_facts_t nf{}; // (one span: line_positions takes the facts itself, and only for records)
+    if (several && newline_facts(own, len, &nf) != 0) return -1;
+    void *dp = nullptr;
+    const olm_line_origin_t origin{line, begin, s.own_end == n ? n : kNoNewline};
+    if (d.count && (!(dp = positions_buffer(d.count * sizeof(LinePos), 0)) ||
+                    line_positions(d.records, d.count, own, s.own_begin, len, origin, dp, several) != 0))
+      return -1;
+    if (!several) return lines_to_host(d.records, dp, d.count, lines_only, out);
     const size_t at = all.size();
     if (d.count) {
-      void *dp = positions_buffer(d.count * sizeof(LinePos), 0);
-      if (!dp || line_positions(d.records, d.count, own, b, e - b, olm_line_origin_t{line, begin, kNoNewline}, dp, true) != 0)
-        return -1;
       all.resize(at + d.count);
       pos.resize(at + d.count);
       if (copy_to_host(all.data() + at, d.records, d.count * sizeof(Record)) != 0 ||
@@ -1366,19 +1249,16 @@ int Engine::lines_host_spans(const uint8_t *haystack, size_t n, const MatchFlags
         return -1;
     }
     if (nf.newlines) {
-      for (size_t i = pending; i < at; ++i) pos[i].end = b + nf.first;
+      for (size_t i = pending; i < at; ++i) pos[i].end = s.own_begin + nf.first;
       pending = pos.size();
       while (pending > at && pos[pending - 1].end == kNoNewline) --pending;
       line += nf.newlines;
-      begin = b + nf.last + 1;
+      begin = s.own_begin + nf.last + 1;
     }
-    if (e < n) { // (as match_host_spans)
-      omega_match_stats_t acc = E.span_acc;
-      E.span_acc = omega_match_stats_t{};
-      collect_stats(&acc);
-      E.span_acc = acc;
-    }
-  }
+    return 0;
+  });
+  if (spans < 0) return -1;
+  if (spans == 1) return 0;
   for (size_t i = pending; i < pos.size(); ++i) pos[i].end = n;
   uint64_t total = all.size();
   if ((f.no_overlap && total > 1) || (lines_only && total)) {
@@ -1395,12 +1275,9 @@ int Engine::lines_host_spans(const uint8_t *haystack, size_t n, const MatchFlags
   }
   if (lines_only) return lines_to_host(nullptr, nullptr, 0, true, out);
   out->total = total;
-  out->results = static_cast<omega_match_results_t *>(std::malloc(sizeof(omega_match_results_t)));
-  if (!out->results) return -1;
-  out->results->count = total;
-  out->results->matches = static_cast<omega_match_result_t *>(host_result_alloc(total * sizeof(omega_match_result_t)));
+  out->results = host_results(total);
   out->positions = static_cast<olm_line_pos_t *>(host_result_alloc(total * sizeof(olm_line_pos_t)));
-  if (!out->results->matches || !out->positions) return -1;
+  if (!out->results || !out->positions) return -1;
   if (total) {
     std::memcpy(out->results->matches, all.data(), total * sizeof(Record));
     std::memcpy(out->positions, pos.data(), total * sizeof(LinePos));
@@ -1411,7 +1288,7 @@ int Engine::lines_host_spans(const uint8_t *haystack, size_t n, const MatchFlags
 void Engine::collect_stats(omega_match_stats_t *s) {
   if (!s) return;
   EngineImpl &E = *impl_;
-  { // spans of a host haystack before the last one (match_host_spans); normally all zero
+  { // spans of a host haystack before the last one (host_spans); normally all zero
     s->total_attempts += E.span_acc.total_attempts;
     s->total_filtered += E.span_acc.total_filtered;
     s->total_misses += E.span_acc.total_misses;

@@ -1,9 +1,13 @@
 // engine.h -- one matcher on one GPU: the uploaded store, work buffers, and the sequence of
 // kernels that make up a match call.  Plain C++ interface; api.cpp puts the C ABI on top.
 #pragma once
+#include <algorithm>
 #include <cstddef>
 #include <cstdint>
+#include <functional>
 #include <string>
+#include <utility>
+#include <vector>
 
 #include "../../include/olm_b200.h"
 #include "store.h"
@@ -24,10 +28,22 @@ struct ScanRange {
   uint64_t match_ptr_base = 0;
 };
 
-// Large result arrays of the host API (cuda_util.cu): pinned, recycled across calls.
-void *pinned_result_alloc(size_t bytes);
-bool pinned_result_release(void *p); // false: not one of ours (plain malloc)
-constexpr size_t kPinnedResultMin = size_t(1) << 20;
+// Byte-range shards of one haystack (SURVEY 8e): a shard OWNS the start positions [own_begin,
+// own_end) and needs the bytes [slice_begin, slice_end).
+struct Shard {
+  uint64_t own_begin = 0, own_end = 0, slice_begin = 0, slice_end = 0;
+};
+// The shard that owns [own_begin, own_end) of `size` bytes: 16 bytes in front (alignment + the previous
+// byte) and the longest pattern + 1 behind.  Stores with a transform flag shard on multiples of the
+// 4 MiB source window and need no halo.  The whole haystack is shard_of(0, size, size, ...).
+inline Shard shard_of(uint64_t own_begin, uint64_t own_end, uint64_t size, uint32_t largest, bool windowed) {
+  if (windowed) return Shard{own_begin, own_end, own_begin, own_end};
+  return Shard{own_begin, own_end, own_begin >= 16 ? own_begin - 16 : 0, std::min<uint64_t>(size, own_end + largest + 1)};
+}
+// The range a call scans for shard `s`; dev: the device bytes of its slice (nullptr: a host slice)
+inline ScanRange scan_range(const Shard &s, uint64_t size, uint64_t match_ptr_base, const void *dev = nullptr) {
+  return ScanRange{dev, s.slice_begin, s.slice_end - s.slice_begin, s.own_begin, s.own_end, size, match_ptr_base};
+}
 
 struct EngineImpl;
 
@@ -38,9 +54,11 @@ struct LinesResult {
   olm_line_t *lines = nullptr;              // lines_only
   uint64_t n_lines = 0, total = 0;          // total: the call's record count
 };
-// Result arrays of the host API: pinned from kPinnedResultMin bytes (freed by host_result_free)
+// Result arrays of the host API (cuda_util.cu): pinned from 1 MiB, freed by host_result_free.
+// host_results: an omega_match_results_t of `count` records (nullptr when out of memory).
 void *host_result_alloc(size_t bytes);
 void host_result_free(void *p);
+omega_match_results_t *host_results(uint64_t count);
 
 class Engine {
 public:
@@ -56,7 +74,8 @@ public:
   // `dev_counts` (the pattern tables loaded: load_pattern_tables) the call adds the count of its
   // final records per pattern to dev_counts[id] instead of writing ids, whether ids are on or off.
   int match_device(const ScanRange &r, const MatchFlags &f, olm_cuda_results_t *out, void *dev_counts = nullptr);
-  // Host input/output: H2D, match_device, D2H into a malloc'ed array.
+  // Host input/output: H2D, match_device, D2H into a host_results array.  One GPU, or
+  // OLM_HOST_SPAN_BYTES spans (host_spans).
   omega_match_results_t *match_host(const uint8_t *haystack, size_t n, const MatchFlags &f);
   // A byte range (range.dev is ignored) whose slice lies in HOST memory: segmented H2D overlapped
   // with the scan, device-resident records.
@@ -76,7 +95,6 @@ public:
   void *ghost_image() const;                 // device image of the reference's scratch buffer (kWindowBytes + 1 bytes) or nullptr
   void *stream() const;                      // the matcher's cudaStream_t
   void *gather_buffer(size_t bytes, size_t *cap = nullptr); // device memory for gathered records (kept until a larger request); *cap = its size
-  int records_to_host(void *host_dst, const void *dev_records, uint64_t count); // asynchronous, on stream()
   int sync();                                // waits for stream()
 
   const olm_cuda_timing_t &timing() const;
@@ -115,7 +133,7 @@ public:
                      const olm_line_origin_t &origin, void *dev_positions, bool tiles_ready = false);
   int matching_lines(const void *dev_positions, uint64_t count, void **dev_lines, uint64_t *n_lines);
   // Host haystack: the records of match_host and their positions, or (lines_only) only the matching
-  // lines; the arrays are host_result_alloc'ed.  One GPU, or OLM_HOST_SPAN_BYTES spans.
+  // lines; the arrays are host_result_alloc'ed.  One GPU, or OLM_HOST_SPAN_BYTES spans (host_spans).
   int lines_host(const uint8_t *haystack, size_t n, const MatchFlags &f, bool lines_only, LinesResult *out);
   // device records + positions -> host arrays, or (lines_only) their matching lines
   int lines_to_host(const void *dev_records, const void *dev_positions, uint64_t count, bool lines_only,
@@ -129,14 +147,33 @@ private:
   int stage_host(const uint8_t *src, size_t n);
   int stage_pageable(const uint8_t *src, size_t n, uint64_t nseg);
   int finish_staging();
-  omega_match_results_t *match_host_spans(const uint8_t *haystack, size_t n, const MatchFlags &f, uint64_t span);
-  int count_host_spans(const uint8_t *haystack, size_t n, const MatchFlags &f, uint64_t span, uint64_t *counts,
-                       uint64_t *total);
-  int lines_host_spans(const uint8_t *haystack, size_t n, const MatchFlags &f, uint64_t span, bool lines_only,
-                       LinesResult *out);
+  // step(span, its device records, several spans)
+  using SpanStep = std::function<int(const Shard &, const olm_cuda_results_t &, bool)>;
+  int host_spans(const uint8_t *haystack, size_t n, const MatchFlags &f, void *dev_counts, const SpanStep &step);
   unsigned long long *zeroed_counts();
   int add_counts_to_host(uint64_t *counts);
   EngineImpl *impl_ = nullptr;
+};
+
+// Pattern ids on for `engines` (their tables loaded) while the guard lives, for a call that needs ids in
+// the pads whatever the caller chose; every engine's own setting comes back on every exit path.
+class PatternIdsOn {
+public:
+  explicit PatternIdsOn(const std::vector<Engine *> &engines, bool on = true) {
+    if (!on) return;
+    for (Engine *e : engines) {
+      saved_.emplace_back(e, e->pattern_ids());
+      e->set_pattern_ids(true, nullptr);
+    }
+  }
+  ~PatternIdsOn() {
+    for (auto &s : saved_) s.first->set_pattern_ids(s.second, nullptr);
+  }
+  PatternIdsOn(const PatternIdsOn &) = delete;
+  PatternIdsOn &operator=(const PatternIdsOn &) = delete;
+
+private:
+  std::vector<std::pair<Engine *, bool>> saved_;
 };
 
 } // namespace olm

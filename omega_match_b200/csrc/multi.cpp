@@ -144,17 +144,9 @@ std::vector<Shard> plan_shards(uint64_t size, int world, uint32_t largest_patter
   const uint64_t unit = windowed ? kWindowBytes : 4096;
   const uint64_t units = (size + unit - 1) / unit;
   for (int r = 0; r < world; ++r) {
-    Shard s;
-    s.own_begin = std::min<uint64_t>(size, units * (uint64_t)r / (uint64_t)world * unit);
-    s.own_end = r + 1 < world ? std::min<uint64_t>(size, units * (uint64_t)(r + 1) / (uint64_t)world * unit) : size;
-    if (windowed) { // windows are independent: no halo at all
-      s.slice_begin = s.own_begin;
-      s.slice_end = s.own_end;
-    } else { // 16 bytes in front (alignment + the previous byte), the longest pattern + 1 behind
-      s.slice_begin = s.own_begin >= 16 ? s.own_begin - 16 : 0;
-      s.slice_end = std::min<uint64_t>(size, s.own_end + largest_pattern + 1);
-    }
-    shards.push_back(s);
+    const uint64_t b = std::min<uint64_t>(size, units * (uint64_t)r / (uint64_t)world * unit);
+    const uint64_t e = r + 1 < world ? std::min<uint64_t>(size, units * (uint64_t)(r + 1) / (uint64_t)world * unit) : size;
+    shards.push_back(shard_of(b, e, size, largest_pattern, windowed));
   }
   return shards;
 }
@@ -186,34 +178,32 @@ MultiMatcher::~MultiMatcher() {
   for (Engine *e : engines_) delete e;
 }
 
-omega_match_results_t *MultiMatcher::match_host(const uint8_t *haystack, size_t n, const MatchFlags &f) {
-  const int N = (int)engines_.size();
-  auto *results = static_cast<omega_match_results_t *>(std::malloc(sizeof(omega_match_results_t)));
-  if (!results) return nullptr;
-  results->count = 0;
-  results->matches = static_cast<omega_match_result_t *>(std::malloc(sizeof(omega_match_result_t)));
+// Starts every host call: clears the last call's state.  An empty haystack, and the stale-tail bytes of
+// SURVEY H6 (2..4 byte patterns of a transforming store under word_boundary: they depend on the windows
+// in front of a window, which a shard does not see), go to `call` -- the same call on the first GPU's
+// engine alone -- after which every engine gets that engine's scratch-buffer image.  Returns true when
+// `call` made the call (*rc: its result), false when the call is to be sharded.
+bool MultiMatcher::first_alone(const uint8_t *haystack, size_t n, const MatchFlags &f, const std::function<int()> &call,
+                               int *rc) {
   last_ = olm_cuda_timing_t{};
-  scanned_.assign(N, false);
-  if (n == 0 || !haystack) return results;
-  auto bail = [&]() -> omega_match_results_t * {
-    if (!pinned_result_release(results->matches)) std::free(results->matches);
-    std::free(results);
-    return nullptr;
-  };
-  // The stale-tail bytes of SURVEY H6 (2..4 byte patterns of a transforming store under word_boundary)
-  // depend on the windows in front of a window -- which a shard does not see.  Such calls run on the
-  // first GPU alone; all other calls shard, and afterwards every engine gets the scratch-buffer image
-  // of the engine that scanned the haystack's last windows.
-  const bool tails = engines_[0]->needs_window_tails();
-  if (tails && f.word_boundary) {
+  scanned_.assign(engines_.size(), false);
+  const bool empty = n == 0 || !haystack;
+  if (!empty && !(engines_[0]->needs_window_tails() && f.word_boundary)) return false;
+  *rc = call();
+  if (!empty) {
     scanned_[0] = true;
-    std::free(results->matches);
-    std::free(results);
-    omega_match_results_t *r = engines_[0]->match_host(haystack, n, f);
     last_ = engines_[0]->timing();
-    if (r) sync_ghost(0);
-    return r;
+    if (*rc == 0) sync_ghost(0);
   }
+  return true;
+}
+
+omega_match_results_t *MultiMatcher::match_host(const uint8_t *haystack, size_t n, const MatchFlags &f) {
+  omega_match_results_t *results = nullptr;
+  int rc = 0;
+  if (first_alone(haystack, n, f, [&] { return (results = engines_[0]->match_host(haystack, n, f)) ? 0 : -1; }, &rc))
+    return results;
+  const int N = (int)engines_.size();
   MatchFlags fs = f;
   fs.no_overlap = false; // crosses shards: once, on the gathered records
   std::vector<olm_cuda_results_t> res(N);
@@ -221,54 +211,21 @@ omega_match_results_t *MultiMatcher::match_host(const uint8_t *haystack, size_t 
   if (run_shards(haystack, n, [&](int g, const uint8_t *slice, const ScanRange &r) {
         return engines_[g]->match_shard_host(slice, r, fs, &res[g]);
       }) != 0)
-    return bail();
+    return nullptr;
   uint64_t total = 0;
-  std::vector<uint64_t> off(N, 0);
-  for (int g = 0; g < N; ++g) {
-    off[g] = total;
-    total += res[g].count;
+  for (const olm_cuda_results_t &r : res) total += r.count;
+  if (f.no_overlap && total > 1) { // the records leave through the first GPU
+    const void *recs = nullptr;
+    const int64_t k = gather_no_overlap(res, total, &recs);
+    if (k < 0) return nullptr;
+    total = uint64_t(k);
+    res.assign(1, olm_cuda_results_t{total, const_cast<void *>(recs), engines_[0]->device()});
   }
-  if (total == 0) return results;
-
-  Engine *E0 = engines_[0];
-  const void *src0 = nullptr; // records that leave through the first GPU (no_overlap)
-  uint64_t kept = total;
-  if (f.no_overlap && total > 1) {
-    const int64_t k = gather_no_overlap(res, total, &src0);
-    if (k < 0) return bail();
-    kept = (uint64_t)k;
-  }
-  std::free(results->matches);
-  const size_t rbytes = std::max<uint64_t>(kept, 1) * sizeof(omega_match_result_t);
-  results->matches = nullptr;
-  if (rbytes >= kPinnedResultMin) results->matches = static_cast<omega_match_result_t *>(pinned_result_alloc(rbytes));
-  if (!results->matches) results->matches = static_cast<omega_match_result_t *>(std::malloc(rbytes));
-  if (!results->matches) {
-    std::free(results);
+  if (!(results = host_results(total))) return nullptr;
+  if (total && copy_out(res, results->matches) != 0) {
+    omega_match_results_destroy(results);
     return nullptr;
   }
-  cudaEvent_t e0 = nullptr, e1 = nullptr;
-  cudaSetDevice(E0->device());
-  cudaEventCreate(&e0);
-  cudaEventCreate(&e1);
-  cudaEventRecord(e0, static_cast<cudaStream_t>(E0->stream()));
-  bool ok = true;
-  if (src0) {
-    ok = E0->records_to_host(results->matches, src0, kept) == 0;
-  } else { // every GPU copies its records into its range of the one array, all links at once
-    for (int g = 0; g < N && ok; ++g)
-      if (res[g].count) ok = engines_[g]->records_to_host(results->matches + off[g], res[g].records, res[g].count) == 0;
-  }
-  for (int g = 0; g < N; ++g)
-    if (engines_[g]->sync() != 0) ok = false;
-  cudaSetDevice(E0->device());
-  cudaEventRecord(e1, static_cast<cudaStream_t>(E0->stream()));
-  cudaEventSynchronize(e1);
-  cudaEventElapsedTime(&last_.d2h_ms, e0, e1);
-  cudaEventDestroy(e0);
-  cudaEventDestroy(e1);
-  if (!ok) return bail();
-  results->count = kept;
   return results;
 }
 
@@ -288,15 +245,7 @@ int MultiMatcher::run_shards(const uint8_t *haystack, size_t n,
       if (s.own_end <= s.own_begin) continue;
       scanned_[g] = true;
       th.emplace_back([&, g]() {
-        const Shard &sh = plan[g];
-        ScanRange r;
-        r.slice_begin = sh.slice_begin;
-        r.slice_len = sh.slice_end - sh.slice_begin;
-        r.own_begin = sh.own_begin;
-        r.own_end = sh.own_end;
-        r.global_size = n;
-        r.match_ptr_base = reinterpret_cast<uint64_t>(haystack);
-        rc[g] = scan(g, haystack + sh.slice_begin, r);
+        rc[g] = scan(g, haystack + plan[g].slice_begin, scan_range(plan[g], n, reinterpret_cast<uint64_t>(haystack)));
       });
     }
     for (auto &t : th) t.join();
@@ -351,19 +300,39 @@ int64_t MultiMatcher::gather_no_overlap(const std::vector<olm_cuda_results_t> &r
   return k;
 }
 
+// Every GPU copies its records res[g] (and with `positions`, positions[g]) into its range of the host
+// arrays, all links at once (res: in shard order); d2h_ms spans all the copies.
+int MultiMatcher::copy_out(const std::vector<olm_cuda_results_t> &res, omega_match_result_t *dst,
+                           const std::vector<void *> *positions, olm_line_pos_t *pos_dst) {
+  Engine *E0 = engines_[0];
+  cudaEvent_t e0 = nullptr, e1 = nullptr;
+  cudaSetDevice(E0->device());
+  cudaEventCreate(&e0);
+  cudaEventCreate(&e1);
+  cudaEventRecord(e0, static_cast<cudaStream_t>(E0->stream()));
+  bool ok = true;
+  uint64_t off = 0;
+  for (size_t g = 0; g < res.size() && ok; off += res[g].count, ++g)
+    if (res[g].count)
+      ok = engines_[g]->copy_to_host(dst + off, res[g].records, res[g].count * sizeof(Record)) == 0 &&
+           (!positions || engines_[g]->copy_to_host(pos_dst + off, (*positions)[g], res[g].count * sizeof(olm_line_pos_t)) == 0);
+  for (Engine *e : engines_)
+    if (e->sync() != 0) ok = false;
+  cudaSetDevice(E0->device());
+  cudaEventRecord(e1, static_cast<cudaStream_t>(E0->stream()));
+  cudaEventSynchronize(e1);
+  cudaEventElapsedTime(&last_.d2h_ms, e0, e1);
+  cudaEventDestroy(e0);
+  cudaEventDestroy(e1);
+  return ok ? 0 : -1;
+}
+
 int MultiMatcher::lines_host(const uint8_t *haystack, size_t n, const MatchFlags &f, bool lines_only, LinesResult *out) {
-  const int N = (int)engines_.size();
   *out = LinesResult{};
-  last_ = olm_cuda_timing_t{};
-  scanned_.assign(N, false);
-  if (n == 0 || !haystack) return engines_[0]->lines_host(haystack, n, f, lines_only, out);
-  if (engines_[0]->needs_window_tails() && f.word_boundary) { // (as match_host)
-    scanned_[0] = true;
-    const int rc = engines_[0]->lines_host(haystack, n, f, lines_only, out);
-    last_ = engines_[0]->timing();
-    if (rc == 0) sync_ghost(0);
+  int rc = 0;
+  if (first_alone(haystack, n, f, [&] { return engines_[0]->lines_host(haystack, n, f, lines_only, out); }, &rc))
     return rc;
-  }
+  const int N = (int)engines_.size();
   MatchFlags fs = f;
   fs.no_overlap = false;
   std::vector<olm_cuda_results_t> res(N);
@@ -394,7 +363,7 @@ int MultiMatcher::lines_host(const uint8_t *haystack, size_t n, const MatchFlags
     if (facts[g].newlines) next = own_begin[g] + facts[g].first;
   }
   std::vector<void *> pos(N, nullptr);
-  std::vector<int> rc(N, 0);
+  std::vector<int> failed(N, 0);
   {
     std::vector<std::thread> th;
     for (int g = 0; g < N; ++g) {
@@ -403,17 +372,15 @@ int MultiMatcher::lines_host(const uint8_t *haystack, size_t n, const MatchFlags
         Engine *e = engines_[g];
         const uint8_t *own = static_cast<const uint8_t *>(e->resident_haystack()) + (own_begin[g] - slice_begin[g]);
         pos[g] = e->positions_buffer(res[g].count * sizeof(olm_line_pos_t), 0);
-        rc[g] = !pos[g] || e->line_positions(res[g].records, res[g].count, own, own_begin[g], own_end[g] - own_begin[g],
-                                             origin[g], pos[g], true) != 0;
+        failed[g] = !pos[g] || e->line_positions(res[g].records, res[g].count, own, own_begin[g], own_end[g] - own_begin[g],
+                                                 origin[g], pos[g], true) != 0;
       });
     }
     for (auto &t : th) t.join();
   }
   uint64_t total = 0;
-  std::vector<uint64_t> off(N, 0);
   for (int g = 0; g < N; ++g) {
-    if (rc[g]) return -1;
-    off[g] = total;
+    if (failed[g]) return -1;
     total += res[g].count;
     last_.total_ms = std::max(last_.total_ms, engines_[g]->timing().total_ms);
   }
@@ -447,38 +414,21 @@ int MultiMatcher::lines_host(const uint8_t *haystack, size_t n, const MatchFlags
     out->n_lines = all.size();
     return 0;
   }
-  out->results = static_cast<omega_match_results_t *>(std::malloc(sizeof(omega_match_results_t)));
-  if (!out->results) return -1;
-  out->results->count = total;
-  out->results->matches = static_cast<omega_match_result_t *>(host_result_alloc(total * sizeof(omega_match_result_t)));
+  out->results = host_results(total);
   out->positions = static_cast<olm_line_pos_t *>(host_result_alloc(total * sizeof(olm_line_pos_t)));
-  if (!out->results->matches || !out->positions) return -1;
-  bool ok = true; // every GPU copies into its range of the arrays, all links at once
-  for (int g = 0; g < N && ok; ++g)
-    if (res[g].count)
-      ok = engines_[g]->records_to_host(out->results->matches + off[g], res[g].records, res[g].count) == 0 &&
-           engines_[g]->copy_to_host(out->positions + off[g], pos[g], res[g].count * sizeof(olm_line_pos_t)) == 0;
-  for (int g = 0; g < N; ++g)
-    if (engines_[g]->sync() != 0) ok = false;
-  return ok ? 0 : -1;
+  if (!out->results || !out->positions) return -1;
+  return total ? copy_out(res, out->results->matches, &pos, out->positions) : 0;
 }
 
 // match_host() counting (include/olm_b200.h olm_cuda_count_patterns).  Without no_overlap every GPU
 // counts its shard and the counts are summed on the host: no record moves.  With it the shards write
 // ids, the gather and the filter run as in match_host, and the first GPU counts the pads.
 int MultiMatcher::count_host(const uint8_t *haystack, size_t n, const MatchFlags &f, uint64_t *counts, uint64_t *total) {
-  const int N = (int)engines_.size();
-  last_ = olm_cuda_timing_t{};
-  scanned_.assign(N, false);
   *total = 0;
-  if (n == 0 || !haystack) return 0;
-  if (engines_[0]->needs_window_tails() && f.word_boundary) { // (as match_host)
-    scanned_[0] = true;
-    const int rc = engines_[0]->count_host(haystack, n, f, counts, total);
-    last_ = engines_[0]->timing();
-    if (rc == 0) sync_ghost(0);
+  int rc = 0;
+  if (first_alone(haystack, n, f, [&] { return engines_[0]->count_host(haystack, n, f, counts, total); }, &rc))
     return rc;
-  }
+  const int N = (int)engines_.size();
   MatchFlags fs = f;
   fs.no_overlap = false;
   const uint64_t P = engines_[0]->pattern_count();
@@ -499,17 +449,12 @@ int MultiMatcher::count_host(const uint8_t *haystack, size_t n, const MatchFlags
     return 0;
   }
   std::vector<olm_cuda_results_t> res(N);
-  std::vector<bool> ids_were(N);
-  for (int g = 0; g < N; ++g) {
-    res[g] = olm_cuda_results_t{0, nullptr, engines_[g]->device()};
-    ids_were[g] = engines_[g]->pattern_ids();
-    engines_[g]->set_pattern_ids(true, nullptr); // (the tables are loaded)
-  }
-  int rc = run_shards(haystack, n, [&](int g, const uint8_t *slice, const ScanRange &r) {
-    return engines_[g]->match_shard_host(slice, r, fs, &res[g]);
-  });
-  for (int g = 0; g < N; ++g) engines_[g]->set_pattern_ids(ids_were[g], nullptr);
-  if (rc != 0) return -1;
+  for (int g = 0; g < N; ++g) res[g] = olm_cuda_results_t{0, nullptr, engines_[g]->device()};
+  PatternIdsOn ids(engines_);
+  if (run_shards(haystack, n, [&](int g, const uint8_t *slice, const ScanRange &r) {
+        return engines_[g]->match_shard_host(slice, r, fs, &res[g]);
+      }) != 0)
+    return -1;
   uint64_t all = 0;
   for (const olm_cuda_results_t &r : res) all += r.count;
   if (all > 1) {

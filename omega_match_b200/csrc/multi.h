@@ -15,12 +15,8 @@ namespace olm {
 // that does not exist
 std::vector<int> parse_device_list(const char *spec, int n_devices);
 
-// Byte-range shards of one haystack (SURVEY 8e): rank r OWNS the start positions [own_begin,
-// own_end) and needs the bytes [slice_begin, slice_end).  Stores with a transform flag shard on
-// multiples of the 4 MiB source window and need no halo.
-struct Shard {
-  uint64_t own_begin = 0, own_end = 0, slice_begin = 0, slice_end = 0;
-};
+// Byte-range shards of one haystack (SURVEY 8e, shard_of): rank r owns the r-th of `world` runs of
+// 4 KiB units (stores with a transform flag: 4 MiB windows).
 std::vector<Shard> plan_shards(uint64_t size, int world, uint32_t largest_pattern, bool windowed);
 
 class MultiMatcher {
@@ -42,10 +38,13 @@ public:
   int size() const { return (int)engines_.size(); }
 
 private:
+  bool first_alone(const uint8_t *haystack, size_t n, const MatchFlags &f, const std::function<int()> &call, int *rc);
   void sync_ghost(int from);
   int run_shards(const uint8_t *haystack, size_t n, const std::function<int(int, const uint8_t *, const ScanRange &)> &scan);
   int64_t gather_no_overlap(const std::vector<olm_cuda_results_t> &res, uint64_t total, const void **dst,
                             const std::vector<void *> *positions = nullptr, void **pos_dst = nullptr);
+  int copy_out(const std::vector<olm_cuda_results_t> &res, omega_match_result_t *dst,
+               const std::vector<void *> *positions = nullptr, olm_line_pos_t *pos_dst = nullptr);
   std::vector<Engine *> engines_;
   std::vector<bool> scanned_; // engines that took part in the last call
   olm_cuda_timing_t last_{};

@@ -1,8 +1,7 @@
 #!/usr/bin/env python3
 """GPU-box checker for the opt-in span path of the host entry point (OLM_HOST_SPAN_BYTES;
-engine.cu `match_host_spans`): a host haystack scanned as consecutive byte-range shards, records
-concatenated, `no_overlap` once on the whole.  Not collected by pytest: written after this round's
-GPU budget was spent, so it has not run on a GPU yet.
+engine.cu `host_spans`): a host haystack scanned as consecutive byte-range shards, records
+concatenated, `no_overlap` once on the whole.  Not collected by pytest.
 
   python tests/gpu_span_check.py        # spans of 4 MiB over 9..21 MiB haystacks vs the oracle
 """

@@ -91,7 +91,7 @@ def test_perf_matrix_on_census_at_16mib(store_cache):
 
 def test_host_span_path(store_cache, monkeypatch):
     """OLM_HOST_SPAN_BYTES: omega_list_matcher_match scans a host haystack as consecutive byte-range
-    shards of that many start positions (engine.cu match_host_spans): matches written across every
+    shards of that many start positions (engine.cu host_spans): matches written across every
     span edge, plain and transforming stores, no_overlap across span edges, exact statistics summed."""
     monkeypatch.setenv("OLM_HOST_SPAN_BYTES", str(4 * MIB))
     names = inputs.case_patterns(dict(patterns="names", store_flags=(0, 0, 0)))

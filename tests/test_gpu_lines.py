@@ -15,6 +15,7 @@ from omega_match_b200 import Matcher
 from omega_match_b200.omega_match import LINE_POS_DTYPE, _flag_ints
 from omega_match_b200.sharding import line_origins, shard_plan
 from oracle.oracle import Oracle
+from test_gpu_multi import _devices
 from test_gpu_pattern_ids import EDGE_FLAGSETS
 from test_lines_cpu import positions
 
@@ -172,30 +173,21 @@ def test_host_span_path(store_cache, monkeypatch):
         monkeypatch.delenv("OLM_HOST_SPAN_BYTES")
 
 
-def _multi_ok():
-    from omega_match_b200 import _lib
-    return _lib.load().olm_cuda_device_count() >= 2
-
-
 @pytest.mark.parametrize("sf", [(0, 0, 0), (1, 1, 1)])
 def test_multi_matcher_lines(store_cache, sf):
-    if not _multi_ok():
-        pytest.skip("needs 2 GPUs")
     names = inputs.case_patterns(dict(patterns="names", store_flags=sf))
     path = store_cache("multi-names", names, sf)
     hay = _span_haystack(13 * MIB + 4321, 31)
-    with Matcher(path) as one, Matcher(path, devices=[0, 1]) as many:
+    with Matcher(path) as one, Matcher(path, devices=_devices(2)) as many:
         for kw in ({}, {"no_overlap": True}, {"longest_only": True, "no_overlap": True}):
             _check(many, hay, one.match_arrays(hay, **kw), f"multi {sf}", **kw)
 
 
 def test_multi_matcher_lines_with_window_tails(store_cache):
-    if not _multi_ok():
-        pytest.skip("needs 2 GPUs")
     sf = (1, 1, 1)
     path = store_cache("counts-tails", b"\n".join([b"ab", b"the", b"king", b"lord", b"of", b"and", b"jesus"]), sf)
     hay = inputs.text_haystack(9 * 4 * MIB + 77, 3).tobytes()
-    with Matcher(path) as one, Matcher(path, devices=[0, 1]) as many:
+    with Matcher(path) as one, Matcher(path, devices=_devices(2)) as many:
         for kw in ({"word_boundary": True}, {"word_boundary": True, "longest_only": True, "no_overlap": True}):
             _check(many, hay, one.match_arrays(hay, **kw), "tails", **kw)
 

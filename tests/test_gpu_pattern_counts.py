@@ -15,6 +15,7 @@ from omega_match_b200 import Compiler, Matcher
 from omega_match_b200.omega_match import _flag_ints
 from omega_match_b200.sharding import WINDOW, shard_plan
 from oracle.oracle import Oracle
+from test_gpu_multi import _devices
 from test_gpu_pattern_ids import EDGE_FLAGSETS, _bucket_records, _device_ids, _normalised_span
 
 pytestmark = pytest.mark.gpu
@@ -297,13 +298,10 @@ def test_host_span_path_counts(store_cache, monkeypatch):
 
 @pytest.mark.parametrize("sf", [(0, 0, 0), (1, 1, 1)])
 def test_multi_matcher_counts(store_cache, sf):
-    from omega_match_b200 import _lib
-    if _lib.load().olm_cuda_device_count() < 2:
-        pytest.skip("needs 2 GPUs")
     names = inputs.case_patterns(dict(patterns="names", store_flags=sf))
     path = store_cache("multi-names", names, sf)
     hay = inputs.text_haystack(13 * MIB + 4321, 31 + sum(sf)).tobytes()
-    with Matcher(path) as one, Matcher(path, devices=[0, 1]) as many:
+    with Matcher(path) as one, Matcher(path, devices=_devices(2)) as many:
         for kw in ({}, {"no_overlap": True}, {"longest_only": True, "no_overlap": True}):
             want = _oracle_only(one, path, hay, sf, **kw)
             counts = np.zeros(many.pattern_count, dtype=np.uint64)
@@ -313,14 +311,11 @@ def test_multi_matcher_counts(store_cache, sf):
 
 def test_multi_matcher_counts_with_window_tails(store_cache):
     """A transforming store with 2..4 byte patterns under word_boundary runs on the first GPU alone."""
-    from omega_match_b200 import _lib
-    if _lib.load().olm_cuda_device_count() < 2:
-        pytest.skip("needs 2 GPUs")
     sf = (1, 1, 1)
     pats = [b"ab", b"the", b"king", b"lord", b"of", b"and", b"jesus"]
     path = store_cache("counts-tails", b"\n".join(pats), sf)
     hay = inputs.text_haystack(9 * WINDOW + 77, 3).tobytes()
-    with Matcher(path) as one, Matcher(path, devices=[0, 1]) as many:
+    with Matcher(path) as one, Matcher(path, devices=_devices(2)) as many:
         for kw in ({"word_boundary": True}, {"word_boundary": True, "longest_only": True, "no_overlap": True}):
             want = _oracle_only(one, path, hay, sf, **kw)
             assert want.sum() > 0

@@ -16,6 +16,7 @@ from conftest import describe_diff, same_matches
 from omega_match_b200 import MATCH_IDS_DTYPE, Compiler, Matcher
 from omega_match_b200.sharding import WINDOW, shard_plan
 from oracle.oracle import Oracle
+from test_gpu_multi import _devices
 from test_gpu_parity import _colliding_patterns
 
 pytestmark = pytest.mark.gpu
@@ -311,13 +312,10 @@ def test_host_span_path_carries_ids(store_cache, monkeypatch):
 
 @pytest.mark.parametrize("sf", [(0, 0, 0), (1, 1, 1)])
 def test_multi_matcher_carries_ids(store_cache, sf):
-    from omega_match_b200 import _lib
-    if _lib.load().olm_cuda_device_count() < 2:
-        pytest.skip("needs 2 GPUs")
     names = inputs.case_patterns(dict(patterns="names", store_flags=sf))
     path = store_cache("multi-names", names, sf)
     hay = inputs.text_haystack(13 * MIB + 4321, 31 + sum(sf)).tobytes()
-    with Matcher(path) as one, Matcher(path, devices=[0, 1]) as many:
+    with Matcher(path) as one, Matcher(path, devices=_devices(2)) as many:
         for kw in ({}, {"no_overlap": True}, {"longest_only": True, "no_overlap": True}):
             want = one.match_ids(hay, **kw)
             assert many.match_ids(hay, **kw).tobytes() == want.tobytes(), f"{sf} {kw}"
