@@ -429,6 +429,69 @@ int olm_cuda_matching_lines_device(const omega_list_matcher_t *matcher, const vo
 /* olm_cuda_gather_records does not carry positions: gather the records, or compute the positions
  * per shard and move them by the job's own means. */
 
+/* Streams: one haystack that arrives in pieces -- a pipe, a log still being written, a file read in
+ * blocks, or bytes a GPU producer writes into a reused device buffer.
+ *
+ * A stream is opened on a matcher with the seven match flags and `match_ptr_base`; the caller then
+ * pushes consecutive pieces of one haystack (host bytes, device bytes, or a mix), the last push
+ * saying it is the last.
+ *   - Equivalence: the records of all pushes, concatenated in push order, are those of
+ *     omega_list_matcher_match over the concatenated pieces with the same flags -- the same offsets
+ *     and lengths in the same order, with ids when ids are on.  One exception: the stale-tail bytes
+ *     (2..4 byte patterns of a transforming store under word_boundary at the very end of a 4 MiB
+ *     window) evolve as in one call only if no other call on the matcher runs between the pushes,
+ *     the condition the reference's own scratch buffer sets.
+ *   - Offsets are global, counted from the stream's first byte, and 64-bit;
+ *     record.match = match_ptr_base + offset (a caller that mapped the whole file passes the
+ *     mapping's address).
+ *   - Settling: after each push the stream reports `received` (bytes pushed so far) and `settled`:
+ *     every record that starts before `settled` has been returned, by this push or an earlier one,
+ *     and no later push returns one that starts there.  Stores without a transform flag:
+ *     settled = max(previous, received - (largest + 1)), where a value below 16 counts as 0 (a
+ *     scan needs 16 bytes in front of its first position).  Stores with a transform flag:
+ *     settled = floor(received / 4 MiB) * 4 MiB.  After the last push settled = received.  The
+ *     end-of-haystack predicates therefore never see the stream's end early.
+ *   - no_overlap carries across pushes (the filter starts from the end of the last kept record);
+ *     longest_only needs nothing carried: records that share an offset settle in the same push.
+ *   - Pieces may be empty, 1 byte long, or cut anywhere (inside a match, inside "\r\n", on a
+ *     window edge).  The stream keeps no pointer to a pushed buffer after the push returns.
+ *   - Statistics attached to the matcher are added to by every push; summed over the pushes they
+ *     equal one call's, exact statistics too.  olm_cuda_last_timing reports the last push, summed
+ *     over its internal calls.
+ *   - Errors return -1 or NULL with a message on stderr: a push after the last one, a NULL
+ *     argument, a CUDA failure; after a failure only close is valid.  Several streams may be open on
+ *     one matcher; their pushes interleave like any other calls.  Close a stream before its matcher
+ *     is destroyed.  On a multi-GPU matcher the stream runs on the first GPU.
+ * Each push scans its settled positions as a byte-range shard of the whole stream.  The stream
+ * carries a small device buffer: the last settled position's 16 bytes in front and what follows it
+ * (at most largest + 17 bytes), or the incomplete 4 MiB window of a transforming store.  Device
+ * pieces of a store without a transform flag (16-byte aligned, readable to the next multiple of 16)
+ * are scanned in place; only the positions up to the piece's 16th byte are scanned from the carried
+ * bytes.  Other pieces are copied behind the carried bytes. */
+typedef struct olm_cuda_stream olm_cuda_stream_t;
+olm_cuda_stream_t *olm_cuda_stream_open(const omega_list_matcher_t *matcher, int no_overlap, int longest_only,
+                                        int word_boundary, int word_prefix, int word_suffix, int line_start,
+                                        int line_end, const void *match_ptr_base);
+/* host bytes -> the records this push settled (destroy with omega_match_results_destroy; never NULL
+ * on success) */
+int olm_cuda_stream_push(olm_cuda_stream_t *s, const uint8_t *bytes, size_t n, int last,
+                         omega_match_results_t **results);
+/* device bytes (the contract of olm_cuda_match_device) -> device records, valid until the next call
+ * on the matcher */
+int olm_cuda_stream_push_device(olm_cuda_stream_t *s, const void *dev_bytes, size_t n, int last,
+                                olm_cuda_results_t *out);
+/* host bytes -> counts[id] += the settled records of pattern id, *total = their number; the records
+ * stay on the GPU (counts as olm_cuda_count_patterns takes them).  Counting device records:
+ * olm_cuda_stream_push_device with ids on, then olm_cuda_count_records. */
+int olm_cuda_stream_count(olm_cuda_stream_t *s, const uint8_t *bytes, size_t n, int last, uint64_t *counts,
+                          uint64_t *total);
+typedef struct {
+  uint64_t received, settled;
+  int finished;
+} olm_cuda_stream_state_t;
+int olm_cuda_stream_state(const olm_cuda_stream_t *s, olm_cuda_stream_state_t *out);
+int olm_cuda_stream_close(olm_cuda_stream_t *s);
+
 /* Pinned host memory helpers (so callers can hand DMA-able buffers to _match). */
 void *olm_cuda_host_alloc(size_t bytes);
 void olm_cuda_host_free(void *p);

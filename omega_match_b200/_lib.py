@@ -60,6 +60,10 @@ class LineOriginC(C.Structure):  # olm_line_origin_t
     _fields_ = [(n, C.c_uint64) for n in ("line", "begin", "next_newline")]
 
 
+class StreamStateC(C.Structure):  # olm_cuda_stream_state_t
+    _fields_ = [("received", C.c_uint64), ("settled", C.c_uint64), ("finished", C.c_int)]
+
+
 class StoreInfoC(C.Structure):
     _fields_ = [(n, C.c_uint32) for n in ("flags", "smallest", "largest", "stored_patterns", "table_size",
                                          "occupied_buckets", "len1", "len2", "len3", "len4")] + [
@@ -137,6 +141,12 @@ ABI = [
     ("olm_cuda_line_positions", _ci, [_vp, _vp, C.c_uint64, _vp, C.c_uint64, C.c_uint64, C.POINTER(LineOriginC), _vp]),
     ("olm_cuda_newline_facts", _ci, [_vp, _vp, C.c_uint64, C.POINTER(NewlineFactsC)]),
     ("olm_cuda_matching_lines_device", _ci, [_vp, _vp, C.c_uint64, C.POINTER(_vp), C.POINTER(C.c_uint64)]),
+    ("olm_cuda_stream_open", _vp, [_vp] + _flags7 + [_vp]),
+    ("olm_cuda_stream_push", _ci, [_vp, _vp, C.c_size_t, _ci, C.POINTER(C.POINTER(MatchResultsC))]),
+    ("olm_cuda_stream_push_device", _ci, [_vp, _vp, C.c_size_t, _ci, C.POINTER(CudaResultsC)]),
+    ("olm_cuda_stream_count", _ci, [_vp, _vp, C.c_size_t, _ci, _vp, C.POINTER(C.c_uint64)]),
+    ("olm_cuda_stream_state", _ci, [_vp, C.POINTER(StreamStateC)]),
+    ("olm_cuda_stream_close", _ci, [_vp]),
     ("olm_cuda_host_alloc", _vp, [C.c_size_t]),
     ("olm_cuda_host_free", None, [_vp]),
     ("olm_store_inspect", _ci, [_cp, C.POINTER(StoreInfoC)]),

@@ -519,6 +519,77 @@ int olm_cuda_matching_lines_device(const omega_list_matcher_t *m, const void *de
   return m->engine->matching_lines(dev_positions, count, dev_lines, n_lines);
 }
 
+struct olm_cuda_stream {
+  const omega_list_matcher_t *m = nullptr;
+  olm::StreamState st;
+};
+
+olm_cuda_stream_t *olm_cuda_stream_open(const omega_list_matcher_t *m, int no_overlap, int longest_only,
+                                        int word_boundary, int word_prefix, int word_suffix, int line_start,
+                                        int line_end, const void *match_ptr_base) {
+  if (!m || !m->engine) return nullptr;
+  auto *s = new olm_cuda_stream();
+  s->m = m;
+  s->st.f = to_flags(no_overlap, longest_only, word_boundary, word_prefix, word_suffix, line_start, line_end);
+  s->st.match_ptr_base = reinterpret_cast<uint64_t>(match_ptr_base);
+  return s;
+}
+
+namespace {
+int stream_push(olm_cuda_stream_t *s, const void *bytes, size_t n, bool on_device, int last, olm_cuda_results_t *out,
+                uint64_t *counts = nullptr) {
+  const int rc = s->m->engine->stream_push(s->st, bytes, n, on_device, last != 0, out, counts);
+  if (rc == 0 && s->m->stats) s->m->engine->collect_stats(s->m->stats);
+  return rc;
+}
+} // namespace
+
+int olm_cuda_stream_push(olm_cuda_stream_t *s, const uint8_t *bytes, size_t n, int last,
+                         omega_match_results_t **results) {
+  if (!s || (!results && null_output("olm_cuda_stream_push"))) return -1;
+  *results = nullptr;
+  olm_cuda_results_t d;
+  if (stream_push(s, bytes, n, false, last, &d) != 0) return -1;
+  omega_match_results_t *r = olm::host_results(d.count);
+  olm::Engine *e = s->m->engine;
+  if (!r || e->copy_to_host(r->matches, d.records, d.count * sizeof(omega_match_result_t)) != 0 || e->sync() != 0) {
+    omega_match_results_destroy(r);
+    s->st.failed = true;
+    return -1;
+  }
+  *results = r;
+  return 0;
+}
+
+int olm_cuda_stream_push_device(olm_cuda_stream_t *s, const void *dev_bytes, size_t n, int last,
+                                olm_cuda_results_t *out) {
+  if (!s || (!out && null_output("olm_cuda_stream_push_device"))) return -1;
+  return stream_push(s, dev_bytes, n, true, last, out);
+}
+
+int olm_cuda_stream_count(olm_cuda_stream_t *s, const uint8_t *bytes, size_t n, int last, uint64_t *counts,
+                          uint64_t *total) {
+  if (!s || ((!counts || !total) && null_output("olm_cuda_stream_count"))) return -1;
+  if (load_pattern_tables(s->m)) return -1;
+  olm_cuda_results_t d;
+  if (stream_push(s, bytes, n, false, last, &d, counts) != 0) return -1;
+  *total = d.count;
+  return 0;
+}
+
+int olm_cuda_stream_state(const olm_cuda_stream_t *s, olm_cuda_stream_state_t *out) {
+  if (!s || !out) return -1;
+  *out = olm_cuda_stream_state_t{s->st.received, s->st.settled, s->st.finished ? 1 : 0};
+  return 0;
+}
+
+int olm_cuda_stream_close(olm_cuda_stream_t *s) {
+  if (!s) return -1;
+  s->m->engine->stream_release(s->st);
+  delete s;
+  return 0;
+}
+
 int olm_cuda_last_timing(const omega_list_matcher_t *m, olm_cuda_timing_t *out) {
   if (!m || !m->engine || !out) return -1;
   *out = m->multi ? m->multi->timing() : m->engine->timing();

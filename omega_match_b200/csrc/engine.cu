@@ -122,6 +122,7 @@ struct EngineImpl {
   // [0, (i+1) * seg_bytes) are in HBM (empty = everything is resident already)
   std::vector<cudaEvent_t> seg_events;
   uint64_t seg_bytes = 0;
+  uint64_t seg_off = 0;  // bytes of the slice in front of the staged ones (a stream's carried bytes)
   size_t seg_waited = 0; // segment events of this call the stream already waits for
   bool streaming = false; // set by match_host around its call of match_device
   Header hdr;
@@ -183,6 +184,7 @@ MiscWords *misc_words(EngineImpl &E) {
 }
 // index of the event after which the first `bytes` bytes of the slice are in HBM
 size_t seg_event_for(const EngineImpl &E, uint64_t bytes) {
+  bytes = bytes > E.seg_off ? bytes - E.seg_off : 0;
   if (E.seg_events.size() <= 1 || E.seg_bytes == 0 || bytes == 0) return 0;
   return std::min<size_t>(E.seg_events.size() - 1, size_t((bytes - 1) / E.seg_bytes));
 }
@@ -374,6 +376,10 @@ int Engine::match_device(const ScanRange &r, const MatchFlags &f, olm_cuda_resul
       return -1;
     }
   }
+  if (r.out_front && f.no_overlap) {
+    std::fprintf(stderr, "libomega_match(b200): internal error: room in front of a filtered output\n");
+    return -1;
+  }
   const uint64_t n_own = r.own_end - r.own_begin;
   if (n_own == 0) return 0;
 
@@ -424,8 +430,9 @@ int Engine::match_device(const ScanRange &r, const MatchFlags &f, olm_cuda_resul
     }
   }
 
+  const uint64_t front = r.out_front;
   uint64_t cap = std::max<uint64_t>(E.out_hint, n_own / 64 + 4096);
-  if (E.out.cap / sizeof(Record) >= cap) cap = E.out.cap / sizeof(Record);
+  if (E.out.cap / sizeof(Record) >= cap + front) cap = E.out.cap / sizeof(Record) - front;
 
   uint32_t fl = 0;
   if (f.word_boundary) fl |= kWordBoundary;
@@ -441,8 +448,8 @@ int Engine::match_device(const ScanRange &r, const MatchFlags &f, olm_cuda_resul
   unsigned long long total = 0, temp_used = 0;
   uint64_t temp_extra = 0; // grows when the block allocator of temp[] wasted more than the slack
   for (int attempt = 0; attempt < 4; ++attempt) {
-    if (E.out.ensure(cap * sizeof(Record))) return -1;
-    cap = E.out.cap / sizeof(Record);
+    if (E.out.ensure((cap + front) * sizeof(Record))) return -1;
+    cap = E.out.cap / sizeof(Record) - front;
     const uint64_t temp_cap = cap + cap / 2 + temp_slack_entries(E.sms) * n_batches + temp_extra;
     if (temp_cap > 0xFFFFFFF0ull) { // chunk descriptors index temp[] with 32 bits
       std::fprintf(stderr, "libomega_match(b200): too many matches for one call\n");
@@ -463,7 +470,7 @@ int Engine::match_device(const ScanRange &r, const MatchFlags &f, olm_cuda_resul
     P.temp = static_cast<uint32_t *>(E.temp.p);
     P.temp_cap = temp_cap;
     P.temp_count = d_temp_count;
-    P.out = static_cast<Record *>(E.out.p);
+    P.out = static_cast<Record *>(E.out.p) + front;
     P.out_cap = cap;
     P.match_ptr_base = r.match_ptr_base;
     P.total = d_total;
@@ -570,14 +577,14 @@ int Engine::match_device(const ScanRange &r, const MatchFlags &f, olm_cuda_resul
   E.last.scan_ms = ms;
   E.last.total_ms = ms;
 
-  void *final_records = E.out.p;
-  if (f.no_overlap && total > 1) {
+  void *final_records = static_cast<Record *>(E.out.p) + front;
+  if (f.no_overlap && total > (r.floor ? 0 : 1)) {
     if (E.out2.ensure(total * sizeof(Record))) return -1;
     if (E.fscratch.ensure(filter_scratch_bytes(total))) return -1;
     uint32_t launches = 0;
     OLM_CUDA(cudaEventRecord(E.ev[2], E.stream));
     OLM_CUDA(no_overlap_launch(static_cast<const Record *>(E.out.p), total, static_cast<Record *>(E.out2.p),
-                               E.fscratch.p, &w->scan.filter_total, E.stream, &launches));
+                               E.fscratch.p, &w->scan.filter_total, E.stream, &launches, r.floor));
     OLM_CUDA(cudaEventRecord(E.ev[3], E.stream));
     OLM_CUDA(cudaMemcpyAsync(&total, &w->scan.filter_total, sizeof total, cudaMemcpyDeviceToHost, E.stream));
     OLM_CUDA(cudaStreamSynchronize(E.stream));
@@ -629,9 +636,9 @@ int Engine::match_device(const ScanRange &r, const MatchFlags &f, olm_cuda_resul
 // H2D of `n` host bytes into the engine's haystack buffer: long inputs arrive in 256 MiB segments
 // on the copy stream while earlier segments are being scanned (match_device waits on the segment
 // events); short ones in one copy.  ev[4]/ev[5] bracket the copies.
-int Engine::stage_host(const uint8_t *src, size_t n) {
+int Engine::stage_host(const uint8_t *src, size_t n, size_t dst_off) {
   EngineImpl &E = *impl_;
-  const size_t padded = ((n + 15) & ~size_t(15)) + 256;
+  const size_t padded = ((dst_off + n + 15) & ~size_t(15)) + 256;
   if (E.hay.ensure(padded)) return -1;
   const uint64_t nseg = n >= kPipelineMin ? (n + kSegmentBytes - 1) / kSegmentBytes : 1;
   while (E.seg_events.size() < nseg) {
@@ -644,6 +651,7 @@ int Engine::stage_host(const uint8_t *src, size_t n) {
     E.seg_events.pop_back();
   }
   E.seg_bytes = nseg > 1 ? kSegmentBytes : 0;
+  E.seg_off = dst_off;
   E.seg_waited = 0;
   OLM_CUDA(cudaEventRecord(E.ev[4], E.copy_stream));
   {
@@ -651,11 +659,12 @@ int Engine::stage_host(const uint8_t *src, size_t n) {
     const bool pinned = cudaPointerGetAttributes(&attr, src) == cudaSuccess &&
                         (attr.type == cudaMemoryTypeHost || attr.type == cudaMemoryTypeManaged);
     cudaGetLastError();
-    if (!pinned && n >= 4 * kPieceBytes) return stage_pageable(src, n, nseg);
+    if (!pinned && n >= 4 * kPieceBytes) return stage_pageable(src, n, nseg, dst_off);
   }
   for (uint64_t i = 0; i < nseg; ++i) {
     const uint64_t b = i * kSegmentBytes, e = nseg > 1 ? std::min<uint64_t>(n, b + kSegmentBytes) : n;
-    OLM_CUDA(cudaMemcpyAsync(static_cast<uint8_t *>(E.hay.p) + b, src + b, e - b, cudaMemcpyHostToDevice, E.copy_stream));
+    OLM_CUDA(cudaMemcpyAsync(static_cast<uint8_t *>(E.hay.p) + dst_off + b, src + b, e - b, cudaMemcpyHostToDevice,
+                             E.copy_stream));
     OLM_CUDA(cudaEventRecord(E.seg_events[i], E.copy_stream));
   }
   OLM_CUDA(cudaEventRecord(E.ev[5], E.copy_stream));
@@ -664,7 +673,7 @@ int Engine::stage_host(const uint8_t *src, size_t n) {
 
 // Pageable memory: see Stager.  Returns after the workers have been started; match_device() waits
 // for a segment's event to be recorded before it lets the stream wait on it, finish_staging() joins.
-int Engine::stage_pageable(const uint8_t *src, size_t n, uint64_t nseg) {
+int Engine::stage_pageable(const uint8_t *src, size_t n, uint64_t nseg, size_t dst_off) {
   EngineImpl &E = *impl_;
   Stager &S = E.stager;
   const uint64_t n_pieces = (n + kPieceBytes - 1) / kPieceBytes;
@@ -691,7 +700,7 @@ int Engine::stage_pageable(const uint8_t *src, size_t n, uint64_t nseg) {
   S.next_piece.store(0);
   S.failed.store(0);
   S.active = true;
-  uint8_t *dst = static_cast<uint8_t *>(E.hay.p);
+  uint8_t *dst = static_cast<uint8_t *>(E.hay.p) + dst_off;
   for (int t = 0; t < T; ++t) {
     S.workers.emplace_back([&E, &S, src, dst, n, n_pieces, per_seg, nseg, t]() {
       if (cudaSetDevice(E.device) != cudaSuccess) S.failed.store(1);
@@ -761,6 +770,173 @@ int Engine::match_shard_host(const uint8_t *host_slice, const ScanRange &range, 
   OLM_CUDA(cudaStreamSynchronize(E.copy_stream));
   cudaEventElapsedTime(&ms, E.ev[4], E.ev[5]);
   E.last.h2d_ms = ms;
+  return 0;
+}
+
+// ---- streams (include/olm_b200.h "Streams")
+//
+// A push scans the owned positions [settled before, settled after) as a byte-range shard of the whole
+// stream (SURVEY 8e) with global_size = received, so no predicate sees the end early.  The bytes it
+// needs in front of the piece are the carried ones: [settled - 16, received) of a plain store, the
+// incomplete window of a transforming one.  Host pieces are staged behind the carried bytes in the
+// haystack buffer and scanned in one call.  Device pieces of a plain store are scanned in place: only
+// the seam -- the positions up to the piece's 16th byte -- is scanned from the carried bytes and the
+// piece's first largest + 17 bytes; its records go in front of the bulk's.  Other device pieces are
+// copied behind the carried bytes.  no_overlap runs on the push's records with the stream's floor.
+
+namespace {
+void add_timing(olm_cuda_timing_t &t, const olm_cuda_timing_t &a) {
+  t.total_ms += a.total_ms;
+  t.transform_ms += a.transform_ms;
+  t.scan_ms += a.scan_ms;
+  t.filter_ms += a.filter_ms;
+  t.h2d_ms += a.h2d_ms;
+  t.d2h_ms += a.d2h_ms;
+  t.scan_launches += a.scan_launches;
+  t.kernel_launches += a.kernel_launches;
+  t.matches_before_filter += a.matches_before_filter;
+}
+} // namespace
+
+void Engine::stream_release(StreamState &s) {
+  if (s.carry) {
+    cudaSetDevice(impl_->device);
+    cudaFree(s.carry);
+  }
+  s.carry = nullptr;
+  s.carry_cap = 0;
+}
+
+int Engine::stream_push(StreamState &s, const void *bytes, size_t n, bool on_device, bool last,
+                        olm_cuda_results_t *out, uint64_t *counts) {
+  EngineImpl &E = *impl_;
+  OLM_CUDA(cudaSetDevice(E.device));
+  out->count = 0;
+  out->records = nullptr;
+  out->device = E.device;
+  if (s.finished || s.failed || (n && !bytes)) {
+    std::fprintf(stderr, "libomega_match(b200): stream push %s\n",
+                 s.failed ? "after a failed push" : s.finished ? "after the last push" : "of NULL bytes");
+    return -1;
+  }
+  s.failed = true; // until the push has succeeded
+  if (on_device) OLM_CUDA(cudaDeviceSynchronize()); // the piece may come from any stream of the caller
+  E.span_acc = omega_match_stats_t{};
+  const bool windowed = E.hdr.flags & kFlagAnyTransform;
+  const uint64_t R = s.received, recv = R + n, largest = E.hdr.largest;
+  uint64_t settled = recv;
+  if (!last && windowed) {
+    settled = recv / kWindowBytes * kWindowBytes;
+  } else if (!last) { // (a shard starts at 0 or has 16 bytes in front: below 16 nothing settles)
+    const uint64_t k = recv > largest + 1 ? recv - largest - 1 : 0;
+    settled = std::max<uint64_t>(s.settled, k >= 16 ? k : 0);
+  }
+  const uint64_t carried = R - s.carry_begin; // bytes in front of the piece
+  unsigned long long *d_counts = nullptr;
+  if (counts && !(d_counts = zeroed_counts())) return -1;
+  MatchFlags fs = s.f;
+  const uint8_t *piece = static_cast<const uint8_t *>(bytes);
+  // plain store, aligned device piece with positions past its 16th byte to settle: in place
+  const bool in_place =
+      on_device && !counts && !windowed && !(reinterpret_cast<uintptr_t>(bytes) & 15) && settled > R + 16;
+  olm_cuda_results_t res{};
+  if (!in_place) { // carried bytes + piece in the haystack buffer, one call
+    if (on_device) {
+      if (E.hay.ensure(((carried + n + 15) & ~size_t(15)) + 256)) return -1;
+      if (n) OLM_CUDA(cudaMemcpyAsync(static_cast<uint8_t *>(E.hay.p) + carried, piece, n, cudaMemcpyDeviceToDevice, E.stream));
+    } else if (n && stage_host(piece, n, carried)) {
+      return -1;
+    } else if (!n && E.hay.ensure(((carried + 15) & ~size_t(15)) + 256)) {
+      return -1;
+    }
+    if (carried) OLM_CUDA(cudaMemcpyAsync(E.hay.p, s.carry, carried, cudaMemcpyDeviceToDevice, E.stream));
+    ScanRange r{E.hay.p, s.carry_begin, recv - s.carry_begin, s.settled, settled, recv, s.match_ptr_base, s.floor, 0};
+    int rc;
+    {
+      const bool staged = !on_device && n;
+      if (staged) E.streaming = true;
+      rc = match_device(r, fs, &res, d_counts);
+      // the new carried bytes are copied out of the buffer below: all of the piece has to be there
+      if (staged) {
+        E.streaming = false;
+        if (rc == 0 && !E.seg_events.empty() && wait_segment(E, E.seg_events.size() - 1)) rc = -1;
+        if (finish_staging() != 0) rc = -1;
+        float ms = 0.f;
+        OLM_CUDA(cudaStreamSynchronize(E.copy_stream));
+        cudaEventElapsedTime(&ms, E.ev[4], E.ev[5]);
+        E.last.h2d_ms = ms;
+      }
+    }
+    if (rc != 0) return -1;
+  } else { // seam from the haystack buffer, then the bulk in the caller's buffer
+    const uint64_t seam_bytes = std::min<uint64_t>(n, largest + 17);
+    if (E.hay.ensure(((carried + seam_bytes + 15) & ~size_t(15)) + 256)) return -1;
+    if (carried) OLM_CUDA(cudaMemcpyAsync(E.hay.p, s.carry, carried, cudaMemcpyDeviceToDevice, E.stream));
+    OLM_CUDA(cudaMemcpyAsync(static_cast<uint8_t *>(E.hay.p) + carried, piece, seam_bytes, cudaMemcpyDeviceToDevice, E.stream));
+    fs.no_overlap = false; // (once, on the concatenation)
+    const ScanRange seam{E.hay.p, s.carry_begin, carried + seam_bytes, s.settled, R + 16, recv, s.match_ptr_base, 0, 0};
+    if (match_device(seam, fs, &res)) return -1;
+    const olm_cuda_timing_t t_seam = E.last;
+    { // the seam's statistics are collected with the bulk's (as host_spans does with its spans)
+      omega_match_stats_t acc{};
+      collect_stats(&acc);
+      E.span_acc = acc;
+    }
+    const uint64_t n_seam = res.count;
+    if (n_seam && E.gather.ensure(n_seam * sizeof(Record))) return -1;
+    if (n_seam) OLM_CUDA(cudaMemcpyAsync(E.gather.p, res.records, n_seam * sizeof(Record), cudaMemcpyDeviceToDevice, E.stream));
+    const ScanRange bulk{piece, R, n, R + 16, settled, recv, s.match_ptr_base, 0, n_seam};
+    if (match_device(bulk, fs, &res)) return -1;
+    add_timing(E.last, t_seam);
+    if (n_seam) OLM_CUDA(cudaMemcpyAsync(E.out.p, E.gather.p, n_seam * sizeof(Record), cudaMemcpyDeviceToDevice, E.stream));
+    res.records = E.out.p;
+    res.count += n_seam;
+    if (s.f.no_overlap && res.count) {
+      const int64_t kept = no_overlap_inplace(E.out.p, res.count, nullptr, s.floor);
+      if (kept < 0) return -1;
+      res.count = uint64_t(kept);
+    }
+  }
+  // the floor of the next push: the end of the last kept record
+  if (s.f.no_overlap && res.count) {
+    Record lastrec;
+    OLM_CUDA(cudaMemcpyAsync(&lastrec, static_cast<const Record *>(res.records) + (res.count - 1), sizeof lastrec,
+                             cudaMemcpyDeviceToHost, E.stream));
+    OLM_CUDA(cudaStreamSynchronize(E.stream));
+    s.floor = lastrec.offset + lastrec.len;
+  }
+  if (counts && add_counts_to_host(counts)) return -1;
+  // carry [next_begin, recv): what lies before the piece from the haystack buffer, the rest from the
+  // buffer too unless the piece was scanned in place
+  const uint64_t next_begin = last ? recv : windowed ? settled : (settled >= 16 ? settled - 16 : 0);
+  const uint64_t keep = recv - next_begin;
+  if (keep > s.carry_cap) {
+    OLM_CUDA(cudaStreamSynchronize(E.stream));
+    if (s.carry) cudaFree(s.carry);
+    s.carry = nullptr;
+    s.carry_cap = 0;
+    const size_t want = std::max<size_t>(keep, 4096);
+    OLM_CUDA(cudaMalloc(&s.carry, want));
+    s.carry_cap = want;
+  }
+  const uint8_t *hay = static_cast<const uint8_t *>(E.hay.p);
+  uint8_t *dst = static_cast<uint8_t *>(s.carry);
+  if (in_place) {
+    const uint64_t a = std::min(next_begin, R); // [a, R) from the carried bytes in front of the seam
+    if (R > a) OLM_CUDA(cudaMemcpyAsync(dst, hay + (a - s.carry_begin), R - a, cudaMemcpyDeviceToDevice, E.stream));
+    const uint64_t b = std::max(next_begin, R);
+    if (recv > b) OLM_CUDA(cudaMemcpyAsync(dst + (b - next_begin), piece + (b - R), recv - b, cudaMemcpyDeviceToDevice, E.stream));
+  } else if (keep) {
+    OLM_CUDA(cudaMemcpyAsync(dst, hay + (next_begin - s.carry_begin), keep, cudaMemcpyDeviceToDevice, E.stream));
+  }
+  OLM_CUDA(cudaStreamSynchronize(E.stream));
+  s.carry_begin = next_begin;
+  s.received = recv;
+  s.settled = settled;
+  s.finished = last;
+  s.failed = false;
+  *out = res;
+  out->device = E.device;
   return 0;
 }
 
@@ -879,10 +1055,10 @@ int Engine::format_records(const void *dev_records, uint64_t count, const void *
   return 0;
 }
 
-int64_t Engine::no_overlap_inplace(void *dev_records, uint64_t count, void *dev_positions) {
+int64_t Engine::no_overlap_inplace(void *dev_records, uint64_t count, void *dev_positions, uint64_t floor) {
   EngineImpl &E = *impl_;
   OLM_CUDA(cudaSetDevice(E.device));
-  if (count < 2) return (int64_t)count;
+  if (count < (floor ? 1 : 2)) return (int64_t)count;
   // the records may have been produced on any stream of the caller (a gather, a copy): the
   // matcher's stream is non-blocking and would not wait for them (same contract as match_device)
   OLM_CUDA(cudaDeviceSynchronize());
@@ -895,7 +1071,7 @@ int64_t Engine::no_overlap_inplace(void *dev_records, uint64_t count, void *dev_
   unsigned long long total = 0;
   if (dev_positions && E.d_pos2.ensure(count * sizeof(LinePos))) return -1;
   OLM_CUDA(no_overlap_launch(static_cast<const Record *>(dev_records), count, static_cast<Record *>(E.out2.p),
-                             E.fscratch.p, d_ftotal, E.stream, &launches, static_cast<const LinePos *>(dev_positions),
+                             E.fscratch.p, d_ftotal, E.stream, &launches, floor, static_cast<const LinePos *>(dev_positions),
                              static_cast<LinePos *>(E.d_pos2.p)));
   OLM_CUDA(cudaMemcpyAsync(&total, d_ftotal, sizeof total, cudaMemcpyDeviceToHost, E.stream));
   OLM_CUDA(cudaStreamSynchronize(E.stream));

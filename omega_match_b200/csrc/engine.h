@@ -26,6 +26,8 @@ struct ScanRange {
   uint64_t own_begin = 0, own_end = 0; // start positions reported by this call
   uint64_t global_size = 0;
   uint64_t match_ptr_base = 0;
+  uint64_t floor = 0;     // no_overlap: records before it are dropped, the chain starts there (filters.cuh)
+  uint64_t out_front = 0; // records left free in front of the call's output (no_overlap off)
 };
 
 // Byte-range shards of one haystack (SURVEY 8e): a shard OWNS the start positions [own_begin,
@@ -46,6 +48,19 @@ inline ScanRange scan_range(const Shard &s, uint64_t size, uint64_t match_ptr_ba
 }
 
 struct EngineImpl;
+
+// One stream (include/olm_b200.h "Streams"): the haystack arrives in pushes; `carry` holds the device
+// bytes [carry_begin, received) the next push scans again (halo, or the incomplete 4 MiB window).
+struct StreamState {
+  MatchFlags f;
+  uint64_t match_ptr_base = 0;
+  uint64_t received = 0, settled = 0;
+  uint64_t floor = 0; // no_overlap: the end of the last kept record
+  bool finished = false, failed = false;
+  void *carry = nullptr;
+  size_t carry_cap = 0;
+  uint64_t carry_begin = 0;
+};
 
 // What olm_cuda_match_lines / olm_cuda_matching_lines return.
 struct LinesResult {
@@ -87,7 +102,8 @@ public:
   int format_records(const void *dev_records, uint64_t count, const void *dev_haystack, uint64_t offset0,
                      void **dev_text, uint64_t *text_bytes);
   // (with dev_positions: the records' line positions are compacted with them)
-  int64_t no_overlap_inplace(void *dev_records, uint64_t count, void *dev_positions = nullptr);
+  // (floor: see ScanRange::floor)
+  int64_t no_overlap_inplace(void *dev_records, uint64_t count, void *dev_positions = nullptr, uint64_t floor = 0);
   int sort_records(void *dev_records, uint64_t count);
 
   // for the multi-GPU layer (multi.cpp)
@@ -138,14 +154,22 @@ public:
   // device records + positions -> host arrays, or (lines_only) their matching lines
   int lines_to_host(const void *dev_records, const void *dev_positions, uint64_t count, bool lines_only,
                     LinesResult *out);
+  // Streams: one push of `n` bytes (host or device memory) -> the records it settles, on the device
+  // (valid until the next call), or with `counts`: counts[id] += the records of pattern id (the tables
+  // loaded).  The piece is not referenced after the call.  stream_release frees the carried bytes.
+  int stream_push(StreamState &s, const void *bytes, size_t n, bool on_device, bool last, olm_cuda_results_t *out,
+                  uint64_t *counts = nullptr);
+  void stream_release(StreamState &s);
+
   const void *resident_haystack() const;           // the device copy of the last host haystack or slice
   void *positions_buffer(size_t bytes, int which); // device buffers for positions: 0 = a call's, 1 = gathered
   int copy_to_host(void *host_dst, const void *dev_src, size_t bytes); // asynchronous, on stream()
 
 private:
   Engine() = default;
-  int stage_host(const uint8_t *src, size_t n);
-  int stage_pageable(const uint8_t *src, size_t n, uint64_t nseg);
+  // (dst_off: where the bytes go in the haystack buffer, which may be reallocated to dst_off + n bytes)
+  int stage_host(const uint8_t *src, size_t n, size_t dst_off = 0);
+  int stage_pageable(const uint8_t *src, size_t n, uint64_t nseg, size_t dst_off);
   int finish_staging();
   // step(span, its device records, several spans)
   using SpanStep = std::function<int(const Shard &, const olm_cuda_results_t &, bool)>;

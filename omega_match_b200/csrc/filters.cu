@@ -8,7 +8,9 @@
 //                  its first accepted match); longest_flags_kernel is the stand-alone form,
 //                  used on gathered shard results and by tests.
 //   no-overlap   : "keep a record iff offset >= end of the previous KEPT record" -- a greedy
-//                  chain.  Parallel form (SURVEY H4): with E_i = max end over records < i,
+//                  chain.  With a floor, records that start before it are dropped and the chain
+//                  starts at the first record at or past it (the records are sorted, so those are
+//                  a prefix: one test per record finds it).  Parallel form (SURVEY H4): with E_i = max end over records < i,
 //                  record i is a CERTAIN START iff E_i <= offset_i (nothing earlier reaches
 //                  it, so it is kept whatever the chain did before).  Chains between certain
 //                  starts are independent; each is walked by one thread with a galloping
@@ -28,15 +30,17 @@ namespace {
 
 __device__ __forceinline__ unsigned long long rec_end(const Record &r) { return r.offset + r.len; }
 
-__global__ void __launch_bounds__(kFThreads) end_max_aggregate_kernel(const Record *r, uint64_t n, unsigned long long *agg) {
-  block_aggregate<MaxOp>(n, agg, [&](uint64_t i) { return rec_end(r[i]); });
+// (records below the floor reach nothing: their end counts as 0, the identity of the max)
+__global__ void __launch_bounds__(kFThreads) end_max_aggregate_kernel(const Record *r, uint64_t n, uint64_t floor,
+                                                                      unsigned long long *agg) {
+  block_aggregate<MaxOp>(n, agg, [&](uint64_t i) { return r[i].offset >= floor ? rec_end(r[i]) : 0ull; });
 }
 __global__ void __launch_bounds__(kFThreads) keep_sum_aggregate_kernel(const uint8_t *keep, uint64_t n, unsigned long long *agg) {
   block_aggregate<SumOp>(n, agg, [&](uint64_t i) { return (unsigned long long)keep[i]; });
 }
 
 // phase 3 (prefix max): certain-start flags
-__global__ void __launch_bounds__(kFThreads) certain_start_kernel(const Record *r, uint64_t n,
+__global__ void __launch_bounds__(kFThreads) certain_start_kernel(const Record *r, uint64_t n, uint64_t floor,
                                                                   const unsigned long long *agg, uint8_t *start) {
   const uint64_t base = (uint64_t)blockIdx.x * kFBlock + (uint64_t)threadIdx.x * kFItems;
   unsigned long long ends[kFItems], offs[kFItems];
@@ -47,7 +51,7 @@ __global__ void __launch_bounds__(kFThreads) certain_start_kernel(const Record *
     if (base + k < n) {
       const Record x = r[base + k];
       offs[k] = x.offset;
-      ends[k] = x.offset + x.len;
+      ends[k] = x.offset >= floor ? x.offset + x.len : 0;
       a = a > ends[k] ? a : ends[k];
     }
   }
@@ -56,7 +60,7 @@ __global__ void __launch_bounds__(kFThreads) certain_start_kernel(const Record *
 #pragma unroll
   for (int k = 0; k < kFItems; ++k) {
     if (base + k < n) {
-      start[base + k] = (base + k == 0 || run <= offs[k]) ? 1 : 0;
+      start[base + k] = (offs[k] >= floor && run <= offs[k]) ? 1 : 0;
       run = run > ends[k] ? run : ends[k];
     }
   }
@@ -134,7 +138,7 @@ static cudaError_t compact(const Record *in, uint64_t n, const uint8_t *keep, un
 }
 
 cudaError_t no_overlap_launch(const Record *in, uint64_t n, Record *out, void *scratch,
-                              unsigned long long *d_total, cudaStream_t st, uint32_t *launches,
+                              unsigned long long *d_total, cudaStream_t st, uint32_t *launches, uint64_t floor,
                               const LinePos *in_pos, LinePos *out_pos) {
   if (n == 0) return cudaSuccess;
   const uint32_t blocks = uint32_t((n + kFBlock - 1) / kFBlock);
@@ -143,9 +147,9 @@ cudaError_t no_overlap_launch(const Record *in, uint64_t n, Record *out, void *s
   unsigned long long *agg = reinterpret_cast<unsigned long long *>((reinterpret_cast<uintptr_t>(keep + n) + 63) & ~uintptr_t(63));
   cudaError_t e = cudaMemsetAsync(keep, 0, n, st);
   if (e != cudaSuccess) return e;
-  end_max_aggregate_kernel<<<blocks, kFThreads, 0, st>>>(in, n, agg);
+  end_max_aggregate_kernel<<<blocks, kFThreads, 0, st>>>(in, n, floor, agg);
   aggregate_scan_kernel<MaxOp><<<1, kFThreads, 0, st>>>(agg, blocks, nullptr);
-  certain_start_kernel<<<blocks, kFThreads, 0, st>>>(in, n, agg, start);
+  certain_start_kernel<<<blocks, kFThreads, 0, st>>>(in, n, floor, agg, start);
   chain_walk_kernel<<<uint32_t((n + kFThreads - 1) / kFThreads), kFThreads, 0, st>>>(in, n, start, keep);
   *launches += 4;
   if ((e = cudaGetLastError()) != cudaSuccess) return e;

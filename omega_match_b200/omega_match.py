@@ -410,6 +410,12 @@ class Matcher:
             raise RuntimeError("olm_cuda_matching_lines_device failed (see stderr)")
         return int(n.value), int(p.value or 0)
 
+    def stream(self, match_ptr_base: int = 0, **kw) -> "MatchStream":
+        """A stream over one haystack that arrives in pieces (include/olm_b200.h "Streams"): the records
+        of all pushes, in push order, are those of one match over the concatenation, with offsets
+        counted from the stream's first byte."""
+        return MatchStream(self, match_ptr_base, **kw)
+
     def match_device(self, dev_ptr: int, size: int, match_ptr_base: Optional[int] = None, **kw):
         """Haystack already in HBM (16-byte aligned device pointer).  Returns (count, device
         pointer of the 24-byte records); the records stay valid until the next call.  With
@@ -508,3 +514,85 @@ class Matcher:
     @property
     def device(self) -> int:
         return self._lib.olm_cuda_matcher_device(self._matcher)
+
+
+class MatchStream:
+    """Consecutive pieces of one haystack pushed into a Matcher (Matcher.stream()).  A context manager;
+    it keeps its Matcher alive and must be closed before the Matcher is destroyed."""
+
+    def __init__(self, matcher: Matcher, match_ptr_base: int = 0, **kw) -> None:
+        self._matcher = matcher
+        self._lib = matcher._lib
+        self._s = self._lib.olm_cuda_stream_open(matcher._matcher, *_flag_ints(kw), match_ptr_base)
+        if not self._s:
+            raise RuntimeError("olm_cuda_stream_open failed")
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *_exc) -> None:
+        self.close()
+
+    def __del__(self):
+        self.close()
+
+    def close(self) -> None:
+        if getattr(self, "_s", None):
+            self._lib.olm_cuda_stream_close(self._s)
+            self._s = None
+
+    def _state(self):
+        st = _lib.StreamStateC()
+        if not self._s or self._lib.olm_cuda_stream_state(self._s, C.byref(st)) != 0:
+            raise RuntimeError("the stream is closed")
+        return st
+
+    @property
+    def received(self) -> int:
+        return int(self._state().received)
+
+    @property
+    def settled(self) -> int:
+        return int(self._state().settled)
+
+    def push(self, data, last: bool = False) -> np.ndarray:
+        """Host bytes (bytes, memoryview or uint8 array) -> the records this push settled: MATCH_DTYPE,
+        or MATCH_IDS_DTYPE while pattern ids are on."""
+        hay, ptr, n = _host_haystack(data)
+        res = C.POINTER(_lib.MatchResultsC)()
+        if not self._s or self._lib.olm_cuda_stream_push(self._s, ptr, n, int(bool(last)), C.byref(res)) != 0:
+            raise RuntimeError("olm_cuda_stream_push failed (see stderr)")
+        cnt = res.contents.count
+        rec = np.zeros(cnt, dtype=RECORD_DTYPE)
+        if cnt:
+            C.memmove(rec.ctypes.data, res.contents.matches, cnt * RECORD_DTYPE.itemsize)
+        self._lib.omega_match_results_destroy(res)
+        ids = self._matcher._pattern_ids
+        out = np.zeros(cnt, dtype=MATCH_IDS_DTYPE if ids else MATCH_DTYPE)
+        out["offset"] = rec["offset"]
+        out["len"] = rec["len"]
+        if ids:
+            out["pattern_id"] = rec["_pad"]
+        return out
+
+    def push_device(self, dev_ptr: int, size: int, last: bool = False):
+        """Device bytes (the contract of Matcher.match_device) -> (device pointer of the settled
+        24-byte records, their count); valid until the next call on the matcher."""
+        res = CudaResultsC()
+        if not self._s or self._lib.olm_cuda_stream_push_device(self._s, dev_ptr, size, int(bool(last)),
+                                                                C.byref(res)) != 0:
+            raise RuntimeError("olm_cuda_stream_push_device failed (see stderr)")
+        return int(res.records or 0), int(res.count)
+
+    def count(self, data, counts: np.ndarray, last: bool = False) -> int:
+        """Host bytes -> counts[id] += the settled records of pattern id (counts: uint64 array of
+        pattern_count entries); returns their number."""
+        if not (isinstance(counts, np.ndarray) and counts.dtype == np.uint64 and counts.flags.c_contiguous
+                and counts.size >= self._matcher.pattern_count):
+            raise ValueError("counts must be a contiguous uint64 array of pattern_count entries")
+        hay, ptr, n = _host_haystack(data)
+        total = C.c_uint64()
+        if not self._s or self._lib.olm_cuda_stream_count(self._s, ptr, n, int(bool(last)), counts.ctypes.data,
+                                                          C.byref(total)) != 0:
+            raise RuntimeError("olm_cuda_stream_count failed (see stderr)")
+        return int(total.value)
