@@ -510,6 +510,7 @@ typedef struct {
   uint32_t class_ranges;   /* 1 or 2 */
   uint32_t class_lo[2], class_hi[2];
   uint32_t key_bytes;      /* leading pattern bytes a key covers (4..8) */
+  uint32_t coop;           /* 1: the scan compares the records of a key as a warp (COOP kernels) */
 } olm_store_info_t;
 int olm_store_inspect(const char *compiled_file, olm_store_info_t *out);
 

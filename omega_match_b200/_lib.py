@@ -69,7 +69,8 @@ class StoreInfoC(C.Structure):
                                          "occupied_buckets", "len1", "len2", "len3", "len4")] + [
         ("store_bytes", C.c_uint64), ("file_bytes", C.c_uint64)] + [
         (n, C.c_uint32) for n in ("gram_keys", "key_buckets", "g4_bits", "class_run", "class_and_mask",
-                                  "class_ranges")] + [("class_lo", C.c_uint32 * 2), ("class_hi", C.c_uint32 * 2), ("key_bytes", C.c_uint32)]
+                                  "class_ranges")] + [("class_lo", C.c_uint32 * 2), ("class_hi", C.c_uint32 * 2), ("key_bytes", C.c_uint32),
+                                  ("coop", C.c_uint32)]
 
     def as_dict(self):
         d = {}

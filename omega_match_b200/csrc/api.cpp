@@ -666,6 +666,7 @@ int olm_store_inspect(const char *compiled_file, olm_store_info_t *out) {
       out->file_bytes = n;
       out->gram_keys = s.n_keys;
       out->key_bytes = s.params.key_bytes;
+      out->coop = s.params.coop;
       out->key_buckets = s.params.key_mask + 1;
       out->g4_bits = s.params.g4_words * 32;
       out->class_run = s.params.cls.run;

@@ -130,7 +130,7 @@ struct EngineImpl {
   ScanGeometry geo;
   bool has_short_234 = false;
   DevBuf d_keys, d_slots, d_recs, d_store, d_g4, d_p23, d_set3, d_bitmap2, d_sx;
-  DevBuf hay, out, out2, chunk_desc, span_base, temp, tfblocks, tfvisible, tfplan, tfextent, misc, windows, ghost, fscratch, gather, text;
+  DevBuf hay, out, out2, chunk_desc, span_base, temp, tfblocks, tfvisible, tfplan, tfextent, misc, windows, ghost, ghost_start, fscratch, gather, text;
   cudaEvent_t ev[8] = {};
   olm_cuda_timing_t last{};
   uint64_t out_hint = 0;
@@ -321,7 +321,7 @@ Engine::~Engine() {
   cudaSetDevice(impl_->device);
   for (DevBuf *b : {&impl_->d_keys, &impl_->d_slots, &impl_->d_recs, &impl_->d_store, &impl_->d_g4, &impl_->d_p23, &impl_->d_sx, &impl_->d_set3,
                     &impl_->d_bitmap2, &impl_->hay, &impl_->out, &impl_->out2, &impl_->chunk_desc, &impl_->span_base, &impl_->temp, &impl_->tfblocks, &impl_->tfvisible, &impl_->tfplan, &impl_->tfextent, &impl_->misc,
-                    &impl_->windows, &impl_->gather, &impl_->text, &impl_->ghost, &impl_->fscratch, &impl_->d_bloom, &impl_->d_smap,
+                    &impl_->windows, &impl_->gather, &impl_->text, &impl_->ghost, &impl_->ghost_start, &impl_->fscratch, &impl_->d_bloom, &impl_->d_smap,
                     &impl_->d_slens, &impl_->d_id_table, &impl_->d_id_refs, &impl_->d_id_short, &impl_->d_counts,
                     &impl_->d_tiles, &impl_->d_pos, &impl_->d_pos2, &impl_->d_pos_gather, &impl_->d_lines, &impl_->d_lscratch})
     b->release();
@@ -445,9 +445,20 @@ int Engine::match_device(const ScanRange &r, const MatchFlags &f, olm_cuda_resul
   if (identity_map) fl |= kIdentityMap;
   if (E.want_stats) fl |= kCountAll;
 
+  // Stores that drop bytes, under word_boundary: every launch group reads its stale tails from the
+  // image and then writes its windows into it (transform.cu window_descs_launch).  A second attempt
+  // has to read the image the call started with, not the one the first attempt left behind.
+  const bool keep_ghost = need_desc && !identity_map;
+  if (keep_ghost) {
+    if (E.ghost_start.ensure(kWindowBytes + 64)) return -1;
+    OLM_CUDA(cudaMemcpyAsync(E.ghost_start.p, E.ghost.p, kWindowBytes + 64, cudaMemcpyDeviceToDevice, E.stream));
+  }
+
   unsigned long long total = 0, temp_used = 0;
   uint64_t temp_extra = 0; // grows when the block allocator of temp[] wasted more than the slack
   for (int attempt = 0; attempt < 4; ++attempt) {
+    if (keep_ghost && attempt > 0)
+      OLM_CUDA(cudaMemcpyAsync(E.ghost.p, E.ghost_start.p, kWindowBytes + 64, cudaMemcpyDeviceToDevice, E.stream));
     if (E.out.ensure((cap + front) * sizeof(Record))) return -1;
     cap = E.out.cap / sizeof(Record) - front;
     const uint64_t temp_cap = cap + cap / 2 + temp_slack_entries(E.sms) * n_batches + temp_extra;
